@@ -2,7 +2,7 @@
 """Benchmark of the batched operational-space controller (BASELINE.json metric:
 robot control cycles/sec, batched OSC torques; p99 cycle latency).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--robots R] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--robots R] [--impl reference] [--dump-outputs DIR]
 
 A step = one control cycle (kinematics/dynamics -> task models -> torques) for one batch of
 R robots per GPU.  Workload (config.workload): BASELINE config 2 -- Panda, MotionForceTask 6-DoF at the
@@ -18,9 +18,14 @@ robots are sharded by batch index, one process per GPU, no collective on the con
          port (oracle/cpp) is timed beside it (`port`), and takes over (kind "port") where the library was not built.
 --impl reference runs only that CPU arm, on the same 65,536 states as the GPU arm, all host threads.
 
-Timing: `--steps K` back-to-back cycles form one bracket (CUDA events, barrier + synchronize on both sides); brackets are
-repeated until at least MIN_TIMED_MS of device time and MIN_PASSES brackets have been taken, and the MEDIAN bracket is
-published (`ms_per_step` = median / K, `timing` lists the passes) -- a 20-step bracket alone lasts 0.7 ms.
+Timing: after SETUP_ROUNDS set-up cycles of every controller instance (`timing.setup_cycles`) and `--warmup W` cycles,
+exactly `--steps K` back-to-back cycles are timed between two CUDA events (barrier + synchronize on both sides);
+`ms_per_step` = that time / K.  A 20-step region lasts about 0.7 ms, so small K is noisy.
+
+--dump-outputs DIR writes the torques of the last timed cycle (rank 0's batch) to DIR/tau.npy, float64, in the [dof, robots]
+layout osc_step returns; above DUMP_BYTES_MAX a fixed sample of robots is written, with their indices (stored as float64)
+in DIR/robot_index.npy.  The inputs depend only on the arguments (seeded), so two builds can be compared output for output.
+The benchmark writes nothing into the source tree.
 """
 import argparse
 import ctypes as C
@@ -33,6 +38,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True    # the source tree may be read-only: no __pycache__ for the modules imported below
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -46,8 +52,8 @@ WORKLOAD = "config2: Panda MotionForceTask 6-DoF + JointTask null space via Robo
 ROBOT = "panda"
 LINK, POINT = "end-effector", (0.0, 0.0, 0.07)
 SEED = 1234
-MIN_TIMED_MS = 60.0           # device time over all brackets
-MIN_PASSES = 5
+DUMP_BYTES_MAX = 64_000_000   # --dump-outputs: larger outputs are written as a fixed sample of robots
+SETUP_ROUNDS = 6              # set-up cycles per controller instance before the warm-up (see gpu_arm)
 LATENCY_SAMPLES = 1000        # SURVEY.md 8d: >= 1000 single-cycle brackets for the percentiles
 
 
@@ -63,6 +69,22 @@ def workload_config(args, world):
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_outputs(out_dir, tau_of_last_step):
+    """--dump-outputs: tau [dof, robots] as DIR/tau.npy; beyond DUMP_BYTES_MAX, a fixed sample of robots (same indices on
+    every run with the same arguments) plus DIR/robot_index.npy, the sampled robots' indices in ascending order, stored as
+    float64 (exact below 2**53) so that every file of the dump has the same dtype"""
+    os.makedirs(out_dir, exist_ok=True)
+    tau = np.ascontiguousarray(tau_of_last_step, dtype=np.float64)
+    n, R = tau.shape
+    if R * n * 8 > DUMP_BYTES_MAX:
+        keep = ((DUMP_BYTES_MAX - 4096) // 8) // (n + 1)     # a sampled robot costs n torques + its index; 4 KB for headers
+        idx = np.sort(np.random.default_rng(0).choice(R, size=keep, replace=False))
+        np.save(os.path.join(out_dir, "robot_index.npy"), idx.astype(np.float64))
+        tau = np.ascontiguousarray(tau[:, idx])
+    np.save(os.path.join(out_dir, "tau.npy"), tau)
+    log("[dump] tau of the last timed cycle, %d x %d float64 -> %s" % (tau.shape[0], tau.shape[1], out_dir))
 
 
 # ------------------------------------------------------------------ synthetic inputs (SURVEY.md 8d)
@@ -282,6 +304,8 @@ def reference_arm(args):
     dt = time.perf_counter() - t0
     if not np.isfinite(tau).all():
         raise SystemExit("bench --impl reference: non-finite torques")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tau_of_last_step=tau.T)
     value = args.robots * args.steps / dt
     sample = "%d robots x %d cycles (the GPU arm's config: same robot count per step, same state filter s_min/s_max >= %.3g), %s, %d host threads" \
              % (args.robots, args.steps, args.min_ratio, KIND_TEXT[kind], cc.threads)
@@ -415,46 +439,42 @@ def gpu_arm(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    launches0 = sum(s["robot"].launchCount() for s in sets)
-    # ---- device-resident timing
-    for w in range(args.warmup):
-        step_device(sets[w % n_sets])
-    barrier()
-    launches0 = sum(s["robot"].launchCount() for s in sets)
+    # ---- device-resident timing.  The clock sampler starts first so that the set-up and warm-up cycles, not an idle
+    # pause, come right before the timed region.
     clocks = ClockSampler(local_rank)
     if rank == 0:
         clocks.start()
         time.sleep(0.25)
+    # set-up: a handle picks its general-path grid from the hand-over counts of completed cycles and needs a few cycles
+    # to settle on the small one (osc_capi.cu run_cycle), so every instance runs them here: rounds of one cycle per
+    # instance, back to back like the timed region, each round completed before the next
+    for _ in range(SETUP_ROUNDS):
+        for s_ in sets:
+            step_device(s_)
+        torch.cuda.synchronize()
+    for w in range(args.warmup):
+        step_device(sets[w % n_sets])
+    barrier()
     t_wall0 = time.time()
-    # one bracket = args.steps back-to-back cycles, nothing else in the stream; brackets are repeated until MIN_TIMED_MS of
-    # device time and MIN_PASSES brackets are in, the median bracket is the published one
-    pass_ms = []
-    launches = 0
-    while True:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        l0 = sum(s["robot"].launchCount() for s in sets)
-        barrier()
-        e0.record()
-        for k in range(args.steps):     # the timed region: K back-to-back cycles, nothing else in the stream
-            step_device(sets[k % n_sets])
-        e1.record()
-        barrier()
-        pass_ms.append(e0.elapsed_time(e1))
-        launches = sum(s["robot"].launchCount() for s in sets) - l0
-        more = 1.0 if (len(pass_ms) < MIN_PASSES or (sum(pass_ms) < MIN_TIMED_MS and len(pass_ms) < 2000)) else 0.0
-        if world > 1:      # every rank takes the same number of brackets
-            flag = torch.tensor([more], device=dev)
-            dist.all_reduce(flag, op=dist.ReduceOp.MAX)
-            more = float(flag.item())
-        if more == 0.0:
-            break
+    # the timed region: exactly args.steps back-to-back cycles between two CUDA events, nothing else in the stream
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    l0 = sum(s["robot"].launchCount() for s in sets)
+    barrier()
+    e0.record()
+    for k in range(args.steps):
+        step_device(sets[k % n_sets])
+    e1.record()
+    barrier()
+    total_ms = e0.elapsed_time(e1)
+    launches = sum(s["robot"].launchCount() for s in sets) - l0
     t_wall1 = time.time()
-    pass_ms = np.array(pass_ms)
-    if world > 1:          # bracket by bracket: the slowest rank
-        t = torch.tensor(pass_ms, dtype=torch.float64, device=dev)
+    if world > 1:          # the slowest rank
+        t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        pass_ms = t.cpu().numpy()
-    total_ms = float(np.median(pass_ms))
+        total_ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        # later sections reuse the controller instances: keep what the last timed cycle returned now
+        dump_outputs(args.dump_outputs, tau_of_last_step=sets[(args.steps - 1) % n_sets]["tau"].cpu().numpy())
     # latency of a single batched cycle, measured in a second pass: an event between two cycles keeps the next fast
     # kernel from being scheduled behind the general-path kernel (programmatic dependent launch), so the per-cycle
     # brackets are not part of the throughput measurement
@@ -691,10 +711,11 @@ def gpu_arm(args):
             "dtype": "f64", "data": "synthetic",
             "config": workload_config(args, world),
             "inputs": {"rejected_fraction": rejected, "robots_on_the_general_path": singular_fraction},
-            "timing": {"brackets": int(pass_ms.size), "bracket_ms_median": total_ms, "bracket_ms_min": float(pass_ms.min()),
-                       "bracket_ms_max": float(pass_ms.max()), "timed_ms_total": float(pass_ms.sum()),
-                       "what": "each bracket = --steps back-to-back cycles between two CUDA events with barrier + synchronize on both sides; "
-                               "max over ranks per bracket; the median bracket is published"},
+            "timing": {"timed_steps": args.steps, "timed_ms_total": total_ms, "setup_cycles": SETUP_ROUNDS * n_sets,
+                       "warmup_cycles": args.warmup,
+                       "what": "--steps back-to-back cycles after setup_cycles (every controller instance until its launch "
+                               "configuration settles) and warmup_cycles, between two CUDA events with barrier + synchronize "
+                               "on both sides; max over ranks"},
             "latency_ms": {"p50": float(np.percentile(per_step_ms, 50)), "p99": float(np.percentile(per_step_ms, 99)),
                            "max": float(per_step_ms.max()), "samples": int(per_step_ms.size), "what": "CUDA events around one batched cycle, rank 0"},
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": int(2 * n * R * 8), "d2h_bytes_per_step": int(n * R * 8),
@@ -764,7 +785,11 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=16.0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--min-ratio", type=float, default=0.1, help="reject states with s_min/s_max below this (0: unfiltered, about half of the Panda states then take the singular branch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the torques of the last timed cycle to DIR/tau.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -3,6 +3,7 @@ reference's own JointTask / MotionForceTask with their internal OTG left ON -- t
 MotionForceTask.h:67): OTG_joints.cpp / OTG_6dof_cartesian.cpp + the vendored Ruckig compiled in place (oracle/_ref/libsai_ref*.so).
 Desired states AND torques are compared every cycle."""
 import math
+import os
 
 import numpy as np
 import pytest
@@ -17,7 +18,9 @@ def tau_err(tau, ref):
     return (np.abs(tau - ref).max(axis=1) / scale).max()
 
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not sai_ref.available(oriented=True), reason="needs oracle/_ref/libsai_ref_orient.so")]
+pytestmark = pytest.mark.gpu
+needs_reference_library = pytest.mark.skipif(not sai_ref.available(oriented=True), reason="needs oracle/_ref/libsai_ref_orient.so")
+GOLD_OTG = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "otg_joints_reference.npz")
 
 
 @pytest.fixture(autouse=True)
@@ -42,6 +45,7 @@ def test_mirror_default_is_the_reference_default():
         jt.enableInternalOtgAccelerationLimited(-1.0, 2.0)     # OTG_joints.cpp:50-54
 
 
+@needs_reference_library
 @pytest.mark.parametrize("robot_name", ["panda", "rrrr"])
 def test_joint_task_with_internal_otg(robot_name):
     """config 1 with the reference's default trajectory generation: goal steps in mid-motion (collinear and not), per-joint limits
@@ -97,6 +101,7 @@ def test_joint_task_with_internal_otg(robot_name):
     assert np.abs(jt.getGoalPosition() - goal).max() == 0.0          # the goal fields still hold the user's goals
 
 
+@needs_reference_library
 def test_motion_force_task_with_internal_otg_in_the_flagship_hierarchy():
     """config 2 with the reference's defaults: MotionForceTask (6-dof Cartesian generator, moving reference frame for the
     orientation) + JointTask (joint generator) through RobotController"""
@@ -172,3 +177,31 @@ def test_otg_on_off_round_trip_keeps_the_goals():
     assert np.abs(jt.getGoalPosition() - goal).max() == 0.0 and np.abs(jt.getDesiredPosition() - goal).max() == 0.0
     jt.enableInternalOtgAccelerationLimited(math.pi / 3, 2 * math.pi)
     assert np.abs(jt.getGoalPosition() - goal).max() == 0.0 and np.abs(jt.getDesiredPosition() - q).max() < 1e-12
+
+
+def test_joint_task_otg_reproduces_the_stored_reference_trajectory():
+    """tests/golden/otg_joints_reference.npz: the reference's vendored Ruckig under the JointTask defaults (acceleration
+    limited, pi/3 rad/s, 2 pi rad/s^2, 1 ms) with goal changes in mid-motion, replayed by the device's JointTask generator
+    cycle by cycle (tests/golden/generate_otg_reference.py wrote it)"""
+    import sai_primitives_b200 as sp
+    d = np.load(GOLD_OTG)
+    N, K, n = 3, d["pos"].shape[0], d["q0"].size
+    q = np.tile(d["q0"], (N, 1))
+    robot = sp.BatchedRobot("panda", N)
+    robot.setQ(q); robot.setDq(np.zeros((N, n))); robot.updateModel()
+    jt = sp.JointTask(robot)
+    ctrl = sp.RobotController(robot, [jt])
+    goal_at = {int(s): g for g, s in zip(d["goals"], d["goal_steps"])}
+    worst = 0.0
+    for k in range(K):
+        if k in goal_at:
+            jt.setGoalPosition(np.tile(goal_at[k], (N, 1)))
+        ctrl.updateControllerTaskModels()
+        ctrl.computeControlTorques()
+        p, v, a = jt.getDesiredPosition(), jt.getDesiredVelocity(), jt.getDesiredAcceleration()
+        worst = max(worst, np.abs(p - d["pos"][k]).max(), np.abs(v - d["vel"][k]).max(), 1e-3 * np.abs(a - d["acc"][k]).max())
+        assert worst < 1e-10, (k, worst)
+        robot.setQ(p); robot.setDq(v); robot.updateModel()      # the robots track the desired motion
+    flags = jt.getInternalOtgFlags()
+    assert (flags & sp.capi.OTG_GOAL_REACHED).all() and not (flags & sp.capi.OTG_ERROR).any()
+    assert (robot.status() & sp.capi.STATUS_UNHANDLED).sum() == 0
