@@ -123,6 +123,16 @@ protected:
 	void setBroadcast(int field, const double* v) { check(h(), osc_set_field(h(), _id, field, v, OSC_MEM_HOST, 1)); }
 	void setBatched(int field, const double* soa, osc_mem_kind where) { check(h(), osc_set_field(h(), _id, field, soa, where, 0)); }
 	void get(int field, double* soa, osc_mem_kind where) const { check(h(), osc_get_field(h(), _id, field, soa, where)); }
+	// osc_set_gains / osc_get_gains: broadcast (ncomp values each) or per robot (SoA ncomp x N each, host or device memory)
+	void setGainsBroadcast(int group, const double* kp, const double* kv, const double* ki) {
+		check(h(), osc_set_gains(h(), _id, group, kp, kv, ki, OSC_MEM_HOST, 0));
+	}
+	void setGainsBatched(int group, const double* kp, const double* kv, const double* ki, osc_mem_kind where) {
+		check(h(), osc_set_gains(h(), _id, group, kp, kv, ki, where, 1));
+	}
+	void getGainsBatched(int group, double* kp, double* kv, double* ki, osc_mem_kind where) const {
+		check(h(), osc_get_gains(h(), _id, group, kp, kv, ki, where));
+	}
 	std::shared_ptr<BatchedRobot> _robot;
 	std::string _task_name;
 	TaskType _task_type;
@@ -166,26 +176,18 @@ public:
 	void getGoalPosition(double* soa, osc_mem_kind where = OSC_MEM_HOST) const { get(OSC_JT_GOAL_POSITION, soa, where); }
 
 	void setGains(double kp, double kv, double ki = 0) {
-		osc_joint_params p = params();
-		for (int a = 0; a < _task_dof; a++) {
-			p.kp[a] = kp;
-			p.kv[a] = kv;
-			p.ki[a] = ki;
-		}
-		apply(p);
+		const std::vector<double> p(_task_dof, kp), v(_task_dof, kv), i(_task_dof, ki);
+		setGainsBroadcast(OSC_GAINS_JOINT, p.data(), v.data(), i.data());
 	}
 	void setGains(const std::vector<double>& kp, const std::vector<double>& kv, const std::vector<double>& ki) {
 		if (kp.size() == 1 && kv.size() == 1 && ki.size() == 1) return setGains(kp[0], kv[0], ki[0]);
 		if ((int)kp.size() != _task_dof || (int)kv.size() != _task_dof || (int)ki.size() != _task_dof)
 			throw std::invalid_argument("size of gain vectors inconsistent with number of task dofs in JointTask::setGains\n");
-		osc_joint_params p = params();
-		for (int a = 0; a < _task_dof; a++) {
-			p.kp[a] = kp[a];
-			p.kv[a] = kv[a];
-			p.ki[a] = ki[a];
-		}
-		apply(p);
+		setGainsBroadcast(OSC_GAINS_JOINT, kp.data(), kv.data(), ki.data());
 	}
+	// per robot: SoA k x N each (gain a of robot i at soa[a * N + i]), host or device memory
+	void setGains(const double* kp, const double* kv, const double* ki, osc_mem_kind where) { setGainsBatched(OSC_GAINS_JOINT, kp, kv, ki, where); }
+	void getGains(double* kp, double* kv, double* ki, osc_mem_kind where = OSC_MEM_HOST) const { getGainsBatched(OSC_GAINS_JOINT, kp, kv, ki, where); }
 	void setDynamicDecouplingType(DynamicDecouplingType type) {
 		osc_joint_params p = params();
 		p.dynamic_decoupling_type = type;
@@ -305,38 +307,23 @@ public:
 	// ---- gains and options
 	void setPosControlGains(double kp, double kv, double ki = 0) { setPosControlGains(Vec3{kp, kp, kp}, Vec3{kv, kv, kv}, Vec3{ki, ki, ki}); }
 	void setPosControlGains(const Vec3& kp, const Vec3& kv, const Vec3& ki = Vec3{0, 0, 0}) {
-		osc_mft_params p = params();
-		for (int k = 0; k < 3; k++) {
-			p.kp_pos[k] = kp[k];
-			p.kv_pos[k] = kv[k];
-			p.ki_pos[k] = ki[k];
-		}
-		apply(p);
+		setGainsBroadcast(OSC_GAINS_POSITION, kp.data(), kv.data(), ki.data());
 	}
 	void setOriControlGains(double kp, double kv, double ki = 0) { setOriControlGains(Vec3{kp, kp, kp}, Vec3{kv, kv, kv}, Vec3{ki, ki, ki}); }
 	void setOriControlGains(const Vec3& kp, const Vec3& kv, const Vec3& ki = Vec3{0, 0, 0}) {
-		osc_mft_params p = params();
-		for (int k = 0; k < 3; k++) {
-			p.kp_ori[k] = kp[k];
-			p.kv_ori[k] = kv[k];
-			p.ki_ori[k] = ki[k];
-		}
-		apply(p);
+		setGainsBroadcast(OSC_GAINS_ORIENTATION, kp.data(), kv.data(), ki.data());
 	}
-	void setForceControlGains(double kp, double kv, double ki) {
-		osc_mft_params p = params();
-		p.kp_force = kp;
-		p.kv_force = kv;
-		p.ki_force = ki;
-		apply(p);
-	}
-	void setMomentControlGains(double kp, double kv, double ki) {
-		osc_mft_params p = params();
-		p.kp_moment = kp;
-		p.kv_moment = kv;
-		p.ki_moment = ki;
-		apply(p);
-	}
+	void setForceControlGains(double kp, double kv, double ki) { setGainsBroadcast(OSC_GAINS_FORCE, &kp, &kv, &ki); }
+	void setMomentControlGains(double kp, double kv, double ki) { setGainsBroadcast(OSC_GAINS_MOMENT, &kp, &kv, &ki); }
+	// per robot: SoA 3 x N (position, orientation) or 1 x N (force, moment) each, host or device memory; getters likewise
+	void setPosControlGains(const double* kp, const double* kv, const double* ki, osc_mem_kind w) { setGainsBatched(OSC_GAINS_POSITION, kp, kv, ki, w); }
+	void setOriControlGains(const double* kp, const double* kv, const double* ki, osc_mem_kind w) { setGainsBatched(OSC_GAINS_ORIENTATION, kp, kv, ki, w); }
+	void setForceControlGains(const double* kp, const double* kv, const double* ki, osc_mem_kind w) { setGainsBatched(OSC_GAINS_FORCE, kp, kv, ki, w); }
+	void setMomentControlGains(const double* kp, const double* kv, const double* ki, osc_mem_kind w) { setGainsBatched(OSC_GAINS_MOMENT, kp, kv, ki, w); }
+	void getPosControlGains(double* kp, double* kv, double* ki, osc_mem_kind w = OSC_MEM_HOST) const { getGainsBatched(OSC_GAINS_POSITION, kp, kv, ki, w); }
+	void getOriControlGains(double* kp, double* kv, double* ki, osc_mem_kind w = OSC_MEM_HOST) const { getGainsBatched(OSC_GAINS_ORIENTATION, kp, kv, ki, w); }
+	void getForceControlGains(double* kp, double* kv, double* ki, osc_mem_kind w = OSC_MEM_HOST) const { getGainsBatched(OSC_GAINS_FORCE, kp, kv, ki, w); }
+	void getMomentControlGains(double* kp, double* kv, double* ki, osc_mem_kind w = OSC_MEM_HOST) const { getGainsBatched(OSC_GAINS_MOMENT, kp, kv, ki, w); }
 	void setFeedforwardForceGain(double k) { auto p = params(); p.kff_force = k; apply(p); }
 	void setFeedforwardmomentGain(double k) { auto p = params(); p.kff_moment = k; apply(p); }
 	void setMaxForceControlFeedbackOutput(double v) { auto p = params(); p.max_force_control_feedback_output = v; apply(p); }

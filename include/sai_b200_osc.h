@@ -286,6 +286,39 @@ int osc_joint_default_params(osc_joint_params* p);
 int osc_joint_get_params(const osc_handle* h, int task_id, osc_joint_params* p);
 int osc_joint_set_params(osc_handle* h, int task_id, const osc_joint_params* p);
 
+/* ---- per-robot control gains.  JointTask::setGains (JointTask.cpp), MotionForceTask::setPosControlGains /
+ * setOriControlGains / setForceControlGains / setMomentControlGains (MotionForceTask.cpp:581-628), each robot of the batch
+ * with its own values (gain sweeps, randomised gains, variable-impedance policies).  Components per robot (ncomp): joint k,
+ * position and orientation 3 (diagonal, world axes), force and moment 1.  Only these PID gains can be per robot; the
+ * feed-forward gains, the maximum feedback outputs, the saturation velocities, the bounded-inertia thresholds, the
+ * singularity handler's gains and bounds and the OTG limits stay broadcast parameters.
+ *   per_robot = 0: kp, kv, ki hold ncomp host values each, applied to every robot.
+ *   per_robot = 1: kp, kv, ki are SoA ncomp x n_robots each, host or device memory (mem_kind).  Device input is checked by a
+ *                  reduction kernel and the call synchronises the handle's stream.
+ * Every value of the three arrays is checked before anything is written: joint, position and orientation gains must be finite
+ * and >= 0, force and moment gains finite (the reference accepts any value there).  A violation returns
+ * OSC_ERR_INVALID_ARGUMENT and leaves the gains as they were.  (The finiteness check is the one difference from the gain update of
+ * osc_mft_set_params / osc_joint_set_params, which checks the sign only.)
+ * The first per_robot = 1 call on a task allocates its gain block (24 doubles per robot), fills it with the current broadcast
+ * gains of every group and then writes the given group; from then on the kernels read that task's gains from the block (there
+ * is no way back), a per_robot = 0 call writes the group for every robot, and osc_mft_set_params / osc_joint_set_params
+ * return OSC_ERR_STATE when a gain member differs from its current broadcast value (other members stay settable).  Before
+ * the first per_robot = 1 call, per_robot = 0 is the gain update osc_*_set_params makes; after it, osc_*_get_params keeps
+ * returning the broadcast gains the task had when it entered per-robot mode, and osc_get_gains is what the kernels use.
+ * osc_reinitialize_task leaves the gains alone.  While a task of the handle has per-robot gains, osc_compute_control_torques / osc_step return
+ * OSC_ERR_UNSUPPORTED in the FP32 mode.  Writes are ordered with the control cycles in the handle's stream like goal writes.
+ * osc_get_gains returns ncomp x n_robots per array in either mode. ---- */
+typedef enum {
+	OSC_GAINS_JOINT = 0,
+	OSC_GAINS_POSITION = 1,
+	OSC_GAINS_ORIENTATION = 2,
+	OSC_GAINS_FORCE = 3,
+	OSC_GAINS_MOMENT = 4
+} osc_gain_group;
+int osc_set_gains(osc_handle* h, int task_id, int group, const double* kp, const double* kv, const double* ki, int mem_kind,
+				  int per_robot);
+int osc_get_gains(osc_handle* h, int task_id, int group, double* kp, double* kv, double* ki, int mem_kind);
+
 /* ---- internal online trajectory generation (SURVEY.md row f-4).  The reference interpolates every task's goal with its
  * vendored Ruckig by default (JointTask.h:38-42, MotionForceTask.h:67-74): acceleration-limited, phase-synchronised.  Tasks are
  * created here with the generator OFF (BASELINE.json runs with it off, and so do the reference's examples that call

@@ -236,6 +236,48 @@ class _Task:
         _check(self._robot.handle, self._lib.osc_get_field(self._robot.handle, self.task_id, field, capi.host_ptr(out), capi.OSC_MEM_HOST))
         return out.T.copy()
 
+    def _set_gains(self, group, ncomp, kp, kv, ki, broadcast_form):
+        """osc_set_gains.  Each gain is a scalar or an (ncomp,) vector applied to every robot (what broadcast_form accepts, as
+        before per-robot gains existed: any array of 1 or ncomp values), or a 2-D (N, 1) / (N, ncomp) array with one row per robot.
+        When one of the three is per robot, the other two are expanded to every robot.  An array of 1 or ncomp values is always
+        the broadcast form, as it was before: with N == ncomp robots an (N, 1) array is read as ncomp per-component gains for every
+        robot, not as one gain per robot (pass (N, ncomp) then)."""
+        N = self._robot.n_robots
+        arrs = [np.asarray(x, dtype=np.float64) for x in (kp, kv, ki)]
+
+        def per_robot(a):
+            return a.ndim == 2 and a.shape[0] == N and a.shape[1] in (1, ncomp) and a.size not in (1, ncomp)
+
+        if not any(per_robot(a) for a in arrs):
+            vals = [np.ascontiguousarray(v, dtype=np.float64) for v in broadcast_form(*arrs)]
+            _check(self._robot.handle, self._lib.osc_set_gains(self._robot.handle, self.task_id, group, capi.host_ptr(vals[0]),
+                                                              capi.host_ptr(vals[1]), capi.host_ptr(vals[2]), capi.OSC_MEM_HOST, 0))
+            return
+        soa = []
+        for a in arrs:
+            if per_robot(a):
+                full = np.broadcast_to(a, (N, ncomp))
+            elif a.size in (1, ncomp):
+                full = np.broadcast_to(a.reshape(1, -1), (N, ncomp))
+            else:
+                raise ValueError("per-robot gains must have shape (%d, 1) or (%d, %d), or 1 or %d values for every robot; got %s"
+                                 % (N, N, ncomp, ncomp, a.shape))
+            soa.append(np.ascontiguousarray(full.T))
+        _check(self._robot.handle, self._lib.osc_set_gains(self._robot.handle, self.task_id, group, capi.host_ptr(soa[0]),
+                                                          capi.host_ptr(soa[1]), capi.host_ptr(soa[2]), capi.OSC_MEM_HOST, 1))
+
+    def _set_gains_device(self, group, kp_ptr, kv_ptr, ki_ptr):
+        """per-robot gains from device memory, SoA [ncomp, N] each (zero copy, like BatchedRobot.setStateDevice)"""
+        _check(self._robot.handle, self._lib.osc_set_gains(self._robot.handle, self.task_id, group, C.c_void_p(kp_ptr), C.c_void_p(kv_ptr),
+                                                          C.c_void_p(ki_ptr), capi.OSC_MEM_DEVICE, 1))
+
+    def _get_gains(self, group, ncomp):
+        N = self._robot.n_robots
+        out = [np.zeros((ncomp, N)) for _ in range(3)]
+        _check(self._robot.handle, self._lib.osc_get_gains(self._robot.handle, self.task_id, group, capi.host_ptr(out[0]),
+                                                          capi.host_ptr(out[1]), capi.host_ptr(out[2]), capi.OSC_MEM_HOST))
+        return tuple(o.T.copy() for o in out)
+
     def reInitializeTask(self):
         _check(self._robot.handle, self._lib.osc_reinitialize_task(self._robot.handle, self.task_id))
 
@@ -303,16 +345,26 @@ class JointTask(_Task):
     def getDesiredAcceleration(self): return self._get(capi.JT_DESIRED_ACCELERATION)
 
     def setGains(self, kp, kv, ki=0.0):
-        kp, kv, ki = (np.atleast_1d(np.asarray(x, dtype=np.float64)) for x in (kp, kv, ki))
+        """JointTask::setGains; also per robot: (N, 1) or (N, k) arrays (see _Task._set_gains)"""
         k = self._task_dof
-        if kp.size == 1 and kv.size == 1 and ki.size == 1:
-            kp, kv, ki = np.full(k, kp[0]), np.full(k, kv[0]), np.full(k, ki[0])
-        if kp.size != k or kv.size != k or ki.size != k:
-            raise ValueError("size of gain vectors inconsistent with number of task dofs in JointTask::setGains")
-        p = self._params()
-        for a in range(k):
-            p.kp[a], p.kv[a], p.ki[a] = kp[a], kv[a], ki[a]
-        self._apply(p)
+
+        def broadcast_form(kp, kv, ki):
+            kp, kv, ki = (np.atleast_1d(x).ravel() for x in (kp, kv, ki))
+            if kp.size == 1 and kv.size == 1 and ki.size == 1:
+                kp, kv, ki = np.full(k, kp[0]), np.full(k, kv[0]), np.full(k, ki[0])
+            if kp.size != k or kv.size != k or ki.size != k:
+                raise ValueError("size of gain vectors inconsistent with number of task dofs in JointTask::setGains")
+            return kp, kv, ki
+
+        self._set_gains(capi.GAINS_JOINT, k, kp, kv, ki, broadcast_form)
+
+    def setGainsDevice(self, kp_ptr, kv_ptr, ki_ptr):
+        """per-robot gains from device memory: SoA [k, N] each"""
+        self._set_gains_device(capi.GAINS_JOINT, kp_ptr, kv_ptr, ki_ptr)
+
+    def getGains(self):
+        """(kp, kv, ki), each [N, k]"""
+        return self._get_gains(capi.GAINS_JOINT, self._task_dof)
 
     def setDynamicDecouplingType(self, t):
         p = self._params(); p.dynamic_decoupling_type = int(t); self._apply(p)
@@ -458,19 +510,37 @@ class MotionForceTask(_Task):
             raise ValueError("gains should be of size 1 or 3 in MotionForceTask::%s" % what)
         return kp, kv, ki
 
+    @staticmethod
+    def _g1(kp, kv, ki, what):
+        vals = [np.asarray(x, dtype=np.float64) for x in (kp, kv, ki)]
+        if any(v.size != 1 for v in vals):
+            raise ValueError("gains should be scalars in MotionForceTask::%s" % what)
+        return [v.reshape(1) for v in vals]
+
+    # MotionForceTask::set*ControlGains; also per robot: (N, 1) or (N, 3) arrays (see _Task._set_gains)
     def setPosControlGains(self, kp, kv, ki=0.0):
-        kp, kv, ki = self._g3(kp, kv, ki, "setPosControlGains")
-        p = self._params(); p.kp_pos[:] = list(kp); p.kv_pos[:] = list(kv); p.ki_pos[:] = list(ki); self._apply(p)
+        self._set_gains(capi.GAINS_POSITION, 3, kp, kv, ki, lambda a, b, c: self._g3(a, b, c, "setPosControlGains"))
 
     def setOriControlGains(self, kp, kv, ki=0.0):
-        kp, kv, ki = self._g3(kp, kv, ki, "setOriControlGains")
-        p = self._params(); p.kp_ori[:] = list(kp); p.kv_ori[:] = list(kv); p.ki_ori[:] = list(ki); self._apply(p)
+        self._set_gains(capi.GAINS_ORIENTATION, 3, kp, kv, ki, lambda a, b, c: self._g3(a, b, c, "setOriControlGains"))
 
     def setForceControlGains(self, kp, kv, ki):
-        p = self._params(); p.kp_force, p.kv_force, p.ki_force = kp, kv, ki; self._apply(p)
+        self._set_gains(capi.GAINS_FORCE, 1, kp, kv, ki, lambda a, b, c: self._g1(a, b, c, "setForceControlGains"))
 
     def setMomentControlGains(self, kp, kv, ki):
-        p = self._params(); p.kp_moment, p.kv_moment, p.ki_moment = kp, kv, ki; self._apply(p)
+        self._set_gains(capi.GAINS_MOMENT, 1, kp, kv, ki, lambda a, b, c: self._g1(a, b, c, "setMomentControlGains"))
+
+    # per-robot gains from device memory: SoA [3, N] (position, orientation) or [1, N] (force, moment) each
+    def setPosControlGainsDevice(self, kp_ptr, kv_ptr, ki_ptr): self._set_gains_device(capi.GAINS_POSITION, kp_ptr, kv_ptr, ki_ptr)
+    def setOriControlGainsDevice(self, kp_ptr, kv_ptr, ki_ptr): self._set_gains_device(capi.GAINS_ORIENTATION, kp_ptr, kv_ptr, ki_ptr)
+    def setForceControlGainsDevice(self, kp_ptr, kv_ptr, ki_ptr): self._set_gains_device(capi.GAINS_FORCE, kp_ptr, kv_ptr, ki_ptr)
+    def setMomentControlGainsDevice(self, kp_ptr, kv_ptr, ki_ptr): self._set_gains_device(capi.GAINS_MOMENT, kp_ptr, kv_ptr, ki_ptr)
+
+    # (kp, kv, ki), each [N, 3] or [N, 1]
+    def getPosControlGains(self): return self._get_gains(capi.GAINS_POSITION, 3)
+    def getOriControlGains(self): return self._get_gains(capi.GAINS_ORIENTATION, 3)
+    def getForceControlGains(self): return self._get_gains(capi.GAINS_FORCE, 1)
+    def getMomentControlGains(self): return self._get_gains(capi.GAINS_MOMENT, 1)
 
     def setFeedforwardForceGain(self, k):
         p = self._params(); p.kff_force = k; self._apply(p)

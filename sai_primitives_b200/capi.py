@@ -93,6 +93,12 @@ OTG_BAD_FINISH = 8
 TASK_NULLSPACE = 48
 TASK_PREVIOUS_NULLSPACE = 49
 TASK_AND_PREVIOUS_NULLSPACE = 50
+# osc_gain_group
+GAINS_JOINT = 0
+GAINS_POSITION = 1
+GAINS_ORIENTATION = 2
+GAINS_FORCE = 3
+GAINS_MOMENT = 4
 
 D = C.c_double
 I32 = C.c_int32
@@ -218,6 +224,8 @@ SYMBOLS = {
     "osc_set_precision": (C.c_int, [_H, C.c_int]),
     "osc_get_precision": (C.c_int, [_H]),
     "osc_sim_integrate": (C.c_int, [_H, _PD, _PD, _PD, C.c_double, C.c_int, C.c_int]),
+    "osc_set_gains": (C.c_int, [_H, C.c_int, C.c_int, _PD, _PD, _PD, C.c_int, C.c_int]),
+    "osc_get_gains": (C.c_int, [_H, C.c_int, C.c_int, _PD, _PD, _PD, C.c_int]),
     "osc_eval_model": (C.c_int, [_H, C.c_int, C.POINTER(LinkFrame), C.POINTER(D), _PD, _PD, _PD, _PD, _PD, C.c_int]),
 }
 

@@ -117,6 +117,11 @@ cudaError_t launch_copy(double* st, int64_t NR, int dst, int src, int ncomp, cud
 	copy_components_kernel<<<grid_for(NR, 256), 256, 0, stream>>>(st, NR, dst, src, ncomp);
 	return cudaGetLastError();
 }
+cudaError_t launch_check_values(const double* v, int64_t n, int32_t* bad, cudaStream_t stream) {
+	const int64_t want = (n + 255) / 256;
+	check_values_kernel<<<(unsigned)(want < 1024 ? (want > 0 ? want : 1) : 1024), 256, 0, stream>>>(v, n, bad);
+	return cudaGetLastError();
+}
 cudaError_t launch_fill_int(int32_t* ist, int64_t NR, int comp, int ncomp, int32_t value, cudaStream_t stream) {
 	fill_int_components_kernel<<<grid_for(NR, 256), 256, 0, stream>>>(ist, NR, comp, ncomp, value);
 	return cudaGetLastError();

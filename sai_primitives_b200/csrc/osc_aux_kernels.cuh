@@ -23,6 +23,19 @@ __global__ void copy_components_kernel(double* st, int64_t NR, int dst, int src,
 	if (i >= NR) return;
 	for (int c = 0; c < ncomp; c++) ST(dst, c) = ST(src, c);
 }
+// Validation of caller values in device memory (osc_set_gains): *bad |= 1 if any of the n values is not finite, |= 2 if any is
+// negative.  Grid-stride, one atomic per warp that found something.
+__global__ void check_values_kernel(const double* v, int64_t n, int32_t* bad) {
+	int32_t f = 0;
+	for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
+		const double x = v[k];
+		if (!isfinite(x)) f |= 1;
+		else if (x < 0.0) f |= 2;
+	}
+#pragma unroll
+	for (int o = 16; o > 0; o >>= 1) f |= __shfl_xor_sync(0xffffffffu, f, o);
+	if (f && (threadIdx.x & 31) == 0) atomicOr(bad, f);
+}
 __global__ void fill_int_components_kernel(int32_t* ist, int64_t NR, int comp, int ncomp, int32_t value) {
 	const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= NR) return;

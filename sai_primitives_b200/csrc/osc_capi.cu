@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -54,6 +55,7 @@ struct osc_handle {
 	double* d_scratch = nullptr;  // output of the on-request observers (osc_observers.cuh)
 	size_t scratch_doubles = 0;
 	int32_t* h_seen = nullptr;	// mapped pinned: hand-over count of the last completed cycle
+	int32_t* d_check = nullptr;	// result word of the device-input validation of osc_set_gains
 	int clean_cycles = 0;
 	int blend_split = -1;  // split blending path: -1 not decided, 0 off (SAI_B200_BLEND_SPLIT=0 or no memory), 1 allocate when needed, 2 allocated
 	int64_t blend_split_min = 0;  // hand-over count (host hint) from which the split path is used
@@ -749,6 +751,8 @@ int osc_mft_set_params(osc_handle* h, int task_id, const osc_mft_params* p) {
 		return fail(h, OSC_ERR_INVALID_ARGUMENT, "closed loop flags must be changed with osc_mft_set_closed_loop_*");
 	if (p->passivity_enabled != c.passivity_enabled)
 		return fail(h, OSC_ERR_INVALID_ARGUMENT, "passivity must be changed with osc_mft_enable_passivity");
+	if (t.gains && std::memcmp(p, &c, GAIN_COUNT * sizeof(double)) != 0)
+		return fail(h, OSC_ERR_STATE, "this task's gains are per robot: change them with osc_set_gains");
 	t.p = *p;
 	return OSC_OK;
 }
@@ -961,8 +965,162 @@ int osc_joint_set_params(osc_handle* h, int task_id, const osc_joint_params* p) 
 	}
 	if (p->dynamic_decoupling_type < 0 || p->dynamic_decoupling_type > 2)
 		return fail(h, OSC_ERR_INVALID_ARGUMENT, "Dynamic decoupling type not recognized in JointTask::updateTaskModel");
+	if (t.gains) {
+		for (int a = 0; a < t.k; a++)
+			if (p->kp[a] != t.p.kp[a] || p->kv[a] != t.p.kv[a] || p->ki[a] != t.p.ki[a])
+				return fail(h, OSC_ERR_STATE, "this task's gains are per robot: change them with osc_set_gains");
+	}
 	t.p = *p;
 	if (t.p.bie_threshold < 0) t.p.bie_threshold = 0;  // JointTask.h:372-378
+	return OSC_OK;
+}
+
+// ---- per-robot gains (osc_set_gains / osc_get_gains) ----
+// The first GAIN_COUNT doubles of both parameter structs have the layout of the gain block (GainComp).
+static_assert(offsetof(osc_mft_params, kp_pos) == 0 && offsetof(osc_mft_params, kp_ori) == MG_KP_ORI * sizeof(double) &&
+				  offsetof(osc_mft_params, kp_force) == MG_KP_FORCE * sizeof(double) &&
+				  offsetof(osc_mft_params, ki_moment) == MG_KI_MOMENT * sizeof(double),
+			  "osc_mft_params gains out of step with GainComp");
+static_assert(offsetof(osc_joint_params, kp) == JG_KP * sizeof(double) && offsetof(osc_joint_params, kv) == JG_KV * sizeof(double) &&
+				  offsetof(osc_joint_params, ki) == JG_KI * sizeof(double),
+			  "osc_joint_params gains out of step with GainComp");
+
+namespace {
+struct GainGroup {
+	double* params;	 // first GAIN_COUNT doubles of the task's broadcast parameters
+	double** block;	 // the task's gain-block pointer
+	int comp[3];	 // first block component of kp, kv, ki
+	int ncomp;
+	bool nonneg;	 // gains must be >= 0 (joint, position, orientation)
+	const char* msg;
+};
+int gain_group(osc_handle* h, int task_id, int group, GainGroup& g) {
+	if (group < OSC_GAINS_JOINT || group > OSC_GAINS_MOMENT) return fail(h, OSC_ERR_INVALID_ARGUMENT, "unknown gain group");
+	int rc = check_task(h, task_id, group == OSC_GAINS_JOINT ? OSC_TASK_JOINT : OSC_TASK_MOTION_FORCE);
+	if (rc != OSC_OK) return rc;
+	const int idx = h->tasks[task_id].index;
+	if (group == OSC_GAINS_JOINT) {
+		DevJt& t = h->prog.jt[idx];
+		g = {reinterpret_cast<double*>(&t.p), &t.gains, {JG_KP, JG_KV, JG_KI}, t.k, true, "gains must be positive or zero in JointTask::setGains"};
+		return OSC_OK;
+	}
+	DevMft& t = h->prog.mft[idx];
+	g.params = reinterpret_cast<double*>(&t.p);
+	g.block = &t.gains;
+	switch (group) {
+		case OSC_GAINS_POSITION:
+			g = {g.params, g.block, {MG_KP_POS, MG_KV_POS, MG_KI_POS}, 3, true, "all gains should be positive or zero in MotionForceTask::setPosControlGains"};
+			break;
+		case OSC_GAINS_ORIENTATION:
+			g = {g.params, g.block, {MG_KP_ORI, MG_KV_ORI, MG_KI_ORI}, 3, true, "all gains should be positive or zero in MotionForceTask::setOriControlGains"};
+			break;
+		case OSC_GAINS_FORCE:
+			g = {g.params, g.block, {MG_KP_FORCE, MG_KV_FORCE, MG_KI_FORCE}, 1, false, "force control gains must be finite"};
+			break;
+		default:
+			g = {g.params, g.block, {MG_KP_MOMENT, MG_KV_MOMENT, MG_KI_MOMENT}, 1, false, "moment control gains must be finite"};
+	}
+	return OSC_OK;
+}
+// 0: all finite (and >= 0 where required), else the message's error
+int check_gain_values(osc_handle* h, const GainGroup& g, int32_t flags) {
+	if (flags & 1) return fail(h, OSC_ERR_INVALID_ARGUMENT, g.nonneg ? std::string(g.msg) + " (non-finite value)" : std::string(g.msg));
+	if ((flags & 2) && g.nonneg) return fail(h, OSC_ERR_INVALID_ARGUMENT, g.msg);
+	return OSC_OK;
+}
+int32_t host_value_flags(const double* v, size_t n) {
+	int32_t f = 0;
+	for (size_t k = 0; k < n; k++) {
+		if (!std::isfinite(v[k])) f |= 1;
+		else if (v[k] < 0.0) f |= 2;
+	}
+	return f;
+}
+}  // namespace
+
+int osc_set_gains(osc_handle* h, int task_id, int group, const double* kp, const double* kv, const double* ki, int mem_kind, int per_robot) {
+	ENTER(h);
+	GainGroup g;
+	int rc = gain_group(h, task_id, group, g);
+	if (rc != OSC_OK) return rc;
+	if (!kp || !kv || !ki) return fail(h, OSC_ERR_INVALID_ARGUMENT, "null gains");
+	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
+	const double* src[3] = {kp, kv, ki};
+	const int64_t NR = h->NR;
+	if (!per_robot) {
+		if (mem_kind != OSC_MEM_HOST) return fail(h, OSC_ERR_INVALID_ARGUMENT, "broadcast values must be in host memory");
+		int32_t f = 0;
+		for (int a = 0; a < 3; a++) f |= host_value_flags(src[a], (size_t)g.ncomp);
+		if ((rc = check_gain_values(h, g, f)) != OSC_OK) return rc;
+		for (int a = 0; a < 3; a++) {
+			if (*g.block) {
+				CUDA_TRY(h, osc::launch_fill(*g.block, NR, g.comp[a], g.ncomp, src[a], h->stream));
+				h->launches++;
+			} else {
+				std::memcpy(g.params + g.comp[a], src[a], (size_t)g.ncomp * sizeof(double));
+			}
+		}
+		return OSC_OK;
+	}
+	// per robot: every value is checked before anything is written
+	const size_t n = (size_t)g.ncomp * (size_t)NR;
+	int32_t f = 0;
+	if (mem_kind == OSC_MEM_HOST) {
+		for (int a = 0; a < 3; a++) f |= host_value_flags(src[a], n);
+	} else {
+		if (!h->d_check) {
+			rc = dev_alloc(h, &h->d_check, 1, false);
+			if (rc != OSC_OK) return rc;
+		}
+		CUDA_TRY(h, cudaMemsetAsync(h->d_check, 0, sizeof(int32_t), h->stream));
+		for (int a = 0; a < 3; a++) {
+			CUDA_TRY(h, osc::launch_check_values(src[a], (int64_t)n, h->d_check, h->stream));
+			h->launches++;
+		}
+		CUDA_TRY(h, cudaMemcpyAsync(&f, h->d_check, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+		CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+	}
+	if ((rc = check_gain_values(h, g, f)) != OSC_OK) return rc;
+	if (!*g.block) {
+		// entering per-robot mode: every group of the block starts from the current broadcast values
+		double* blk = nullptr;
+		rc = dev_alloc(h, &blk, (size_t)GAIN_COUNT * NR, false);
+		if (rc != OSC_OK) return rc;
+		CUDA_TRY(h, osc::launch_fill(blk, NR, 0, 16, g.params, h->stream));
+		CUDA_TRY(h, osc::launch_fill(blk, NR, 16, GAIN_COUNT - 16, g.params + 16, h->stream));
+		h->launches += 2;
+		*g.block = blk;
+	}
+	for (int a = 0; a < 3; a++)
+		CUDA_TRY(h, cudaMemcpyAsync(*g.block + (size_t)g.comp[a] * NR, src[a], n * sizeof(double),
+									mem_kind == OSC_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, h->stream));
+	if (mem_kind == OSC_MEM_HOST) CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+	return OSC_OK;
+}
+
+int osc_get_gains(osc_handle* h, int task_id, int group, double* kp, double* kv, double* ki, int mem_kind) {
+	ENTER(h);
+	GainGroup g;
+	int rc = gain_group(h, task_id, group, g);
+	if (rc != OSC_OK) return rc;
+	if (!kp || !kv || !ki) return fail(h, OSC_ERR_INVALID_ARGUMENT, "null output");
+	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
+	double* dst[3] = {kp, kv, ki};
+	const int64_t NR = h->NR;
+	const size_t n = (size_t)g.ncomp * (size_t)NR;
+	for (int a = 0; a < 3; a++) {
+		if (*g.block) {
+			CUDA_TRY(h, cudaMemcpyAsync(dst[a], *g.block + (size_t)g.comp[a] * NR, n * sizeof(double),
+										mem_kind == OSC_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, h->stream));
+		} else if (mem_kind == OSC_MEM_DEVICE) {
+			CUDA_TRY(h, osc::launch_fill(dst[a], NR, 0, g.ncomp, g.params + g.comp[a], h->stream));
+			h->launches++;
+		} else {
+			for (int c = 0; c < g.ncomp; c++)
+				for (int64_t i = 0; i < NR; i++) dst[a][(size_t)c * NR + i] = g.params[g.comp[a] + c];
+		}
+	}
+	if (mem_kind == OSC_MEM_HOST) CUDA_TRY(h, cudaStreamSynchronize(h->stream));
 	return OSC_OK;
 }
 
@@ -1211,6 +1369,9 @@ static int run_cycle(osc_handle* h, double* tau_out, int mem_kind, bool sync_hos
 		if (!(h->sig_R == 6 && h->prog.mft[0].full && osc::cycle_spec_eligible(h->prog, h->sig_jt, &motion) && motion && osc::fused_f32_available(h->model.n)))
 			return fail(h, OSC_ERR_UNSUPPORTED,
 						"FP32 mode covers a full six-dof MotionForceTask under pure motion control (alone or with a full JointTask) on an all-revolute-z chain only");
+		for (int k = 0; k < 2; k++)
+			if (h->prog.mft[k].gains || h->prog.jt[k].gains)
+				return fail(h, OSC_ERR_UNSUPPORTED, "FP32 mode: the kernels have no single-precision form with per-robot gains (osc_set_gains)");
 	}
 	h->prog.tau = (mem_kind == OSC_MEM_DEVICE) ? tau_out : h->d_tau;
 	h->prog.update_models = h->models_armed ? 1 : 0;

@@ -131,8 +131,9 @@ DEVI void reduce_task_vector(const DevMft& t, const double (&v6)[6], double (&y)
 
 // One bulk prefetch (cp.async.bulk.prefetch.L2) per state component for the robots of block `blk`: they are contiguous
 // in every component row, so thread k asks for row k of the list below -- one instruction per thread instead of one
-// prefetch per thread and component.
-template <int N, int R, bool HAS_JT>
+// prefetch per thread and component.  MG > 0 (per-robot gains): also the first MG rows of the motion-force task's gain block
+// and the joint task's 3 N gain rows (at most 2 N + 31 + 4 N + 24 + 3 N = 127 rows for eight joints).
+template <int N, int R, bool HAS_JT, int MG = 0>
 DEVI void prefetch_block_rows(const OscProgram& P, uint64_t blk) {
 	const uint64_t nrl = (uint64_t)P.n_robots;
 	const uint64_t b0 = blk * blockDim.x;
@@ -160,6 +161,17 @@ DEVI void prefetch_block_rows(const OscProgram& P, uint64_t blk) {
 				const int grp = k / N, c = k - grp * N;
 				const int comp = (grp == 0 ? JC_GOAL_POS : grp == 1 ? JC_GOAL_VEL : grp == 2 ? JC_GOAL_ACC : JC_INT) + c;
 				row = (const char*)(jt.st + (uint64_t)comp * nrl);
+			}
+			if constexpr (MG > 0) k -= 4 * N;
+		}
+		if constexpr (MG > 0 && R > 0) {
+			if (k >= 0 && k < MG && P.mft[0].gains) row = (const char*)(P.mft[0].gains + (uint64_t)k * nrl);
+			k -= MG;
+		}
+		if constexpr (MG > 0 && HAS_JT) {
+			if (k >= 0 && k < 3 * N && P.jt[0].gains) {
+				const int grp = k / N, c = k - grp * N;
+				row = (const char*)(P.jt[0].gains + (uint64_t)((grp == 0 ? JG_KP : grp == 1 ? JG_KV : JG_KI) + c) * nrl);
 			}
 		}
 	}
@@ -219,7 +231,10 @@ DEVI void park_for_blend(const OscProgram& P, int slot, int64_t i, const double 
 // law (partial tasks, force / moment spaces, closed loops, POPC) on top of the same rolled kinematics.
 // PARK (full six-dof task only): hand-overs also leave kinematics and dynamics in the scratch block of the split blending path
 // (osc_blend.cuh); a separate instantiation, because compiled into the kernel of the headline it costs 6 registers and 0.7 %.
-template <int N, int R, bool HAS_JT, bool FULL, bool SPEC = false, bool GRAV = false, bool MOTION = SPEC, bool PARK = false>
+// PRG (with SPEC, or for a JointTask alone): a task of the launch carries per-robot PID gains (osc_set_gains), read from its gain block in global
+// memory (a task without a block: its parameters); the instantiations without it read the broadcast parameters (SPEC) or test
+// the block pointer at run time (the others).
+template <int N, int R, bool HAS_JT, bool FULL, bool SPEC = false, bool GRAV = false, bool MOTION = SPEC, bool PARK = false, bool PRG = false>
 __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(const __grid_constant__ OscProgram P) {
 	extern __shared__ double sm[];
 	// Programmatic dependent launch on both sides: the general-path kernel of this cycle may be scheduled into whatever
@@ -248,8 +263,15 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 	// in the middle of the control law cannot be hidden with two warps per scheduler, and a block that was scheduled
 	// while the previous kernel of the stream is still running (programmatic dependent launch) uses the wait for it.
 	// Prefetches are safe ahead of griddepcontrol.wait: they only move lines into L2, which stays coherent.
+	static_assert(!PRG || SPEC || R == 0, "per-robot gain instantiations: the specialised ones and the joint task alone");
+	// where the control laws read the gains: a JointTask alone (R = 0) has a per-robot instantiation like the specialised kernels,
+	// the other non-specialised instantiations test the block pointer at run time
+	constexpr int G = PRG ? GAINS_ROBOT : (SPEC || R == 0) ? GAINS_BCAST : GAINS_ANY;
 #ifndef OSC_NO_PREFETCH
-	prefetch_block_rows<N, R, HAS_JT>(P, blockIdx.x);
+	if constexpr (PRG)
+		prefetch_block_rows<N, R, HAS_JT, MOTION ? MG_KP_FORCE : GAIN_COUNT>(P, blockIdx.x);
+	else
+		prefetch_block_rows<N, R, HAS_JT>(P, blockIdx.x);
 #endif
 	grid_dependency_wait(P);
 	stamp_block(P, 0);
@@ -292,7 +314,7 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 			double dq[N];
 #pragma unroll
 			for (int j = 0; j < N; j++) dq[j] = P.dq[(IDX)j * NR + i];
-			joint_control_law<N, N>(t, NR, i, q, dq, pid, acc);
+			joint_control_law<N, N, false, IDX, G>(t, NR, i, q, dq, pid, acc);
 		}
 #pragma unroll
 		for (int r = 0; r < N; r++) {
@@ -495,7 +517,7 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 			double fstar[6] = {0, 0, 0, 0, 0, 0}, F[6] = {0, 0, 0, 0, 0, 0};
 			has_F = true;
 			if (alive)
-				has_F = mft_control_law<MOTION>(t, NR, i, x, Rc, v, w, P.write_observers != 0, fstar, F, status,
+				has_F = mft_control_law<MOTION, IDX, G>(t, NR, i, x, Rc, v, w, P.write_observers != 0, fstar, F, status,
 												MOTION ? smt + (size_t)(kSmFactor<N> + N * R) * sms : nullptr, sms);
 			reduce_task_vector<R, FULL>(t, fstar, yf);
 			reduce_task_vector<R, FULL>(t, F, yF);
@@ -638,7 +660,7 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 #pragma unroll
 				for (int j = 0; j < N; j++) pid[j] = acc[j] = 0.0;
 				if constexpr (SPEC) {
-					if (alive) joint_control_law_staged<N>(jt, NR, i, smt + (size_t)kSmFactor<N> * sms, sms, pid, acc);
+					if (alive) joint_control_law_staged<N, IDX, G>(jt, NR, i, smt + (size_t)kSmFactor<N> * sms, sms, pid, acc);
 				} else if (alive) {
 					double qj[N], dqj[N];  // re-read (L2 hot) rather than kept live across the task above
 #pragma unroll

@@ -39,7 +39,7 @@ static int sm_count() {
 	return v;
 }
 
-template <int N, int R, bool JT, bool FULL, bool SPEC = false, bool GRAV = false, bool MOTION = SPEC, bool PARK = false>
+template <int N, int R, bool JT, bool FULL, bool SPEC = false, bool GRAV = false, bool MOTION = SPEC, bool PARK = false, bool PRG = false>
 static cudaError_t launch_variant(const OscProgram& P, cudaStream_t stream) {
 	const unsigned grid = (unsigned)((P.n_robots + kCycleBlock - 1) / kCycleBlock);
 	constexpr int smem = cycle_smem_doubles<N, R, SPEC, MOTION>() * kCycleBlock * (int)sizeof(double);
@@ -49,7 +49,7 @@ static cudaError_t launch_variant(const OscProgram& P, cudaStream_t stream) {
 	int dev = 0;
 	cudaGetDevice(&dev);
 	if (dev < 0 || dev >= 64 || !configured[dev].load(std::memory_order_acquire)) {
-		cudaError_t e = cudaFuncSetAttribute(osc_cycle_kernel<N, R, JT, FULL, SPEC, GRAV, MOTION, PARK>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+		cudaError_t e = cudaFuncSetAttribute(osc_cycle_kernel<N, R, JT, FULL, SPEC, GRAV, MOTION, PARK, PRG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
 		if (e != cudaSuccess) return e;
 		if (dev >= 0 && dev < 64) configured[dev].store(true, std::memory_order_release);
 	}
@@ -73,7 +73,7 @@ static cudaError_t launch_variant(const OscProgram& P, cudaStream_t stream) {
 		attr[0].val.programmaticStreamSerializationAllowed = 1;
 		cfg.attrs = attr;
 		cfg.numAttrs = 1;
-		cudaError_t e = cudaLaunchKernelEx(&cfg, osc_cycle_kernel<N, R, JT, FULL, SPEC, GRAV, MOTION, PARK>, P);
+		cudaError_t e = cudaLaunchKernelEx(&cfg, osc_cycle_kernel<N, R, JT, FULL, SPEC, GRAV, MOTION, PARK, PRG>, P);
 		if (e != cudaSuccess) return e;
 	}
 #if defined(OSC_TRACE)
@@ -100,12 +100,25 @@ static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
 		const bool spec = cycle_spec_eligible(P, JT, &motion);
 		// with many robots on the general path the hand-overs also park their kinematics and dynamics for the split blending path
 		const bool park = P.mft[0].full && blend_split_selected(P);
+		const bool prg = cycle_per_robot_gains(P, JT);
 		if (P.precision_fp32) {
 			// optional single-precision mode: only the specialised pure-motion kernel has an FP32 instantiation (osc_cycle_f32.cu)
 			if (!(P.mft[0].full && spec && motion)) return cudaErrorNotSupported;
 			e0 = launch_cycle_fused_f32(N, JT, P, stream);
 		} else if (!P.mft[0].full)
 			e0 = launch_variant<N, R, JT, false>(P, stream);
+		else if (prg && cycle_prg_specialised(R, spec, motion)) {
+			// per-robot gains: the pure-motion specialisation has its own instantiations (the others test the pointer at run time)
+			if (!park)
+				e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, true, false, true>(P, stream)
+									: launch_variant<N, R, JT, true, true, false, true, false, true>(P, stream);
+			else
+				e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, true, true, true>(P, stream)
+									: launch_variant<N, R, JT, true, true, false, true, true, true>(P, stream);
+		} else if (prg && !park)
+			e0 = launch_variant<N, R, JT, true>(P, stream);
+		else if (prg)
+			e0 = launch_variant<N, R, JT, true, false, false, false, true>(P, stream);
 		else if (spec && motion && !park)
 			e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true>(P, stream) : launch_variant<N, R, JT, true, true, false>(P, stream);
 		else if (spec && motion)
@@ -121,10 +134,17 @@ static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
 	} else if constexpr (R == 3) {
 		// the other common shape: three controlled directions (position only, or a planar task), any control law
 		bool motion = false;
-		if (cycle_spec_eligible(P, JT, &motion))
+		const bool spec = cycle_spec_eligible(P, JT, &motion);
+		if (spec && cycle_per_robot_gains(P, JT) && cycle_prg_specialised(R, spec, motion))
+			e0 = P.gravity_comp ? launch_variant<N, R, JT, false, true, true, false, false, true>(P, stream)
+								: launch_variant<N, R, JT, false, true, false, false, false, true>(P, stream);
+		else if (spec)
 			e0 = P.gravity_comp ? launch_variant<N, R, JT, false, true, true, false>(P, stream) : launch_variant<N, R, JT, false, true, false, false>(P, stream);
 		else
 			e0 = launch_variant<N, R, JT, false>(P, stream);
+	} else if constexpr (R == 0) {
+		// a JointTask alone: per-robot gains have their own instantiation, the broadcast one reads the parameters
+		e0 = cycle_per_robot_gains(P, JT) ? launch_variant<N, R, JT, false, false, false, false, false, true>(P, stream) : launch_variant<N, R, JT, false>(P, stream);
 	} else {
 		e0 = launch_variant<N, R, JT, false>(P, stream);
 	}

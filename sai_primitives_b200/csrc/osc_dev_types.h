@@ -58,6 +58,17 @@ enum MftIntComp : int {
 
 enum JtComp : int { JC_GOAL_POS = 0, JC_GOAL_VEL = 8, JC_GOAL_ACC = 16, JC_INT = 24, JC_COUNT = 32 };
 
+// SoA layout of a task's per-robot gain block (osc_set_gains), GAIN_COUNT x N.  A MotionForceTask uses every component, a
+// JointTask of dof k the components JG_KP.. JG_KP + k - 1 and the same of JG_KV, JG_KI.
+enum GainComp : int {
+	MG_KP_POS = 0, MG_KV_POS = 3, MG_KI_POS = 6,  // 3 each
+	MG_KP_ORI = 9, MG_KV_ORI = 12, MG_KI_ORI = 15,
+	MG_KP_FORCE = 18, MG_KV_FORCE = 19, MG_KI_FORCE = 20,
+	MG_KP_MOMENT = 21, MG_KV_MOMENT = 22, MG_KI_MOMENT = 23,
+	JG_KP = 0, JG_KV = 8, JG_KI = 16,  // OSC_MAX_DOF each
+	GAIN_COUNT = 24
+};
+
 #define OSC_HIST_MAX 256
 
 struct DevModel {
@@ -101,6 +112,7 @@ struct DevMft {
 	double* st;	   // MC_COUNT x N
 	int32_t* ist;  // MI_COUNT x N
 	double* ring;  // ring_capacity x N (or null)
+	double* gains;	// per-robot PID gains, GAIN_COUNT x N (osc_set_gains); null: every robot uses those of p
 	DevOtg otg;
 };
 
@@ -111,6 +123,7 @@ struct DevJt {
 	double dt;
 	osc_joint_params p;
 	double* st;	 // JC_COUNT x N
+	double* gains;	// per-robot PID gains, GAIN_COUNT x N (osc_set_gains); null: every robot uses those of p
 	DevOtg otg;
 };
 

@@ -84,6 +84,15 @@ inline bool cycle_spec_eligible(const OscProgram& P, bool has_jt, bool* motion) 
 	return true;
 }
 
+// Per-robot PID gains (osc_set_gains): a leading task of the hierarchy has a gain block.
+inline bool cycle_per_robot_gains(const OscProgram& P, bool has_jt) {
+	return (P.n_tasks >= 1 && P.tasks[0].type == OSC_TASK_MOTION_FORCE && P.mft[0].gains != nullptr) || (has_jt && P.jt[0].gains != nullptr);
+}
+// With per-robot gains, the specialised fused kernel of signature R (spec, motion: cycle_spec_eligible) has an instantiation that
+// reads them (PRG): the pure-motion full six-dof task and the three-direction task.  Otherwise the launch takes the
+// non-specialised kernel, which tests the gain-block pointers at run time.
+inline bool cycle_prg_specialised(int R, bool spec, bool motion) { return spec && ((R == 6 && motion) || R == 3); }
+
 // The optional single-precision mode (osc_cycle_f32.cu): the fused kernel of [full six-dof MotionForceTask under pure motion
 // control (+ full JointTask)] computed in FP32 on the FP64 state in global memory; robots it hands over continue on the FP64
 // general path.  cudaErrorNotSupported for a dof that is not compiled in (fused_f32_available).
@@ -108,6 +117,8 @@ cudaError_t launch_eval_model(const OscProgram& P, const osc_link_frame& frame, 
 							  double* g, cudaStream_t stream);
 cudaError_t launch_fill(double* st, int64_t NR, int comp, int ncomp, const double* vals, cudaStream_t stream);
 cudaError_t launch_copy(double* st, int64_t NR, int dst, int src, int ncomp, cudaStream_t stream);
+// *bad |= 1: some of the n values is not finite, |= 2: some is negative (*bad is not cleared)
+cudaError_t launch_check_values(const double* v, int64_t n, int32_t* bad, cudaStream_t stream);
 cudaError_t launch_fill_int(int32_t* ist, int64_t NR, int comp, int ncomp, int32_t value, cudaStream_t stream);
 
 }  // namespace osc

@@ -159,6 +159,34 @@ DEVI void popc_step(const DevMft& t, IDX NR, IDX i, const double fd[3], const do
 	ist[(int64_t)MI_RING_SIZE * NR + i] = size;
 }
 
+// Where a control law reads its PID gains: the task's broadcast parameters (GAINS_BCAST); its per-robot gain block
+// (GAINS_ROBOT: osc_set_gains, GainComp layout), loaded into registers once per robot -- or, for a task of the launch that has
+// no block, its parameters (one uniform branch); or, per use, whichever of the two the block pointer says (GAINS_ANY: the
+// non-specialised and general-path kernels).
+enum GainSrc : int { GAINS_BCAST = 0, GAINS_ROBOT = 1, GAINS_ANY = 2 };
+// pb: the task's parameters, whose first GAIN_COUNT values have the block's layout (checked in osc_capi.cu)
+template <int G, typename IDX>
+DEVI void load_gain_block(const gdouble* blk, const double* pb, IDX NR, IDX i, int c0, int nc, double* g) {
+	if constexpr (G == GAINS_ROBOT) {
+		if (blk) {
+#pragma unroll
+			for (int c = 0; c < nc; c++) g[c] = blk[(IDX)(c0 + c) * NR + i];
+		} else {
+#pragma unroll
+			for (int c = 0; c < nc; c++) g[c] = pb[c0 + c];
+		}
+	}
+}
+// gain `member[k]` (block component comp + k) of robot i
+#define OSC_GAIN(member, comp, k)                                                     \
+	(G == GAINS_BCAST	? p.member[k]                                                  \
+	 : G == GAINS_ROBOT ? kg[(comp) + (k)]                                             \
+						: (t.gains ? t.gains[(IDX)((comp) + (k)) * NR + i] : p.member[k]))
+#define OSC_GAIN1(member, comp)                                          \
+	(G == GAINS_BCAST	? p.member                                        \
+	 : G == GAINS_ROBOT ? kg[comp]                                        \
+						: (t.gains ? t.gains[(IDX)(comp) * NR + i] : p.member))
+
 DEVI void scale_to_norm(double v[3], double maxn) {
 	const double n = sqrt(dot3(v, v));
 	if (n > maxn) {
@@ -186,13 +214,17 @@ DEVI void mft_stage_goals(const DevMft& t, IDX NR, IDX i, double* sg, int sgs) {
 #pragma unroll
 	for (int c = 0; c < 6; c++) cp_async8(sg + (24 + c) * sgs, &ST(MC_INT_POS, c));
 }
-template <bool MOTION = false, typename IDX = int64_t>
+// G: where the gains come from (GainSrc).
+template <bool MOTION = false, typename IDX = int64_t, int G = GAINS_ANY>
 DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], const double R[9], const double v_in[3],
 						  const double w_in[3], bool write_observers, double fstar[6], double F[6], uint32_t& status,
 						  const double* sg = nullptr, int sgs = 0) {
 	gdouble* st = t.st;
 	const osc_mft_params& p = t.p;
 	const double dt = t.dt;
+	// per-robot gains: requested first (the fused kernel prefetched their rows into L2); pure motion control reads the motion ones only
+	double kg[GAIN_COUNT];
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, 0, MOTION ? MG_KP_FORCE : GAIN_COUNT, kg);
 	double v[3] = {v_in[0], v_in[1], v_in[2]}, w[3] = {w_in[0], w_in[1], w_in[2]};
 	if (!MOTION && !t.full) {	// _jacobian = P * J0  (MotionForceTask.cpp:280-282, 293-298)
 		double tv[3], tw[3];
@@ -251,8 +283,8 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 			Ip[k] += ex * dt;
 			Io[k] += ori_err_goal[k] * dt;
 			if (MOTION || !p.use_velocity_saturation) {
-				fstar[k] = ad[k] - p.kp_pos[k] * ex - p.kv_pos[k] * (v[k] - vd[k]) - p.ki_pos[k] * Ip[k];
-				fstar[3 + k] = ald[k] - p.kp_ori[k] * ori_err_goal[k] - p.kv_ori[k] * (w[k] - wd[k]) - p.ki_ori[k] * Io[k];
+				fstar[k] = ad[k] - OSC_GAIN(kp_pos, MG_KP_POS, k) * ex - OSC_GAIN(kv_pos, MG_KV_POS, k) * (v[k] - vd[k]) - OSC_GAIN(ki_pos, MG_KI_POS, k) * Ip[k];
+				fstar[3 + k] = ald[k] - OSC_GAIN(kp_ori, MG_KP_ORI, k) * ori_err_goal[k] - OSC_GAIN(kv_ori, MG_KV_ORI, k) * (w[k] - wd[k]) - OSC_GAIN(ki_ori, MG_KI_ORI, k) * Io[k];
 			}
 			F[k] = 0.0;
 			F[3 + k] = 0.0;
@@ -261,16 +293,16 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 			double vdes[3], wdes[3];
 #pragma unroll
 			for (int k = 0; k < 3; k++) {
-				const double kvi = pinv_gain(p.kv_pos[k]), kwi = pinv_gain(p.kv_ori[k]);
-				vdes[k] = -p.kp_pos[k] * kvi * (x[k] - xd[k]) - p.ki_pos[k] * kvi * Ip[k];
-				wdes[k] = -p.kp_ori[k] * kwi * ori_err_goal[k] - p.ki_ori[k] * kwi * Io[k];
+				const double kvi = pinv_gain(OSC_GAIN(kv_pos, MG_KV_POS, k)), kwi = pinv_gain(OSC_GAIN(kv_ori, MG_KV_ORI, k));
+				vdes[k] = -OSC_GAIN(kp_pos, MG_KP_POS, k) * kvi * (x[k] - xd[k]) - OSC_GAIN(ki_pos, MG_KI_POS, k) * kvi * Ip[k];
+				wdes[k] = -OSC_GAIN(kp_ori, MG_KP_ORI, k) * kwi * ori_err_goal[k] - OSC_GAIN(ki_ori, MG_KI_ORI, k) * kwi * Io[k];
 			}
 			scale_to_norm(vdes, p.linear_saturation_velocity);
 			scale_to_norm(wdes, p.angular_saturation_velocity);
 #pragma unroll
 			for (int k = 0; k < 3; k++) {
-				fstar[k] = ad[k] - p.kv_pos[k] * (v[k] - vdes[k]);
-				fstar[3 + k] = ald[k] - p.kv_ori[k] * (w[k] - wdes[k]);
+				fstar[k] = ad[k] - OSC_GAIN(kv_pos, MG_KV_POS, k) * (v[k] - vdes[k]);
+				fstar[3 + k] = ald[k] - OSC_GAIN(kv_ori, MG_KV_ORI, k) * (w[k] - wdes[k]);
 			}
 		}
 		store3(st, NR, i, MC_INT_POS, Ip);
@@ -340,7 +372,7 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 		store3(st, NR, i, MC_INT_FORCE, If);
 		double pre[3], fb[3];
 #pragma unroll
-		for (int k = 0; k < 3; k++) pre[k] = -p.kp_force * e[k] - p.ki_force * If[k];
+		for (int k = 0; k < 3; k++) pre[k] = -OSC_GAIN1(kp_force, MG_KP_FORCE) * e[k] - OSC_GAIN1(ki_force, MG_KI_FORCE) * If[k];
 		mat3_vec(Sf, pre, fb);
 		scale_to_norm(fb, p.max_force_control_feedback_output);
 		double a_fd[3], a_fs[3], a_vcl[3], a_vr[3];
@@ -348,9 +380,9 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 		mat3_vec(Sf, fs, a_fs);
 		mat3_vec(Sf, fb, a_vcl);
 		mat3_vec(Sf, v, a_vr);
-		popc_step(t, NR, i, a_fd, a_fs, a_vcl, a_vr, p.kv_force, p.kff_force, force_fb, status);
+		popc_step(t, NR, i, a_fd, a_fs, a_vcl, a_vr, OSC_GAIN1(kv_force, MG_KV_FORCE), p.kff_force, force_fb, status);
 	} else {
-		double pre[3] = {-p.kv_force * v[0], -p.kv_force * v[1], -p.kv_force * v[2]};
+		double pre[3] = {-OSC_GAIN1(kv_force, MG_KV_FORCE) * v[0], -OSC_GAIN1(kv_force, MG_KV_FORCE) * v[1], -OSC_GAIN1(kv_force, MG_KV_FORCE) * v[2]};
 		mat3_vec(Sf, pre, force_fb);
 	}
 	// ---- moment ----  :357-383
@@ -366,14 +398,14 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 		store3(st, NR, i, MC_INT_MOMENT, Im);
 		double pre[3], mb[3];
 #pragma unroll
-		for (int k = 0; k < 3; k++) pre[k] = -p.kp_moment * e[k] - p.ki_moment * Im[k];
+		for (int k = 0; k < 3; k++) pre[k] = -OSC_GAIN1(kp_moment, MG_KP_MOMENT) * e[k] - OSC_GAIN1(ki_moment, MG_KI_MOMENT) * Im[k];
 		mat3_vec(Sm, pre, mb);
 		scale_to_norm(mb, p.max_moment_control_feedback_output);
 #pragma unroll
-		for (int k = 0; k < 3; k++) pre[k] = mb[k] - p.kv_moment * w[k];
+		for (int k = 0; k < 3; k++) pre[k] = mb[k] - OSC_GAIN1(kv_moment, MG_KV_MOMENT) * w[k];
 		mat3_vec(Sm, pre, moment_fb);
 	} else {
-		double pre[3] = {-p.kv_moment * w[0], -p.kv_moment * w[1], -p.kv_moment * w[2]};
+		double pre[3] = {-OSC_GAIN1(kv_moment, MG_KV_MOMENT) * w[0], -OSC_GAIN1(kv_moment, MG_KV_MOMENT) * w[1], -OSC_GAIN1(kv_moment, MG_KV_MOMENT) * w[2]};
 		mat3_vec(Sm, pre, moment_fb);
 	}
 
@@ -391,19 +423,19 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 		double vdes[3];
 #pragma unroll
 		for (int k = 0; k < 3; k++) {
-			const double kvi = pinv_gain(p.kv_pos[k]);
-			vdes[k] = -p.kp_pos[k] * kvi * sex[k] - p.ki_pos[k] * kvi * Ip[k];
+			const double kvi = pinv_gain(OSC_GAIN(kv_pos, MG_KV_POS, k));
+			vdes[k] = -OSC_GAIN(kp_pos, MG_KP_POS, k) * kvi * sex[k] - OSC_GAIN(ki_pos, MG_KI_POS, k) * kvi * Ip[k];
 		}
 		scale_to_norm(vdes, p.linear_saturation_velocity);
 		double pre[3];
 #pragma unroll
-		for (int k = 0; k < 3; k++) pre[k] = ad[k] - p.kv_pos[k] * (v[k] - vdes[k]);
+		for (int k = 0; k < 3; k++) pre[k] = ad[k] - OSC_GAIN(kv_pos, MG_KV_POS, k) * (v[k] - vdes[k]);
 		mat3_vec(Sp, pre, pos_force);
 	} else {
 		double pre[3];
 #pragma unroll
 		for (int k = 0; k < 3; k++)
-			pre[k] = ad[k] - p.kp_pos[k] * ex[k] - p.kv_pos[k] * (v[k] - vd[k]) - p.ki_pos[k] * Ip[k];
+			pre[k] = ad[k] - OSC_GAIN(kp_pos, MG_KP_POS, k) * ex[k] - OSC_GAIN(kv_pos, MG_KV_POS, k) * (v[k] - vd[k]) - OSC_GAIN(ki_pos, MG_KI_POS, k) * Ip[k];
 		mat3_vec(Sp, pre, pos_force);
 	}
 	// ---- angular motion ----  :439-468
@@ -418,19 +450,19 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 		double wdes[3];
 #pragma unroll
 		for (int k = 0; k < 3; k++) {
-			const double kvi = pinv_gain(p.kv_ori[k]);
-			wdes[k] = -p.kp_ori[k] * kvi * eo[k] - p.ki_ori[k] * kvi * Io[k];
+			const double kvi = pinv_gain(OSC_GAIN(kv_ori, MG_KV_ORI, k));
+			wdes[k] = -OSC_GAIN(kp_ori, MG_KP_ORI, k) * kvi * eo[k] - OSC_GAIN(ki_ori, MG_KI_ORI, k) * kvi * Io[k];
 		}
 		scale_to_norm(wdes, p.angular_saturation_velocity);
 		double pre[3];
 #pragma unroll
-		for (int k = 0; k < 3; k++) pre[k] = ald[k] - p.kv_ori[k] * (w[k] - wdes[k]);
+		for (int k = 0; k < 3; k++) pre[k] = ald[k] - OSC_GAIN(kv_ori, MG_KV_ORI, k) * (w[k] - wdes[k]);
 		mat3_vec(So, pre, ori_force);
 	} else {
 		double pre[3];
 #pragma unroll
 		for (int k = 0; k < 3; k++)
-			pre[k] = ald[k] - p.kp_ori[k] * eo[k] - p.kv_ori[k] * (w[k] - wd[k]) - p.ki_ori[k] * Io[k];
+			pre[k] = ald[k] - OSC_GAIN(kp_ori, MG_KP_ORI, k) * eo[k] - OSC_GAIN(kv_ori, MG_KV_ORI, k) * (w[k] - wd[k]) - OSC_GAIN(ki_ori, MG_KI_ORI, k) * Io[k];
 		mat3_vec(So, pre, ori_force);
 	}
 	// ---- assemble ----  :470-491
@@ -484,10 +516,14 @@ DEVI void joint_stage_goals(const DevJt& t, const gdouble* qg, const gdouble* dq
 	}
 }
 // full joint task without velocity saturation from the staged copy (the SPEC instantiation)
-template <int N, typename IDX>
+template <int N, typename IDX, int G = GAINS_ANY>
 DEVI void joint_control_law_staged(const DevJt& t, IDX NR, IDX i, const double* sg, int sgs, double (&pid)[N], double (&acc)[N]) {
 	gdouble* st = t.st;
 	const osc_joint_params& p = t.p;
+	double kg[GAIN_COUNT];
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, JG_KP, N, kg + JG_KP);
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, JG_KV, N, kg + JG_KV);
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, JG_KI, N, kg + JG_KI);
 	cp_async_wait_all();
 	double I[N];
 #pragma unroll
@@ -495,17 +531,21 @@ DEVI void joint_control_law_staged(const DevJt& t, IDX NR, IDX i, const double* 
 		const double e = sg[(4 * N + a) * sgs] - sg[a * sgs];
 		acc[a] = sg[(2 * N + a) * sgs];
 		I[a] = sg[(3 * N + a) * sgs] + e * t.dt;
-		pid[a] = -p.kp[a] * e - p.kv[a] * (sg[(5 * N + a) * sgs] - sg[(N + a) * sgs]) - p.ki[a] * I[a];
+		pid[a] = -OSC_GAIN(kp, JG_KP, a) * e - OSC_GAIN(kv, JG_KV, a) * (sg[(5 * N + a) * sgs] - sg[(N + a) * sgs]) - OSC_GAIN(ki, JG_KI, a) * I[a];
 	}
 #pragma unroll
 	for (int a = 0; a < N; a++) ST(JC_INT, a) = I[a];
 }
 
-template <int N, int K, bool SPEC = false, typename IDX = int64_t>  // SPEC: full selection, no velocity saturation (host check)
+template <int N, int K, bool SPEC = false, typename IDX = int64_t, int G = GAINS_ANY>  // SPEC: full selection, no velocity saturation (host check)
 DEVI void joint_control_law(const DevJt& t, IDX NR, IDX i, const double (&q)[N], const double (&dq)[N],
 							double (&pid)[K], double (&acc)[K]) {
 	gdouble* st = t.st;
 	const osc_joint_params& p = t.p;
+	double kg[GAIN_COUNT];
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, JG_KP, K, kg + JG_KP);
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, JG_KV, K, kg + JG_KV);
+	load_gain_block<G>(t.gains, reinterpret_cast<const double*>(&p), NR, i, JG_KI, K, kg + JG_KI);
 	// all loads first, all stores last: the compiler cannot prove that the integrator stores do not alias the
 	// following goal loads, and would otherwise serialise one memory round trip per task coordinate
 	double gp[K], gv[K], I[K];
@@ -534,15 +574,15 @@ DEVI void joint_control_law(const DevJt& t, IDX NR, IDX i, const double (&q)[N],
 		const double e = pos - gp[a];
 		I[a] += e * t.dt;
 		if (!SPEC && p.use_velocity_saturation) {
-			const double kvi = pinv_gain(p.kv[a]);
-			double vdes = -p.kp[a] * kvi * e - p.ki[a] * kvi * I[a];
+			const double kvi = pinv_gain(OSC_GAIN(kv, JG_KV, a));
+			double vdes = -OSC_GAIN(kp, JG_KP, a) * kvi * e - OSC_GAIN(ki, JG_KI, a) * kvi * I[a];
 			if (vdes > p.saturation_velocity[a])
 				vdes = p.saturation_velocity[a];
 			else if (vdes < -p.saturation_velocity[a])
 				vdes = -p.saturation_velocity[a];
-			pid[a] = -p.kv[a] * (vel - vdes);
+			pid[a] = -OSC_GAIN(kv, JG_KV, a) * (vel - vdes);
 		} else {
-			pid[a] = -p.kp[a] * e - p.kv[a] * (vel - gv[a]) - p.ki[a] * I[a];
+			pid[a] = -OSC_GAIN(kp, JG_KP, a) * e - OSC_GAIN(kv, JG_KV, a) * (vel - gv[a]) - OSC_GAIN(ki, JG_KI, a) * I[a];
 		}
 	}
 #pragma unroll
@@ -555,6 +595,9 @@ static __device__ __noinline__ void joint_control_law_rt(const DevJt& t, int64_t
 														  double* pid, double* acc) {
 	gdouble* st = t.st;
 	const osc_joint_params& p = t.p;
+	constexpr int G = GAINS_ANY;
+	using IDX = int64_t;
+	double* kg = nullptr;  // unused with GAINS_ANY
 	for (int a = 0; a < k; a++) {
 		double pos = 0.0, vel = 0.0;
 		for (int j = 0; j < N; j++) {
@@ -568,18 +611,20 @@ static __device__ __noinline__ void joint_control_law_rt(const DevJt& t, int64_t
 		I += e * t.dt;
 		ST(JC_INT, a) = I;
 		if (p.use_velocity_saturation) {
-			const double kvi = pinv_gain(p.kv[a]);
-			double vdes = -p.kp[a] * kvi * e - p.ki[a] * kvi * I;
+			const double kvi = pinv_gain(OSC_GAIN(kv, JG_KV, a));
+			double vdes = -OSC_GAIN(kp, JG_KP, a) * kvi * e - OSC_GAIN(ki, JG_KI, a) * kvi * I;
 			if (vdes > p.saturation_velocity[a])
 				vdes = p.saturation_velocity[a];
 			else if (vdes < -p.saturation_velocity[a])
 				vdes = -p.saturation_velocity[a];
-			pid[a] = -p.kv[a] * (vel - vdes);
+			pid[a] = -OSC_GAIN(kv, JG_KV, a) * (vel - vdes);
 		} else {
-			pid[a] = -p.kp[a] * e - p.kv[a] * (vel - vd) - p.ki[a] * I;
+			pid[a] = -OSC_GAIN(kp, JG_KP, a) * e - OSC_GAIN(kv, JG_KV, a) * (vel - vd) - OSC_GAIN(ki, JG_KI, a) * I;
 		}
 	}
 }
 
+#undef OSC_GAIN
+#undef OSC_GAIN1
 #undef ST
 }  // namespace osc
