@@ -360,6 +360,23 @@ public:
 	int getMomentSpaceDimension() const { return params().moment_space_dimension; }
 	void setClosedLoopForceControl(bool on = true) { check(h(), osc_mft_set_closed_loop_force_control(h(), _id, on)); }
 	void setClosedLoopMomentControl(bool on = true) { check(h(), osc_mft_set_closed_loop_moment_control(h(), _id, on)); }
+	// per robot (osc_mft_parametrize_spaces_batched / osc_mft_set_closed_loop_batched), host or device memory: dims int32 x N, axes
+	// SoA 3 x N (axis of robot i at axes[k * N + i]), was_reset int32 x N or null; flags int32 x N of 0 / 1
+	void parametrizeForceMotionSpaces(const int32_t* dims, const double* axes, int32_t* was_reset, osc_mem_kind where) {
+		check(h(), osc_mft_parametrize_spaces_batched(h(), _id, 0, dims, axes, was_reset, where));
+	}
+	void parametrizeMomentRotMotionSpaces(const int32_t* dims, const double* axes, int32_t* was_reset, osc_mem_kind where) {
+		check(h(), osc_mft_parametrize_spaces_batched(h(), _id, 1, dims, axes, was_reset, where));
+	}
+	void setClosedLoopForceControl(const int32_t* flags, osc_mem_kind where) { check(h(), osc_mft_set_closed_loop_batched(h(), _id, 0, flags, where)); }
+	void setClosedLoopMomentControl(const int32_t* flags, osc_mem_kind where) { check(h(), osc_mft_set_closed_loop_batched(h(), _id, 1, flags, where)); }
+	// what the kernels use: dims int32 x N, axes SoA 3 x N, closed_loop int32 x N (any may be null)
+	void getForceMotionSpaces(int32_t* dims, double* axes, int32_t* closed_loop, osc_mem_kind where = OSC_MEM_HOST) const {
+		check(h(), osc_mft_get_spaces(h(), _id, 0, dims, axes, closed_loop, where));
+	}
+	void getMomentRotMotionSpaces(int32_t* dims, double* axes, int32_t* closed_loop, osc_mem_kind where = OSC_MEM_HOST) const {
+		check(h(), osc_mft_get_spaces(h(), _id, 1, dims, axes, closed_loop, where));
+	}
 	void enablePassivity(int ring_capacity = 0) { check(h(), osc_mft_enable_passivity(h(), _id, 1, ring_capacity)); }
 	void disablePassivity() { check(h(), osc_mft_enable_passivity(h(), _id, 0, 0)); }
 	void setForceSensorFrame(const std::string& link_name, const Affine& transformation_in_link) {

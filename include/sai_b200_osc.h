@@ -34,7 +34,7 @@ extern "C" {
 
 #define OSC_MAX_DOF 8
 #define OSC_MAX_TASKS 4
-#define OSC_ABI_VERSION 1
+#define OSC_ABI_VERSION 2
 
 typedef enum {
 	OSC_OK = 0,
@@ -318,6 +318,41 @@ typedef enum {
 int osc_set_gains(osc_handle* h, int task_id, int group, const double* kp, const double* kv, const double* ki, int mem_kind,
 				  int per_robot);
 int osc_get_gains(osc_handle* h, int task_id, int group, double* kp, double* kv, double* ki, int mem_kind);
+
+/* ---- per-robot force / moment spaces and closed-loop flags.  MotionForceTask::parametrizeForceMotionSpaces /
+ * parametrizeMomentRotMotionSpaces (MotionForceTask.cpp:830-890) and setClosedLoopForceControl / setClosedLoopMomentControl
+ * (:973-986), each robot of the batch with its own values (robots that touch their surfaces on different cycles and along
+ * different normals).  which = 0: force / motion space and closed-loop force control; which = 1: moment / rot-motion space and
+ * closed-loop moment control.  Passivity, in_compliant, the selection, the force sensor frame and the feed-forward and
+ * saturation parameters stay task-wide.
+ *   osc_mft_parametrize_spaces_batched: dims int32 x n_robots (0..3), axes SoA 3 x n_robots (read for robots of dimension 1 or
+ *     2 only), was_reset int32 x n_robots or NULL, all in mem_kind memory.  Robot i gets exactly what parametrize*(dims[i],
+ *     axis_i) does to a task object of the reference: the axis is normalised (dimension 0 or 3: the stored axis stays), and
+ *     the robot is reset when its dimension changes or its normalised axis is not Eigen's isApprox to the stored one -- goal
+ *     position (orientation) := current, linear (angular) velocity and acceleration goals := 0, position and force
+ *     (orientation and moment) integrators := 0; with the internal OTG on, its generator is re-initialised linearly (angularly)
+ *     instead of the goal copy.  was_reset[i] = 1 for a robot that was reset.  Robots that are not reset are left untouched.
+ *   osc_mft_set_closed_loop_batched: enabled int32 x n_robots (0 or 1).  A robot whose flag changes gets its linear (force) or
+ *     angular (moment) integrators zeroed.  POPC state advances only for robots with closed-loop force control on.
+ *   osc_mft_get_spaces: what the kernels use, in either mode: dims int32 x n_robots, axes SoA 3 x n_robots (normalised),
+ *     closed_loop int32 x n_robots; any pointer may be NULL.
+ * Every value is checked before anything is written: a dimension outside 0..3, an axis of a dimension-1/2 robot that is not
+ * finite or shorter than 1e-2, or a flag other than 0/1 returns OSC_ERR_INVALID_ARGUMENT with the reference's message and
+ * leaves every robot as it was.  Device input is checked by a reduction kernel and the call synchronises the handle's stream;
+ * host input and output synchronise too.  Writes are ordered with the control cycles in the handle's stream like goal writes.
+ * The first batched call on a task allocates its space block (one int32 and 6 doubles per robot), fills it from the task's
+ * broadcast parameters and then applies the call; there is no way back.  From then on osc_mft_parametrize_* and
+ * osc_mft_set_closed_loop_* apply the same values to every robot through the per-robot path, each robot deciding its own
+ * reset (*was_reset = 1 if any robot was reset), osc_mft_set_params keeps rejecting changes to these fields, and
+ * osc_mft_get_params reports the values of the last broadcast call.
+ * While every robot of the task is in free motion (dimension 0 in both spaces, both loops open) the launch selects the same
+ * pure-motion kernels as for a broadcast task, which never read the block; once one robot is not, the force-capable kernels.
+ * The FP32 mode follows the same rule: it runs while every robot is in free motion and returns OSC_ERR_UNSUPPORTED otherwise.
+ * ---- */
+int osc_mft_parametrize_spaces_batched(osc_handle* h, int task_id, int which, const int32_t* dims, const double* axes, int32_t* was_reset,
+									   int mem_kind);
+int osc_mft_set_closed_loop_batched(osc_handle* h, int task_id, int which, const int32_t* enabled, int mem_kind);
+int osc_mft_get_spaces(osc_handle* h, int task_id, int which, int32_t* dims, double* axes, int32_t* closed_loop, int mem_kind);
 
 /* ---- internal online trajectory generation (SURVEY.md row f-4).  The reference interpolates every task's goal with its
  * vendored Ruckig by default (JointTask.h:38-42, MotionForceTask.h:67-74): acceleration-limited, phase-synchronised.  Tasks are

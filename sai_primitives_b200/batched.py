@@ -38,6 +38,11 @@ def _check(handle, rc):
     raise OscError(rc, msg)
 
 
+def _int_ptr(a):
+    assert a.dtype == np.int32 and a.flags["C_CONTIGUOUS"]
+    return a.ctypes.data_as(C.c_void_p)
+
+
 def _soa(a, n_robots, ncomp):
     """[N, ncomp] (or [ncomp] broadcast) -> contiguous SoA [ncomp, N]"""
     a = np.asarray(a, dtype=np.float64)
@@ -585,21 +590,83 @@ class MotionForceTask(_Task):
     def setSingularityHandlingGains(self, kp_type_1, kv_type_1, kv_type_2):
         p = self._params(); p.kp_type_1, p.kv_type_1, p.kv_type_2 = kp_type_1, kv_type_1, kv_type_2; self._apply(p)
 
+    def _parametrize(self, which, dim, axis, broadcast_fn):
+        """A scalar dim with a 3-vector: every robot (returns bool).  dim[N] with axis[N, 3] (or one 3-vector for every robot):
+        per robot, osc_mft_parametrize_spaces_batched (returns bool[N], True where the robot was reset)."""
+        if np.ndim(dim) == 0:
+            ax = (C.c_double * 3)(*[float(x) for x in np.asarray(axis, dtype=np.float64).reshape(3)]); r = C.c_int(0)
+            _check(self._robot.handle, broadcast_fn(self._robot.handle, self.task_id, int(dim), ax, C.byref(r)))
+            return bool(r.value)
+        N = self._robot.n_robots
+        dims = np.asarray(dim)
+        if dims.shape != (N,) or not np.issubdtype(dims.dtype, np.integer):
+            raise ValueError("per-robot dimensions must be an integer array of shape (%d,), got %s %s" % (N, dims.dtype, dims.shape))
+        dims = np.ascontiguousarray(dims, dtype=np.int32)
+        a = np.asarray(axis, dtype=np.float64)
+        if a.shape == (3,):
+            a = np.broadcast_to(a, (N, 3))
+        axes = _soa(a, N, 3)
+        reset = np.zeros(N, dtype=np.int32)
+        _check(self._robot.handle, self._lib.osc_mft_parametrize_spaces_batched(self._robot.handle, self.task_id, which, _int_ptr(dims),
+                                                                               capi.host_ptr(axes), _int_ptr(reset), capi.OSC_MEM_HOST))
+        return reset != 0
+
     def parametrizeForceMotionSpaces(self, dim, axis=(0.0, 0.0, 0.0)):
-        ax = (C.c_double * 3)(*[float(x) for x in axis]); r = C.c_int(0)
-        _check(self._robot.handle, self._lib.osc_mft_parametrize_force_motion_spaces(self._robot.handle, self.task_id, int(dim), ax, C.byref(r)))
-        return bool(r.value)
+        return self._parametrize(0, dim, axis, self._lib.osc_mft_parametrize_force_motion_spaces)
 
     def parametrizeMomentRotMotionSpaces(self, dim, axis=(0.0, 0.0, 0.0)):
-        ax = (C.c_double * 3)(*[float(x) for x in axis]); r = C.c_int(0)
-        _check(self._robot.handle, self._lib.osc_mft_parametrize_moment_rotmotion_spaces(self._robot.handle, self.task_id, int(dim), ax, C.byref(r)))
-        return bool(r.value)
+        return self._parametrize(1, dim, axis, self._lib.osc_mft_parametrize_moment_rotmotion_spaces)
+
+    def _parametrize_device(self, which, dims_ptr, axes_ptr, was_reset_ptr):
+        _check(self._robot.handle, self._lib.osc_mft_parametrize_spaces_batched(self._robot.handle, self.task_id, which, C.c_void_p(dims_ptr),
+                                                                               C.c_void_p(axes_ptr), C.c_void_p(was_reset_ptr or None),
+                                                                               capi.OSC_MEM_DEVICE))
+
+    # per robot from device memory: dims int32 [N], axes float64 SoA [3, N], was_reset int32 [N] or 0 (zero copy)
+    def parametrizeForceMotionSpacesDevice(self, dims_ptr, axes_ptr, was_reset_ptr=0): self._parametrize_device(0, dims_ptr, axes_ptr, was_reset_ptr)
+    def parametrizeMomentRotMotionSpacesDevice(self, dims_ptr, axes_ptr, was_reset_ptr=0): self._parametrize_device(1, dims_ptr, axes_ptr, was_reset_ptr)
+
+    def _set_closed_loop(self, which, flag, broadcast_fn):
+        if np.ndim(flag) == 0:
+            _check(self._robot.handle, broadcast_fn(self._robot.handle, self.task_id, 1 if flag else 0))
+            return
+        N = self._robot.n_robots
+        f = np.asarray(flag)
+        if f.shape != (N,):
+            raise ValueError("per-robot closed-loop flags must have shape (%d,), got %s" % (N, f.shape))
+        f = np.ascontiguousarray(f.astype(bool), dtype=np.int32)
+        _check(self._robot.handle, self._lib.osc_mft_set_closed_loop_batched(self._robot.handle, self.task_id, which, _int_ptr(f), capi.OSC_MEM_HOST))
 
     def setClosedLoopForceControl(self, flag=True):
-        _check(self._robot.handle, self._lib.osc_mft_set_closed_loop_force_control(self._robot.handle, self.task_id, 1 if flag else 0))
+        """bool for every robot, or bool[N] per robot"""
+        self._set_closed_loop(0, flag, self._lib.osc_mft_set_closed_loop_force_control)
 
     def setClosedLoopMomentControl(self, flag=True):
-        _check(self._robot.handle, self._lib.osc_mft_set_closed_loop_moment_control(self._robot.handle, self.task_id, 1 if flag else 0))
+        """bool for every robot, or bool[N] per robot"""
+        self._set_closed_loop(1, flag, self._lib.osc_mft_set_closed_loop_moment_control)
+
+    # per robot from device memory: int32 [N] of 0 / 1
+    def setClosedLoopForceControlDevice(self, flags_ptr):
+        _check(self._robot.handle, self._lib.osc_mft_set_closed_loop_batched(self._robot.handle, self.task_id, 0, C.c_void_p(flags_ptr), capi.OSC_MEM_DEVICE))
+
+    def setClosedLoopMomentControlDevice(self, flags_ptr):
+        _check(self._robot.handle, self._lib.osc_mft_set_closed_loop_batched(self._robot.handle, self.task_id, 1, C.c_void_p(flags_ptr), capi.OSC_MEM_DEVICE))
+
+    def _get_spaces(self, which):
+        N = self._robot.n_robots
+        dims, cl = np.zeros(N, dtype=np.int32), np.zeros(N, dtype=np.int32)
+        axes = np.zeros((3, N))
+        _check(self._robot.handle, self._lib.osc_mft_get_spaces(self._robot.handle, self.task_id, which, _int_ptr(dims), capi.host_ptr(axes),
+                                                                _int_ptr(cl), capi.OSC_MEM_HOST))
+        return dims, axes.T.copy(), cl != 0
+
+    def getForceMotionSpaces(self):
+        """what the kernels use: (dims int32 [N], normalised axes [N, 3], closed-loop force control bool [N])"""
+        return self._get_spaces(0)
+
+    def getMomentRotMotionSpaces(self):
+        """what the kernels use: (dims int32 [N], normalised axes [N, 3], closed-loop moment control bool [N])"""
+        return self._get_spaces(1)
 
     def enablePassivity(self, ring_capacity=0):
         _check(self._robot.handle, self._lib.osc_mft_enable_passivity(self._robot.handle, self.task_id, 1, int(ring_capacity)))

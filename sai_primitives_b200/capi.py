@@ -17,7 +17,7 @@ LIB_PATH = os.environ.get("SAI_B200_OSC_LIB", os.path.join(_HERE, "libsai_b200_o
 
 OSC_MAX_DOF = 8
 OSC_MAX_TASKS = 4
-OSC_ABI_VERSION = 1
+OSC_ABI_VERSION = 2
 
 OSC_OK = 0
 OSC_ERR_INVALID_ARGUMENT = -1
@@ -226,6 +226,9 @@ SYMBOLS = {
     "osc_sim_integrate": (C.c_int, [_H, _PD, _PD, _PD, C.c_double, C.c_int, C.c_int]),
     "osc_set_gains": (C.c_int, [_H, C.c_int, C.c_int, _PD, _PD, _PD, C.c_int, C.c_int]),
     "osc_get_gains": (C.c_int, [_H, C.c_int, C.c_int, _PD, _PD, _PD, C.c_int]),
+    "osc_mft_parametrize_spaces_batched": (C.c_int, [_H, C.c_int, C.c_int, _PD, _PD, _PD, C.c_int]),
+    "osc_mft_set_closed_loop_batched": (C.c_int, [_H, C.c_int, C.c_int, _PD, C.c_int]),
+    "osc_mft_get_spaces": (C.c_int, [_H, C.c_int, C.c_int, _PD, _PD, _PD, C.c_int]),
     "osc_eval_model": (C.c_int, [_H, C.c_int, C.POINTER(LinkFrame), C.POINTER(D), _PD, _PD, _PD, _PD, _PD, C.c_int]),
 }
 

@@ -1,6 +1,7 @@
 #include "osc_aux_kernels.cuh"
 #include "osc_observers.cuh"
 #include "osc_otg_kernels.cuh"
+#include "osc_space_kernels.cuh"
 #include "osc_launch.h"
 
 namespace osc {
@@ -120,6 +121,25 @@ cudaError_t launch_copy(double* st, int64_t NR, int dst, int src, int ncomp, cud
 cudaError_t launch_check_values(const double* v, int64_t n, int32_t* bad, cudaStream_t stream) {
 	const int64_t want = (n + 255) / 256;
 	check_values_kernel<<<(unsigned)(want < 1024 ? (want > 0 ? want : 1) : 1024), 256, 0, stream>>>(v, n, bad);
+	return cudaGetLastError();
+}
+cudaError_t launch_check_spaces(const int32_t* dims, const double* axes, const int32_t* flags, int64_t n, int32_t* out, cudaStream_t stream) {
+	const int64_t want = (n + 255) / 256;
+	check_spaces_kernel<<<(unsigned)(want < 1024 ? (want > 0 ? want : 1) : 1024), 256, 0, stream>>>(dims, axes, flags, n, out);
+	return cudaGetLastError();
+}
+cudaError_t launch_apply_spaces(const OscProgram& P, int mft_index, int moment, const int32_t* dims, const double* axes, int dim,
+								const double axis[3], int32_t* was_reset, int32_t* any_reset, cudaStream_t stream) {
+	SpaceArgs a{dims, axes, dim, {axis[0], axis[1], axis[2]}, was_reset, any_reset};
+	apply_spaces_kernel<<<grid_for(P.n_robots, 64), 64, 0, stream>>>(P, mft_index, moment, a);
+	return cudaGetLastError();
+}
+cudaError_t launch_set_closed_loop(const OscProgram& P, int mft_index, int moment, const int32_t* flags, int flag, cudaStream_t stream) {
+	set_closed_loop_kernel<<<grid_for(P.n_robots, 256), 256, 0, stream>>>(P, mft_index, moment, flags, flag);
+	return cudaGetLastError();
+}
+cudaError_t launch_get_spaces(const OscProgram& P, int mft_index, int moment, int32_t* dims, double* axes, int32_t* closed_loop, cudaStream_t stream) {
+	get_spaces_kernel<<<grid_for(P.n_robots, 256), 256, 0, stream>>>(P, mft_index, moment, dims, axes, closed_loop);
 	return cudaGetLastError();
 }
 cudaError_t launch_fill_int(int32_t* ist, int64_t NR, int comp, int ncomp, int32_t value, cudaStream_t stream) {

@@ -55,7 +55,10 @@ struct osc_handle {
 	double* d_scratch = nullptr;  // output of the on-request observers (osc_observers.cuh)
 	size_t scratch_doubles = 0;
 	int32_t* h_seen = nullptr;	// mapped pinned: hand-over count of the last completed cycle
-	int32_t* d_check = nullptr;	// result word of the device-input validation of osc_set_gains
+	int32_t* d_check = nullptr;	// result word of the device-input validation of osc_set_gains and of the per-robot space calls
+	// staging of the per-robot space calls with host buffers: axes (3 x N), dims or flags (N) and was_reset / closed_loop (N)
+	double* d_space_axes = nullptr;
+	int32_t* d_space_ints = nullptr;
 	int clean_cycles = 0;
 	int blend_split = -1;  // split blending path: -1 not decided, 0 off (SAI_B200_BLEND_SPLIT=0 or no memory), 1 allocate when needed, 2 allocated
 	int64_t blend_split_min = 0;  // hand-over count (host hint) from which the split path is used
@@ -757,37 +760,100 @@ int osc_mft_set_params(osc_handle* h, int task_id, const osc_mft_params* p) {
 	return OSC_OK;
 }
 
+// ---- force / moment spaces and closed-loop flags, broadcast and per robot ----
+namespace {
+const char* space_dim_msg(bool moment) {
+	return moment ? "Moment space dimension should be between 0 and 3 in MotionForceTask::parametrizeMomentRotMotionSpaces"
+				  : "Force space dimension should be between 0 and 3 in MotionForceTask::parametrizeForceMotionSpaces";
+}
+const char* space_axis_msg(bool moment) {
+	return moment ? "Moment or rot motion axis should be a non singular vector in MotionForceTask::parametrizeMomentRotMotionSpaces"
+				  : "Force or motion axis should be a non singular vector in MotionForceTask::parametrizeForceMotionSpaces";
+}
+int32_t space_summary(const osc_mft_params& p) {
+	return (p.force_space_dimension ? SPS_FORCE_DIM : 0) | (p.moment_space_dimension ? SPS_MOMENT_DIM : 0) |
+		   (p.closed_loop_force_control ? SPS_CL_FORCE : 0) | (p.closed_loop_moment_control ? SPS_CL_MOMENT : 0);
+}
+void set_summary_bit(DevMft& t, int32_t bit, bool on) { t.space_any = (t.space_any & ~bit) | (on ? bit : 0); }
+// The first per-robot call on a task: its space block, every robot as the broadcast parameters say.  There is no way back.
+int space_block(osc_handle* h, DevMft& t) {
+	if (t.space_mode) return OSC_OK;
+	int32_t* mode = nullptr;
+	double* axes = nullptr;
+	int rc = dev_alloc(h, &mode, (size_t)h->NR, false);
+	if (rc != OSC_OK) return rc;
+	if ((rc = dev_alloc(h, &axes, (size_t)SP_AXES_COUNT * h->NR, false)) != OSC_OK) return rc;
+	const osc_mft_params& p = t.p;
+	const double v[SP_AXES_COUNT] = {p.force_or_motion_axis[0], p.force_or_motion_axis[1], p.force_or_motion_axis[2],
+									 p.moment_or_rotmotion_axis[0], p.moment_or_rotmotion_axis[1], p.moment_or_rotmotion_axis[2]};
+	CUDA_TRY(h, osc::launch_fill_int(mode, h->NR, 0, 1,
+									 space_mode_word(p.force_space_dimension, p.moment_space_dimension, p.closed_loop_force_control != 0,
+													 p.closed_loop_moment_control != 0),
+									 h->stream));
+	CUDA_TRY(h, osc::launch_fill(axes, h->NR, 0, SP_AXES_COUNT, v, h->stream));
+	h->launches += 2;
+	t.space_mode = mode;
+	t.space_axes = axes;
+	t.space_any = space_summary(p);
+	return OSC_OK;
+}
+int space_staging(osc_handle* h) {
+	if (h->d_space_axes) return OSC_OK;
+	int rc = dev_alloc(h, &h->d_space_axes, (size_t)3 * h->NR, false);
+	if (rc != OSC_OK) return rc;
+	return dev_alloc(h, &h->d_space_ints, (size_t)2 * h->NR, false);
+}
+// h->d_check, cleared in stream order
+int clear_check_word(osc_handle* h) {
+	if (!h->d_check) {
+		int rc = dev_alloc(h, &h->d_check, 1, false);
+		if (rc != OSC_OK) return rc;
+	}
+	CUDA_TRY(h, cudaMemsetAsync(h->d_check, 0, sizeof(int32_t), h->stream));
+	return OSC_OK;
+}
+// SpaceCheck bits of per-robot values in device memory (dims / axes or flags); synchronises the stream
+int check_spaces_device(osc_handle* h, const int32_t* dims, const double* axes, const int32_t* flags, int32_t* f) {
+	int rc = clear_check_word(h);
+	if (rc != OSC_OK) return rc;
+	CUDA_TRY(h, osc::launch_check_spaces(dims, axes, flags, h->NR, h->d_check, h->stream));
+	h->launches++;
+	CUDA_TRY(h, cudaMemcpyAsync(f, h->d_check, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+	CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+	return OSC_OK;
+}
+}  // namespace
+
 static int parametrize_common(osc_handle* h, int task_id, int dim, const double axis[3], bool moment, int* was_reset) {
 	int rc = check_task(h, task_id, OSC_TASK_MOTION_FORCE);
 	if (rc != OSC_OK) return rc;
-	DevMft& t = h->prog.mft[h->tasks[task_id].index];
-	if (dim < 0 || dim > 3)
-		return fail(h, OSC_ERR_INVALID_ARGUMENT,
-					moment ? "Moment space dimension should be between 0 and 3 in MotionForceTask::parametrizeMomentRotMotionSpaces"
-						   : "Force space dimension should be between 0 and 3 in MotionForceTask::parametrizeForceMotionSpaces");
+	const int idx = h->tasks[task_id].index;
+	DevMft& t = h->prog.mft[idx];
+	if (dim < 0 || dim > 3) return fail(h, OSC_ERR_INVALID_ARGUMENT, space_dim_msg(moment));
 	int32_t& cur_dim = moment ? t.p.moment_space_dimension : t.p.force_space_dimension;
 	double* cur_axis = moment ? t.p.moment_or_rotmotion_axis : t.p.force_or_motion_axis;
 	bool reset = dim != cur_dim;
 	if (dim == 1 || dim == 2) {
 		if (!axis) return fail(h, OSC_ERR_INVALID_ARGUMENT, "axis required for dimension 1 or 2");
-		const double nrm = std::sqrt(axis[0] * axis[0] + axis[1] * axis[1] + axis[2] * axis[2]);
-		if (nrm < 1e-2)
-			return fail(h, OSC_ERR_INVALID_ARGUMENT,
-						moment ? "Moment or rot motion axis should be a non singular vector in "
-								 "MotionForceTask::parametrizeMomentRotMotionSpaces"
-							   : "Force or motion axis should be a non singular vector in "
-								 "MotionForceTask::parametrizeForceMotionSpaces");
-		const double a[3] = {axis[0] / nrm, axis[1] / nrm, axis[2] / nrm};
-		// Eigen isApprox: |a-b|^2 <= 1e-24 min(|a|^2, |b|^2)
-		double d2 = 0, b2 = 0;
-		for (int k = 0; k < 3; k++) {
-			d2 += (a[k] - cur_axis[k]) * (a[k] - cur_axis[k]);
-			b2 += cur_axis[k] * cur_axis[k];
-		}
-		reset = reset || !(d2 <= 1e-24 * std::min(1.0, b2));
+		double a[3];
+		if (space_normalize(axis, a) < 1e-2) return fail(h, OSC_ERR_INVALID_ARGUMENT, space_axis_msg(moment));
+		reset = reset || !space_axis_is_approx(a, cur_axis);
 		for (int k = 0; k < 3; k++) cur_axis[k] = a[k];
 	}
 	cur_dim = dim;
+	if (t.space_mode) {
+		// per-robot spaces: the same values for every robot, each robot decides its own reset; *was_reset: any robot was reset
+		set_summary_bit(t, moment ? SPS_MOMENT_DIM : SPS_FORCE_DIM, dim != 0);
+		if ((rc = clear_check_word(h)) != OSC_OK) return rc;
+		const double none[3] = {0, 0, 0};
+		CUDA_TRY(h, osc::launch_apply_spaces(h->prog, idx, moment ? 1 : 0, nullptr, nullptr, dim, axis ? axis : none, nullptr, h->d_check, h->stream));
+		h->launches++;
+		int32_t any = 0;
+		CUDA_TRY(h, cudaMemcpyAsync(&any, h->d_check, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+		CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+		if (was_reset) *was_reset = any ? 1 : 0;
+		return OSC_OK;
+	}
 	if (reset && t.otg.enabled) {
 		// the same resets with the internal OTG on: goals and generator together (_otg->reInitializeLinear / Angular, :854, :886)
 		CUDA_TRY(h, osc::launch_otg_init(h->prog, task_id, moment ? 2 : 1, 0, h->stream));
@@ -840,26 +906,132 @@ int osc_mft_reset_integrators(osc_handle* h, int task_id, int which) {
 	return OSC_OK;
 }
 
-int osc_mft_set_closed_loop_force_control(osc_handle* h, int task_id, int enabled) {
-	ENTER(h);
+static int set_closed_loop_common(osc_handle* h, int task_id, int enabled, bool moment) {
 	int rc = check_task(h, task_id, OSC_TASK_MOTION_FORCE);
 	if (rc != OSC_OK) return rc;
-	DevMft& t = h->prog.mft[h->tasks[task_id].index];
-	if ((t.p.closed_loop_force_control != 0) != (enabled != 0)) {
-		t.p.closed_loop_force_control = enabled ? 1 : 0;
-		return osc_mft_reset_integrators(h, task_id, 1);
+	const int idx = h->tasks[task_id].index;
+	DevMft& t = h->prog.mft[idx];
+	int32_t& cur = moment ? t.p.closed_loop_moment_control : t.p.closed_loop_force_control;
+	const bool changed = (cur != 0) != (enabled != 0);
+	cur = enabled ? 1 : 0;
+	if (t.space_mode) {
+		// per-robot flags: every robot gets the flag, a robot whose flag changes gets its integrators zeroed
+		set_summary_bit(t, moment ? SPS_CL_MOMENT : SPS_CL_FORCE, enabled != 0);
+		CUDA_TRY(h, osc::launch_set_closed_loop(h->prog, idx, moment ? 1 : 0, nullptr, enabled ? 1 : 0, h->stream));
+		h->launches++;
+		return OSC_OK;
 	}
-	return OSC_OK;
+	return changed ? osc_mft_reset_integrators(h, task_id, moment ? 2 : 1) : OSC_OK;
+}
+int osc_mft_set_closed_loop_force_control(osc_handle* h, int task_id, int enabled) {
+	ENTER(h);
+	return set_closed_loop_common(h, task_id, enabled, false);
 }
 int osc_mft_set_closed_loop_moment_control(osc_handle* h, int task_id, int enabled) {
 	ENTER(h);
+	return set_closed_loop_common(h, task_id, enabled, true);
+}
+
+int osc_mft_parametrize_spaces_batched(osc_handle* h, int task_id, int which, const int32_t* dims, const double* axes, int32_t* was_reset,
+									   int mem_kind) {
+	ENTER(h);
 	int rc = check_task(h, task_id, OSC_TASK_MOTION_FORCE);
 	if (rc != OSC_OK) return rc;
-	DevMft& t = h->prog.mft[h->tasks[task_id].index];
-	if ((t.p.closed_loop_moment_control != 0) != (enabled != 0)) {
-		t.p.closed_loop_moment_control = enabled ? 1 : 0;
-		return osc_mft_reset_integrators(h, task_id, 2);
+	if (which != 0 && which != 1) return fail(h, OSC_ERR_INVALID_ARGUMENT, "which must be 0 (force / motion) or 1 (moment / rot motion)");
+	if (!dims || !axes) return fail(h, OSC_ERR_INVALID_ARGUMENT, "null dims or axes");
+	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
+	const bool moment = which == 1, host = mem_kind == OSC_MEM_HOST;
+	const int idx = h->tasks[task_id].index;
+	DevMft& t = h->prog.mft[idx];
+	const int64_t NR = h->NR;
+	// every value is checked before anything is written
+	int32_t f = 0;
+	if (host) {
+		for (int64_t i = 0; i < NR; i++)
+			f |= (dims[i] == 1 || dims[i] == 2) ? space_check(dims[i], axes[i], axes[NR + i], axes[2 * NR + i]) : space_check(dims[i], 0, 0, 0);
+	} else if ((rc = check_spaces_device(h, dims, axes, nullptr, &f)) != OSC_OK) {
+		return rc;
 	}
+	if (f & SPC_BAD_DIM) return fail(h, OSC_ERR_INVALID_ARGUMENT, space_dim_msg(moment));
+	if (f & SPC_BAD_AXIS) return fail(h, OSC_ERR_INVALID_ARGUMENT, space_axis_msg(moment));
+	if ((rc = space_block(h, t)) != OSC_OK) return rc;
+	const int32_t* d_dims = dims;
+	const double* d_axes = axes;
+	int32_t* d_reset = was_reset;
+	if (host) {
+		if ((rc = space_staging(h)) != OSC_OK) return rc;
+		CUDA_TRY(h, cudaMemcpyAsync(h->d_space_ints, dims, (size_t)NR * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+		CUDA_TRY(h, cudaMemcpyAsync(h->d_space_axes, axes, (size_t)3 * NR * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+		d_dims = h->d_space_ints;
+		d_axes = h->d_space_axes;
+		d_reset = was_reset ? h->d_space_ints + NR : nullptr;
+	}
+	const double none[3] = {0, 0, 0};
+	CUDA_TRY(h, osc::launch_apply_spaces(h->prog, idx, moment ? 1 : 0, d_dims, d_axes, 0, none, d_reset, nullptr, h->stream));
+	h->launches++;
+	set_summary_bit(t, moment ? SPS_MOMENT_DIM : SPS_FORCE_DIM, (f & SPC_NONZERO) != 0);
+	if (host) {
+		if (was_reset) CUDA_TRY(h, cudaMemcpyAsync(was_reset, d_reset, (size_t)NR * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+		CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+	}
+	return OSC_OK;
+}
+
+int osc_mft_set_closed_loop_batched(osc_handle* h, int task_id, int which, const int32_t* enabled, int mem_kind) {
+	ENTER(h);
+	int rc = check_task(h, task_id, OSC_TASK_MOTION_FORCE);
+	if (rc != OSC_OK) return rc;
+	if (which != 0 && which != 1) return fail(h, OSC_ERR_INVALID_ARGUMENT, "which must be 0 (force) or 1 (moment)");
+	if (!enabled) return fail(h, OSC_ERR_INVALID_ARGUMENT, "null flags");
+	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
+	const bool moment = which == 1, host = mem_kind == OSC_MEM_HOST;
+	const int idx = h->tasks[task_id].index;
+	DevMft& t = h->prog.mft[idx];
+	const int64_t NR = h->NR;
+	int32_t f = 0;
+	if (host) {
+		for (int64_t i = 0; i < NR; i++) f |= closed_loop_check(enabled[i]);
+	} else if ((rc = check_spaces_device(h, nullptr, nullptr, enabled, &f)) != OSC_OK) {
+		return rc;
+	}
+	if (f & SPC_BAD_FLAG) return fail(h, OSC_ERR_INVALID_ARGUMENT, "closed loop flags must be 0 or 1");
+	if ((rc = space_block(h, t)) != OSC_OK) return rc;
+	const int32_t* d_flags = enabled;
+	if (host) {
+		if ((rc = space_staging(h)) != OSC_OK) return rc;
+		CUDA_TRY(h, cudaMemcpyAsync(h->d_space_ints, enabled, (size_t)NR * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+		d_flags = h->d_space_ints;
+	}
+	CUDA_TRY(h, osc::launch_set_closed_loop(h->prog, idx, moment ? 1 : 0, d_flags, 0, h->stream));
+	h->launches++;
+	set_summary_bit(t, moment ? SPS_CL_MOMENT : SPS_CL_FORCE, (f & SPC_NONZERO) != 0);
+	if (host) CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+	return OSC_OK;
+}
+
+int osc_mft_get_spaces(osc_handle* h, int task_id, int which, int32_t* dims, double* axes, int32_t* closed_loop, int mem_kind) {
+	ENTER(h);
+	int rc = check_task(h, task_id, OSC_TASK_MOTION_FORCE);
+	if (rc != OSC_OK) return rc;
+	if (which != 0 && which != 1) return fail(h, OSC_ERR_INVALID_ARGUMENT, "which must be 0 (force / motion) or 1 (moment / rot motion)");
+	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
+	const int idx = h->tasks[task_id].index;
+	const int64_t NR = h->NR;
+	if (mem_kind == OSC_MEM_DEVICE) {
+		CUDA_TRY(h, osc::launch_get_spaces(h->prog, idx, which, dims, axes, closed_loop, h->stream));
+		h->launches++;
+		return OSC_OK;
+	}
+	if ((rc = space_staging(h)) != OSC_OK) return rc;
+	int32_t* d_dims = dims ? h->d_space_ints : nullptr;
+	int32_t* d_cl = closed_loop ? h->d_space_ints + NR : nullptr;
+	double* d_axes = axes ? h->d_space_axes : nullptr;
+	CUDA_TRY(h, osc::launch_get_spaces(h->prog, idx, which, d_dims, d_axes, d_cl, h->stream));
+	h->launches++;
+	if (dims) CUDA_TRY(h, cudaMemcpyAsync(dims, d_dims, (size_t)NR * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+	if (closed_loop) CUDA_TRY(h, cudaMemcpyAsync(closed_loop, d_cl, (size_t)NR * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+	if (axes) CUDA_TRY(h, cudaMemcpyAsync(axes, d_axes, (size_t)3 * NR * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+	CUDA_TRY(h, cudaStreamSynchronize(h->stream));
 	return OSC_OK;
 }
 

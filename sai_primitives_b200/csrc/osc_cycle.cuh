@@ -132,8 +132,10 @@ DEVI void reduce_task_vector(const DevMft& t, const double (&v6)[6], double (&y)
 // One bulk prefetch (cp.async.bulk.prefetch.L2) per state component for the robots of block `blk`: they are contiguous
 // in every component row, so thread k asks for row k of the list below -- one instruction per thread instead of one
 // prefetch per thread and component.  MG > 0 (per-robot gains): also the first MG rows of the motion-force task's gain block
-// and the joint task's 3 N gain rows (at most 2 N + 31 + 4 N + 24 + 3 N = 127 rows for eight joints).
-template <int N, int R, bool HAS_JT, int MG = 0>
+// and the joint task's 3 N gain rows (at most 2 N + 31 + 4 N + 24 + 3 N = 127 rows for eight joints).  SP (the instantiations
+// without MOTION, whose control law reads the per-robot spaces): also the motion-force task's space block when it has one, last,
+// so that in the one case with more rows than threads (eight joints and per-robot gains) only some of its rows go unrequested.
+template <int N, int R, bool HAS_JT, int MG = 0, bool SP = false>
 DEVI void prefetch_block_rows(const OscProgram& P, uint64_t blk) {
 	const uint64_t nrl = (uint64_t)P.n_robots;
 	const uint64_t b0 = blk * blockDim.x;
@@ -162,7 +164,7 @@ DEVI void prefetch_block_rows(const OscProgram& P, uint64_t blk) {
 				const int comp = (grp == 0 ? JC_GOAL_POS : grp == 1 ? JC_GOAL_VEL : grp == 2 ? JC_GOAL_ACC : JC_INT) + c;
 				row = (const char*)(jt.st + (uint64_t)comp * nrl);
 			}
-			if constexpr (MG > 0) k -= 4 * N;
+			if constexpr (MG > 0 || SP) k -= 4 * N;
 		}
 		if constexpr (MG > 0 && R > 0) {
 			if (k >= 0 && k < MG && P.mft[0].gains) row = (const char*)(P.mft[0].gains + (uint64_t)k * nrl);
@@ -172,6 +174,15 @@ DEVI void prefetch_block_rows(const OscProgram& P, uint64_t blk) {
 			if (k >= 0 && k < 3 * N && P.jt[0].gains) {
 				const int grp = k / N, c = k - grp * N;
 				row = (const char*)(P.jt[0].gains + (uint64_t)((grp == 0 ? JG_KP : grp == 1 ? JG_KV : JG_KI) + c) * nrl);
+			}
+			if constexpr (SP) k -= 3 * N;
+		}
+		if constexpr (SP && R > 0) {
+			if (k == 0 && P.mft[0].space_mode) {
+				row = (const char*)P.mft[0].space_mode;
+				esz = 4;
+			} else if (k >= 1 && k <= SP_AXES_COUNT && P.mft[0].space_axes) {
+				row = (const char*)(P.mft[0].space_axes + (uint64_t)(k - 1) * nrl);
 			}
 		}
 	}
@@ -269,9 +280,9 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 	constexpr int G = PRG ? GAINS_ROBOT : (SPEC || R == 0) ? GAINS_BCAST : GAINS_ANY;
 #ifndef OSC_NO_PREFETCH
 	if constexpr (PRG)
-		prefetch_block_rows<N, R, HAS_JT, MOTION ? MG_KP_FORCE : GAIN_COUNT>(P, blockIdx.x);
+		prefetch_block_rows<N, R, HAS_JT, MOTION ? MG_KP_FORCE : GAIN_COUNT, !MOTION>(P, blockIdx.x);
 	else
-		prefetch_block_rows<N, R, HAS_JT>(P, blockIdx.x);
+		prefetch_block_rows<N, R, HAS_JT, 0, !MOTION>(P, blockIdx.x);
 #endif
 	grid_dependency_wait(P);
 	stamp_block(P, 0);

@@ -173,9 +173,7 @@ static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
 			if (P.mft[0].full && blend_split_selected(P)) {
 				// hand-overs are expected (host hint): prefix / variants / fallback as three kernels, each grid-stride over
 				// its list with as many blocks as the device holds at once
-				const osc_mft_params& mp = P.mft[0].p;
-				const bool motion = mp.force_space_dimension == 0 && mp.moment_space_dimension == 0 && !mp.closed_loop_force_control &&
-									!mp.closed_loop_moment_control && !mp.use_velocity_saturation;
+				const bool motion = mft_pure_motion(P.mft[0]);
 				constexpr int vsmem = kBlendSmem ? blend_smem_doubles<N>() * kBlendBlock * (int)sizeof(double) : 0;
 				static_assert(vsmem <= 48 * 1024, "variants kernel: dynamic shared memory beyond the default limit");
 				static std::atomic<int> per_sm[64][3];

@@ -2,6 +2,7 @@
 // One OscProgram is passed to every kernel as a __grid_constant__ parameter, so its
 // members are served from the constant bank (warp-uniform broadcast reads).
 #pragma once
+#include <math.h>
 #include <stdint.h>
 
 #include "../../include/sai_b200_osc.h"
@@ -69,6 +70,57 @@ enum GainComp : int {
 	GAIN_COUNT = 24
 };
 
+// Per-robot force / moment spaces of a MotionForceTask (osc_mft_parametrize_spaces_batched): one mode word per robot
+// (bits 0-1 force space dimension, 2-3 moment space dimension, 4 closed-loop force, 5 closed-loop moment) and the
+// normalised axes, SoA SP_AXES_COUNT x N (force / motion axis in rows 0-2, moment / rot-motion axis in rows 3-5).
+// A word of 0 is pure motion control.
+enum SpaceBits : int32_t { SP_FDIM_SHIFT = 0, SP_MDIM_SHIFT = 2, SP_CL_FORCE = 16, SP_CL_MOMENT = 32, SP_AXES_COUNT = 6 };
+// host-side OR over the robots of a task (DevMft::space_any)
+enum SpaceSummary : int32_t { SPS_FORCE_DIM = 1, SPS_MOMENT_DIM = 2, SPS_CL_FORCE = 4, SPS_CL_MOMENT = 8 };
+#if defined(__CUDACC__)
+#define OSC_HD __host__ __device__ inline
+#else
+#define OSC_HD inline
+#endif
+OSC_HD int32_t space_mode_word(int fdim, int mdim, bool cl_force, bool cl_moment) {
+	return (int32_t)((fdim << SP_FDIM_SHIFT) | (mdim << SP_MDIM_SHIFT) | (cl_force ? SP_CL_FORCE : 0) | (cl_moment ? SP_CL_MOMENT : 0));
+}
+// Sums of squares without fused multiply-adds, so that the host and the kernels normalise an axis and take a reset decision
+// bit for bit alike (a broadcast call and a per-robot call with the same values give the same stored axes).
+OSC_HD double sq3_rn(double x, double y, double z) {
+#if defined(__CUDA_ARCH__)
+	return __dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z));
+#else
+	return x * x + y * y + z * z;
+#endif
+}
+// |axis|, and the normalised axis in u (MotionForceTask.cpp:838, :868)
+OSC_HD double space_normalize(const double axis[3], double u[3]) {
+	const double nrm = sqrt(sq3_rn(axis[0], axis[1], axis[2]));
+	for (int k = 0; k < 3; k++) u[k] = axis[k] / nrm;
+	return nrm;
+}
+// the reset rule of parametrizeForceMotionSpaces / parametrizeMomentRotMotionSpaces (MotionForceTask.cpp:845, :877): the new
+// normalised axis a is Eigen's isApprox to the stored axis b, |a - b|^2 <= 1e-24 min(|a|^2, |b|^2) with |a| = 1
+OSC_HD bool space_axis_is_approx(const double a[3], const double b[3]) {
+	const double d2 = sq3_rn(a[0] - b[0], a[1] - b[1], a[2] - b[2]), b2 = sq3_rn(b[0], b[1], b[2]);
+	return d2 <= 1e-24 * (b2 < 1.0 ? b2 : 1.0);
+}
+// Validation of per-robot values (SpaceCheck bits; SPC_NONZERO feeds the host's summary): a space dimension in 0..3 and, for
+// dimension 1 or 2, a finite axis of norm >= 1e-2; a closed-loop flag 0 or 1.
+enum SpaceCheck : int32_t { SPC_BAD_DIM = 1, SPC_BAD_AXIS = 2, SPC_BAD_FLAG = 4, SPC_NONZERO = 8 };
+OSC_HD int32_t space_check(int32_t dim, double a0, double a1, double a2) {
+	if (dim < 0 || dim > 3) return SPC_BAD_DIM;
+	if (dim == 0) return 0;
+	if (dim == 3) return SPC_NONZERO;
+	// x - x is 0 for a finite x and NaN for an infinite or NaN one
+	const bool finite = (a0 - a0) == 0.0 && (a1 - a1) == 0.0 && (a2 - a2) == 0.0;
+	const double axis[3] = {a0, a1, a2};
+	double u[3];
+	return (finite && space_normalize(axis, u) >= 1e-2) ? SPC_NONZERO : SPC_BAD_AXIS;
+}
+OSC_HD int32_t closed_loop_check(int32_t flag) { return flag == 0 ? 0 : flag == 1 ? SPC_NONZERO : SPC_BAD_FLAG; }
+
 #define OSC_HIST_MAX 256
 
 struct DevModel {
@@ -113,6 +165,10 @@ struct DevMft {
 	int32_t* ist;  // MI_COUNT x N
 	double* ring;  // ring_capacity x N (or null)
 	double* gains;	// per-robot PID gains, GAIN_COUNT x N (osc_set_gains); null: every robot uses those of p
+	// per-robot spaces and closed-loop flags (SpaceBits); null: every robot uses those of p
+	int32_t* space_mode;  // N
+	double* space_axes;	  // SP_AXES_COUNT x N
+	int32_t space_any;	  // SpaceSummary over the robots, kept by the host while space_mode is set
 	DevOtg otg;
 };
 

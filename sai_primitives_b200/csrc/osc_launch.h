@@ -48,6 +48,18 @@ inline double min_eig_sym3(const double* I) {
 	return q + 2.0 * p * std::cos(phi + 2.0 * 3.14159265358979323846 / 3.0);
 }
 
+// Every robot of the motion-force task is under pure motion control of a full task without velocity saturation, so the
+// MOTION instantiations, which never read the per-robot space block, compute what the general control law would: no force or
+// moment space and both loops open -- the task's parameters, or with per-robot spaces (osc_mft_parametrize_spaces_batched)
+// the host's summary over the robots.
+inline bool mft_pure_motion(const DevMft& t) {
+	const osc_mft_params& p = t.p;
+	const bool free = t.space_mode ? t.space_any == 0
+								   : (p.force_space_dimension == 0 && p.moment_space_dimension == 0 && !p.closed_loop_force_control &&
+									  !p.closed_loop_moment_control);
+	return t.full && free && !p.use_velocity_saturation;
+}
+
 // Conditions under which the specialised instantiation (SPEC, osc_cycle.cuh) computes the same thing as the general one.
 // *motion: the motion-force task additionally is a full task under pure motion control (the MOTION flag of the kernel)
 inline bool cycle_spec_eligible(const OscProgram& P, bool has_jt, bool* motion) {
@@ -71,12 +83,9 @@ inline bool cycle_spec_eligible(const OscProgram& P, bool has_jt, bool* motion) 
 		}
 		if (may_clamp > 1) return false;
 	}
-	const DevMft& t = P.mft[0];
-	const osc_mft_params& p = t.p;
 	// IMPEDANCE decoupling needs no code of its own (Lambda_modified = I: the solves are skipped); velocity saturation of the
 	// motion-force task is part of the general control law, which the structural specialisation (MOTION = false) keeps
-	*motion = t.full && p.force_space_dimension == 0 && p.moment_space_dimension == 0 && !p.closed_loop_force_control &&
-			  !p.closed_loop_moment_control && !p.use_velocity_saturation;
+	*motion = mft_pure_motion(P.mft[0]);
 	if (has_jt) {
 		const DevJt& j = P.jt[0];
 		if (!j.full || j.p.use_velocity_saturation) return false;  // the staged joint control law has no velocity saturation
@@ -119,6 +128,13 @@ cudaError_t launch_fill(double* st, int64_t NR, int comp, int ncomp, const doubl
 cudaError_t launch_copy(double* st, int64_t NR, int dst, int src, int ncomp, cudaStream_t stream);
 // *bad |= 1: some of the n values is not finite, |= 2: some is negative (*bad is not cleared)
 cudaError_t launch_check_values(const double* v, int64_t n, int32_t* bad, cudaStream_t stream);
+// per-robot force / moment spaces (osc_space_kernels.cuh).  check: *out |= SpaceCheck bits over the n robots (dims / axes and
+// flags may each be null).  apply: parametrize* per robot (dims == null: dim and axis for every robot).  moment: 0 force, 1 moment.
+cudaError_t launch_check_spaces(const int32_t* dims, const double* axes, const int32_t* flags, int64_t n, int32_t* out, cudaStream_t stream);
+cudaError_t launch_apply_spaces(const OscProgram& P, int mft_index, int moment, const int32_t* dims, const double* axes, int dim,
+								const double axis[3], int32_t* was_reset, int32_t* any_reset, cudaStream_t stream);
+cudaError_t launch_set_closed_loop(const OscProgram& P, int mft_index, int moment, const int32_t* flags, int flag, cudaStream_t stream);
+cudaError_t launch_get_spaces(const OscProgram& P, int mft_index, int moment, int32_t* dims, double* axes, int32_t* closed_loop, cudaStream_t stream);
 cudaError_t launch_fill_int(int32_t* ist, int64_t NR, int comp, int ncomp, int32_t value, cudaStream_t stream);
 
 }  // namespace osc

@@ -165,22 +165,23 @@ __global__ void __launch_bounds__(64) osc_observer_kernel(const __grid_constant_
 	}
 	// motion-force task observers from the state the last computeTorques left (current pose, orientation error) and the goals
 	const DevMft& t = P.mft[P.tasks[task].index];
-	const osc_mft_params& p = t.p;
 	double R[9];
 	for (int k = 0; k < 9; k++) R[k] = t.st[(int64_t)(MC_CUR_ORI + k) * NR + i];
-	double uf[3], um[3];
+	const int32_t mode = mft_space_mode(t, i);	// this robot's spaces, as the control law reads them
+	double af[3], am[3], uf[3], um[3];
+	mft_space_axes(t, NR, i, af, am);
 	if (t.in_compliant) {
-		mat3_vec(R, p.force_or_motion_axis, uf);
-		mat3_vec(R, p.moment_or_rotmotion_axis, um);
+		mat3_vec(R, af, uf);
+		mat3_vec(R, am, um);
 	} else {
 		for (int k = 0; k < 3; k++) {
-			uf[k] = p.force_or_motion_axis[k];
-			um[k] = p.moment_or_rotmotion_axis[k];
+			uf[k] = af[k];
+			um[k] = am[k];
 		}
 	}
 	double Sf[9], Sm[9], Sp[9], So[9];
-	sigma_space(p.force_space_dimension, t.Pt, uf, Sf);
-	sigma_space(p.moment_space_dimension, t.Pr, um, Sm);
+	sigma_space((mode >> SP_FDIM_SHIFT) & 3, t.Pt, uf, Sf);
+	sigma_space((mode >> SP_MDIM_SHIFT) & 3, t.Pr, um, Sm);
 	sigma_complement(t.Pt, Sf, Sp);
 	sigma_complement(t.Pr, Sm, So);
 	if (kind == OBS_POSITION_ERROR || kind == OBS_ORIENTATION_ERROR) {

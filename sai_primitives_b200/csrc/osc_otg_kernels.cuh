@@ -96,6 +96,37 @@ static __device__ __noinline__ void otg_cart_step(const DevMft& t, int64_t NR, i
 	otg_cart_write_desired(t, o, NR, i);
 }
 
+// Reset of robot i's generator by parametrizeForceMotionSpaces (reInitializeLinear, angular = false) or
+// parametrizeMomentRotMotionSpaces (reInitializeAngular) with the generator on: the user's goals of that part become the current
+// pose at rest, the generator restarts from there, and the desired state goes into the goal slots.
+static __device__ __noinline__ void otg_cart_reinit_part(const DevMft& t, int64_t NR, int64_t i, bool angular) {
+	const DevOtg& g = t.otg;
+	double x[3], R[9];
+	for (int c = 0; c < 3; c++) x[c] = t.st[(int64_t)(MC_CUR_POS + c) * NR + i];
+	for (int c = 0; c < 9; c++) R[c] = t.st[(int64_t)(MC_CUR_ORI + c) * NR + i];
+	otg::CartesianOtg o;
+	otg_load(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
+	o.g.flags = g.flags[i];
+	if (!angular) {
+		for (int c = 0; c < 3; c++) {
+			g.st[(int64_t)(OC_USER + MC_GOAL_POS + c) * NR + i] = x[c];
+			g.st[(int64_t)(OC_USER + MC_GOAL_LINVEL + c) * NR + i] = 0.0;
+			g.st[(int64_t)(OC_USER + MC_GOAL_LINACC + c) * NR + i] = 0.0;
+		}
+		o.reinitialize_linear(x);
+	} else {
+		for (int c = 0; c < 9; c++) g.st[(int64_t)(OC_USER + MC_GOAL_ORI + c) * NR + i] = R[c];
+		for (int c = 0; c < 3; c++) {
+			g.st[(int64_t)(OC_USER + MC_GOAL_ANGVEL + c) * NR + i] = 0.0;
+			g.st[(int64_t)(OC_USER + MC_GOAL_ANGACC + c) * NR + i] = 0.0;
+		}
+		o.reinitialize_angular(R);
+	}
+	otg_store(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
+	g.flags[i] = o.g.flags;
+	otg_cart_write_desired(t, o, NR, i);
+}
+
 // one launch per control cycle when any task has its generator on
 __global__ void __launch_bounds__(64) otg_update_kernel(const __grid_constant__ OscProgram P) {
 	const int64_t NR = P.n_robots;
@@ -169,6 +200,10 @@ __global__ void otg_init_kernel(const __grid_constant__ OscProgram P, int task, 
 		g.flags[i] |= otg::OTG_DIRTY;
 		return;
 	}
+	if (!fresh && (mode == 1 || mode == 2)) {
+		otg_cart_reinit_part(t, NR, i, mode == 2);
+		return;
+	}
 	double x[3], R[9];
 	for (int c = 0; c < 3; c++) x[c] = t.st[(int64_t)(MC_CUR_POS + c) * NR + i];
 	for (int c = 0; c < 9; c++) R[c] = t.st[(int64_t)(MC_CUR_ORI + c) * NR + i];
@@ -179,26 +214,10 @@ __global__ void otg_init_kernel(const __grid_constant__ OscProgram P, int task, 
 	} else {
 		otg_load(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
 		o.g.flags = g.flags[i];
-		if (mode == 0) {
-			for (int c = 0; c < 24; c++) g.st[(int64_t)(OC_USER + c) * NR + i] = 0.0;
-			for (int c = 0; c < 3; c++) g.st[(int64_t)(OC_USER + MC_GOAL_POS + c) * NR + i] = x[c];
-			for (int c = 0; c < 9; c++) g.st[(int64_t)(OC_USER + MC_GOAL_ORI + c) * NR + i] = R[c];
-			o.reinitialize(x, R);
-		} else if (mode == 1) {
-			for (int c = 0; c < 3; c++) {
-				g.st[(int64_t)(OC_USER + MC_GOAL_POS + c) * NR + i] = x[c];
-				g.st[(int64_t)(OC_USER + MC_GOAL_LINVEL + c) * NR + i] = 0.0;
-				g.st[(int64_t)(OC_USER + MC_GOAL_LINACC + c) * NR + i] = 0.0;
-			}
-			o.reinitialize_linear(x);
-		} else {
-			for (int c = 0; c < 9; c++) g.st[(int64_t)(OC_USER + MC_GOAL_ORI + c) * NR + i] = R[c];
-			for (int c = 0; c < 3; c++) {
-				g.st[(int64_t)(OC_USER + MC_GOAL_ANGVEL + c) * NR + i] = 0.0;
-				g.st[(int64_t)(OC_USER + MC_GOAL_ANGACC + c) * NR + i] = 0.0;
-			}
-			o.reinitialize_angular(R);
-		}
+		for (int c = 0; c < 24; c++) g.st[(int64_t)(OC_USER + c) * NR + i] = 0.0;  // mode 0
+		for (int c = 0; c < 3; c++) g.st[(int64_t)(OC_USER + MC_GOAL_POS + c) * NR + i] = x[c];
+		for (int c = 0; c < 9; c++) g.st[(int64_t)(OC_USER + MC_GOAL_ORI + c) * NR + i] = R[c];
+		o.reinitialize(x, R);
 	}
 	otg_store(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
 	g.flags[i] = o.g.flags;

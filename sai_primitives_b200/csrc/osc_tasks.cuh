@@ -187,6 +187,25 @@ DEVI void load_gain_block(const gdouble* blk, const double* pb, IDX NR, IDX i, i
 	 : G == GAINS_ROBOT ? kg[comp]                                        \
 						: (t.gains ? t.gains[(IDX)(comp) * NR + i] : p.member))
 
+// Force / moment spaces and closed-loop flags of robot i (SpaceBits): its row of the per-robot space block
+// (osc_mft_parametrize_spaces_batched), or, for a task without one, its parameters.
+template <typename IDX>
+DEVI int32_t mft_space_mode(const DevMft& t, IDX i) {
+	const osc_mft_params& p = t.p;
+	return t.space_mode ? t.space_mode[i]
+						: space_mode_word(p.force_space_dimension, p.moment_space_dimension, p.closed_loop_force_control != 0, p.closed_loop_moment_control != 0);
+}
+// the force / motion and moment / rot-motion axes of robot i as parametrised (compliant frame or world axes)
+template <typename IDX>
+DEVI void mft_space_axes(const DevMft& t, IDX NR, IDX i, double af[3], double am[3]) {
+	const osc_mft_params& p = t.p;
+#pragma unroll
+	for (int k = 0; k < 3; k++) {
+		af[k] = t.space_axes ? t.space_axes[(IDX)k * NR + i] : p.force_or_motion_axis[k];
+		am[k] = t.space_axes ? t.space_axes[(IDX)(3 + k) * NR + i] : p.moment_or_rotmotion_axis[k];
+	}
+}
+
 DEVI void scale_to_norm(double v[3], double maxn) {
 	const double n = sqrt(dot3(v, v));
 	if (n > maxn) {
@@ -263,9 +282,10 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 	orientation_error(Rd, R, ori_err_goal);	 // :291-292 (desired == goal with OTG off)
 
 	// Pure motion control of a full task (no force/moment space, open loop): every sigma is 0 or the identity
-	// (MotionForceTask.cpp:892-971), the force-related terms vanish and only the two PID laws remain.
-	if (MOTION || (t.full && p.force_space_dimension == 0 && p.moment_space_dimension == 0 && !p.closed_loop_force_control &&
-				   !p.closed_loop_moment_control)) {
+	// (MotionForceTask.cpp:892-971), the force-related terms vanish and only the two PID laws remain.  MOTION: known for every
+	// robot (host check); otherwise decided per robot from its mode word (a word of 0 is pure motion control).
+	const int32_t mode = MOTION ? 0 : mft_space_mode(t, i);
+	if (MOTION || (t.full && mode == 0)) {
 		double Ip[3], Io[3];
 		if (MOTION && sg) {
 #pragma unroll
@@ -323,26 +343,30 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 	if constexpr (MOTION) return false;
 	// selection matrices
 	const double I3[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+	const bool cl_force = (mode & SP_CL_FORCE) != 0, cl_moment = (mode & SP_CL_MOMENT) != 0;
 	double uf[3], um[3];
-	if (t.in_compliant) {
-		mat3_vec(R, p.force_or_motion_axis, uf);
-		mat3_vec(R, p.moment_or_rotmotion_axis, um);
-	} else {
+	{
+		double af[3], am[3];
+		mft_space_axes(t, NR, i, af, am);
+		if (t.in_compliant) {
+			mat3_vec(R, af, uf);
+			mat3_vec(R, am, um);
+		} else {
 #pragma unroll
-		for (int k = 0; k < 3; k++) {
-			uf[k] = p.force_or_motion_axis[k];
-			um[k] = p.moment_or_rotmotion_axis[k];
+			for (int k = 0; k < 3; k++) {
+				uf[k] = af[k];
+				um[k] = am[k];
+			}
 		}
 	}
 	double Sf[9], Sm[9], Sp[9], So[9];
-	sigma_space(p.force_space_dimension, t.Pt, uf, Sf);
-	sigma_space(p.moment_space_dimension, t.Pr, um, Sm);
+	sigma_space((mode >> SP_FDIM_SHIFT) & 3, t.Pt, uf, Sf);
+	sigma_space((mode >> SP_MDIM_SHIFT) & 3, t.Pr, um, Sm);
 	sigma_complement(t.Pt, Sf, Sp);
 	sigma_complement(t.Pr, Sm, So);
 
 	double gf_raw[3] = {0, 0, 0}, gm_raw[3] = {0, 0, 0}, gf[3], gm[3];
-	const bool any_force = (p.force_space_dimension != 0) || (p.moment_space_dimension != 0) ||
-						   p.closed_loop_force_control || p.closed_loop_moment_control;
+	const bool any_force = mode != 0;
 	if (any_force) {
 		load3(st, NR, i, MC_GOAL_FORCE, gf_raw);
 		load3(st, NR, i, MC_GOAL_MOMENT, gm_raw);
@@ -360,7 +384,7 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 
 	double force_fb[3], moment_fb[3];
 	// ---- force ----  :327-354
-	if (p.closed_loop_force_control) {
+	if (cl_force) {
 		double fs[3], If[3], e[3], se[3];
 		load3(st, NR, i, MC_SENSED_F, fs);
 		load3(st, NR, i, MC_INT_FORCE, If);
@@ -386,7 +410,7 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 		mat3_vec(Sf, pre, force_fb);
 	}
 	// ---- moment ----  :357-383
-	if (p.closed_loop_moment_control) {
+	if (cl_moment) {
 		double ms[3], Im[3], e[3], se[3];
 		load3(st, NR, i, MC_SENSED_M, ms);
 		load3(st, NR, i, MC_INT_MOMENT, Im);
@@ -469,7 +493,7 @@ DEVI bool mft_control_law(const DevMft& t, IDX NR, IDX i, const double x[3], con
 	double ff_f[3], ff_m[3];
 	mat3_vec(Sf, gf, ff_f);
 	mat3_vec(Sm, gm, ff_m);
-	if (p.closed_loop_force_control) {	// keyed on the force flag only (:484-487)
+	if (cl_force) {	 // keyed on the force flag only (:484-487)
 #pragma unroll
 		for (int k = 0; k < 3; k++) {
 			ff_f[k] *= p.kff_force;
