@@ -23,6 +23,9 @@
 // The bounded-inertia variant M_BIE = M + diag(d) is a rank-one update M + h h^T whenever a single
 // diagonal entry is clamped (always the case for the Panda: SURVEY.md Appendix D), handled by
 // Sherman-Morrison on the factors already at hand; several clamped entries take the general route.
+// When the null space is one-dimensional (the flagship: seven joints under a six-dof pure-motion task) the specialised
+// kernel needs neither X nor the QR: the null vector n of J_t and the Cholesky factor of G = J_t J_t^T give the task
+// torque and the joint task in closed form (RANK1 below, tests/test_rank_one_tail.py).
 // No singular value decomposition is needed on this (non-singular) branch: the branch
 // decision uses the sound spectral test in osc_math.cuh; robots that fail it are handed to the
 // general-path kernel (osc_singular.cuh) through a compacted list.
@@ -278,6 +281,10 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 	// where the control laws read the gains: a JointTask alone (R = 0) has a per-robot instantiation like the specialised kernels,
 	// the other non-specialised instantiations test the block pointer at run time
 	constexpr int G = PRG ? GAINS_ROBOT : (SPEC || R == 0) ? GAINS_BCAST : GAINS_ANY;
+	// task tail of a one-dimensional null space (the flagship: a 7-joint robot under a six-dof pure-motion task) built from
+	// the null vector of J_t instead of a Householder QR.  Every other signature keeps the QR route; in the specialisation
+	// without MOTION (general control law) the new tail would push the kernel, already at 255 registers, into more spills.
+	constexpr bool RANK1 = SPEC && MOTION && FULL && HAS_JT && R > 1 && N - R == 1;
 #ifndef OSC_NO_PREFETCH
 	if constexpr (PRG)
 		prefetch_block_rows<N, R, HAS_JT, MOTION ? MG_KP_FORCE : GAIN_COUNT, !MOTION>(P, blockIdx.x);
@@ -393,6 +400,7 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 		// staged in shared memory behind the factor (the joint axes and origins are dead after this loop)
 		double* Js = smt + (size_t)kSmFactor<N> * sms;
 		double v[3] = {0, 0, 0}, w[3] = {0, 0, 0};
+		double Cg[R][R], invc[R];  // RANK1: G = J_t J_t^T = C C^T
 		{
 			double G[R][R];
 #pragma unroll
@@ -463,7 +471,11 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 			// Branch decision of SingularityHandler::updateTaskModel (:83-105), taken before any task state is touched:
 			// robots that are not provably non-singular are appended (warp-aggregated) to the list of the general-path
 			// kernel and leave this kernel.
-			bool leave = !sound_nonsingular_gram<R>(G, p.s_max, p.s_abs_tol);
+			bool leave;
+			if constexpr (RANK1)
+				leave = !sound_nonsingular_gram_factor<R>(G, p.s_max, p.s_abs_tol, Cg, invc);
+			else
+				leave = !sound_nonsingular_gram<R>(G, p.s_max, p.s_abs_tol);
 			if constexpr (SPEC) {
 				// the specialisation carries the rank-zero and rank-one bounded-inertia updates only
 				double hh[N], dd;
@@ -535,285 +547,405 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 		}
 		OSC_LS_K();
 
-		// ---- X = L^-1 J_t^T row by row (row r needs column r of J only), operands from shared memory
-		double X[N][R];
+		if constexpr (RANK1) {
+			// ---- one-dimensional null space (N - R = 1, DESIGN.md section 4).  With G = J_t J_t^T = C C^T (factored with
+			// the branch test), column k of the projector I - J_t^T G^-1 J_t is parallel to the null vector n of J_t; the
+			// column with the largest diagonal entry 1 - |C^-1 J_k|^2 (at least 1/N) is taken.  The scale of n is free.
+			double ub[R], pbest = 0.0;
+			int kb = 0;
 #pragma unroll
-		for (int r = 0; r < N; r++) {
-			double cr[R];
+			for (int k = 0; k < N; k++) {
+				double u[R];
 #pragma unroll
-			for (int a = 0; a < R; a++) cr[a] = Js[(r * R + a) * sms];
+				for (int a = 0; a < R; a++) u[a] = Js[(k * R + a) * sms];
+				solve_lower<R>(Cg, invc, u);
+				double pk = 1.0;
 #pragma unroll
-			for (int k = 0; k < r; k++) {
-				const double l = Ls.L(r, k);
+				for (int a = 0; a < R; a++) pk -= u[a] * u[a];
+				const bool better = (k == 0) || pk > pbest;
+				pbest = better ? pk : pbest;
+				kb = better ? k : kb;
 #pragma unroll
-				for (int a = 0; a < R; a++) cr[a] -= l * X[k][a];
+				for (int a = 0; a < R; a++) ub[a] = better ? u[a] : ub[a];
 			}
-			const double inv = Ls.invd(r);
+			solve_lower_t<R>(Cg, invc, ub);	 // G^-1 J_kb
+			// v = J_t^T G^-1 f, the minimum-norm solution of J_t v = f: no component along n (impedance decoupling: J_t^T f)
+			const int dec = p.dynamic_decoupling_type;
+			if (dec != OSC_IMPEDANCE) solve_spd<R>(Cg, invc, yf);
+			double nv[N], tv[N];
 #pragma unroll
-			for (int a = 0; a < R; a++) X[r][a] = cr[a] * inv;
-		}
-		// the Jacobian columns are dead: their slots receive the joint task's goals, integrator and q, dq, requested now
-		// and read after the factorisation below
-		if constexpr (SPEC && HAS_JT) joint_stage_goals<N>(P.jt[0], P.q, P.dq, NR, i, smt + (size_t)kSmFactor<N> * sms, sms);
-		OSC_LS_K();
-		// bounded inertia estimates: M_BIE = M + diag(d); with one clamped entry: M + delta e e^T,
-		// g = L^-1 e, mu = g.g, z = J M^-1 e = X^T g
-		const int dec = p.dynamic_decoupling_type;
-		int kclamp = 0;
-		double z[R], mu = 0.0, delta = 0.0;
-		double h[N];
-		if (dec == OSC_BOUNDED_INERTIA_ESTIMATES) {
-			kclamp = bie_shift<N>(Mdiag, p.bie_threshold, h, delta);
-			if (kclamp == 1) {
-				double g[N];
-#pragma unroll
-				for (int j = 0; j < N; j++) g[j] = (h[j] > 0.0) ? 1.0 : 0.0;
-				Ls.solve_lower(g);
-#pragma unroll
-				for (int j = 0; j < N; j++) mu += g[j] * g[j];
+			for (int j = 0; j < N; j++) {
+				double sn = (j == kb) ? 1.0 : 0.0, sv = 0.0, sF = 0.0;
 #pragma unroll
 				for (int a = 0; a < R; a++) {
-					double s = 0.0;
-#pragma unroll
-					for (int j = 0; j < N; j++) s += X[j][a] * g[j];
-					z[a] = s;
+					const double c = Js[(j * R + a) * sms];
+					sn -= c * ub[a];
+					sv += c * yf[a];
+					sF += c * yF[a];
 				}
+				nv[j] = sn;
+				tv[j] = sv;
+				if (has_F) tau[j] += sF;
 			}
-		}
-		OSC_LS_K();
-		double vhead[R], beta[R], rinv[R];
-		householder_qr<N, R, 0>(X, vhead, beta, rinv);
-		OSC_LS_K();
+			// the Jacobian columns are dead: their slots receive the joint task's goals, integrator and q, dq, requested now
+			// and read after the task torque below
+			joint_stage_goals<N>(P.jt[0], P.q, P.dq, NR, i, smt + (size_t)kSmFactor<N> * sms, sms);
+			OSC_LS_K();
+			// tau_task = J_t^T Lambda_b f = M_b v - M_b n (n . M_b v) / (n . M_b n),  M_b = M + diag(d): the two projectors
+			// M_b^-1 J_t^T Lambda_b J_t and n (n^T M_b n)^-1 n^T M_b are M_b-orthogonal and add up to I
+			double Mn[N], Mv[N], dm[N], dsum;
+			Ls.mul_llt(nv, Mn);
+			Ls.mul_llt(tv, Mv);
+			if (dec == OSC_BOUNDED_INERTIA_ESTIMATES)
+				bie_shift<N>(Mdiag, p.bie_threshold, dm, dsum);
+			else {
+#pragma unroll
+				for (int j = 0; j < N; j++) dm[j] = 0.0;
+			}
+			double Mbn[N], nMbv = 0.0, nMbn = 0.0;
+#pragma unroll
+			for (int j = 0; j < N; j++) {
+				Mv[j] += dm[j] * tv[j];
+				Mbn[j] = Mn[j] + dm[j] * nv[j];
+				nMbv += nv[j] * Mv[j];
+				nMbn += nv[j] * Mbn[j];
+			}
+			const double cf = div_nz(nMbv, nMbn);
+#pragma unroll
+			for (int j = 0; j < N; j++) tau[j] += (dec == OSC_IMPEDANCE) ? tv[j] : Mv[j] - Mbn[j] * cf;
+			OSC_LS_K();
 
-		if (dec == OSC_FULL_DYNAMIC_DECOUPLING || (dec == OSC_BOUNDED_INERTIA_ESTIMATES && kclamp == 0)) {
-			solve_rtr<N, R, 0>(X, rinv, yf);
-		} else if (dec == OSC_BOUNDED_INERTIA_ESTIMATES && kclamp == 1) {
-			// (A - delta z z^T / (1 + delta mu))^-1 y = A^-1 y + (A^-1 z) (z . A^-1 y) delta / ((1 + delta mu) - delta z . A^-1 z)
-			double sz[R];
-#pragma unroll
-			for (int a = 0; a < R; a++) sz[a] = z[a];
-			solve_rtr<N, R, 0>(X, rinv, sz);
-			solve_rtr<N, R, 0>(X, rinv, yf);
-			double zs = 0.0, zt = 0.0;
-#pragma unroll
-			for (int a = 0; a < R; a++) {
-				zs += z[a] * sz[a];
-				zt += z[a] * yf[a];
-			}
-			const double f = delta * zt / ((1.0 + delta * mu) - delta * zs);
-#pragma unroll
-			for (int a = 0; a < R; a++) yf[a] += sz[a] * f;
-		}
-		else if (!SPEC && dec == OSC_BOUNDED_INERTIA_ESTIMATES) {
-			// general route (two or more clamped entries): A_b = W^T W, W = L_b^-1 J_t^T with J_t^T = L Q [R; 0]
-			double Lf[N][N], Lb[N][N], invdb[N];
-#pragma unroll
-			for (int r = 0; r < N; r++)
-#pragma unroll
-				for (int c = 0; c <= r; c++) Lf[r][c] = Ls.L(r, c);
-			bie_cholesky_from_factor<N>(Lf, h, Lb, invdb);
-			double Wb[N][R];
-#pragma unroll
-			for (int a = 0; a < R; a++) {
-				double e[N], col[N];
-#pragma unroll
-				for (int j = 0; j < N; j++) e[j] = (j <= a) ? X[j][a] : 0.0;  // column a of [R; 0]
-				apply_q<N, R, 0>(X, vhead, beta, e);
-				mul_lower<N>(Lf, e, col);
-				solve_lower<N>(Lb, invdb, col);
-#pragma unroll
-				for (int j = 0; j < N; j++) Wb[j][a] = col[j];
-			}
-			double Ab[R][R], invda[R];
-#pragma unroll
-			for (int a = 0; a < R; a++)
-#pragma unroll
-				for (int b = 0; b <= a; b++) {
-					double s = 0.0;
-#pragma unroll
-					for (int j = 0; j < N; j++) s += Wb[j][a] * Wb[j][b];
-					Ab[a][b] = s;
-				}
-			cholesky_lower<R>(Ab, invda);
-			solve_spd<R>(Ab, invda, yf);
-		}  // IMPEDANCE: Lambda_modified = I
-		OSC_LS_K();
-		// tau_task = J_t^T y = L Q [R y; 0]
-		{
-			if (has_F) {
-#pragma unroll
-				for (int a = 0; a < R; a++) yf[a] += yF[a];
-			}
-			double e[N], lt[N];
-#pragma unroll
-			for (int r = 0; r < N; r++) {
-				double s = 0.0;
-				if (r < R) {
-#pragma unroll
-					for (int a = r; a < R; a++) s += X[r][a] * yf[a];
-				}
-				e[r] = s;
-			}
-			apply_q<N, R, 0>(X, vhead, beta, e);
-			Ls.mul_lower(e, lt);
-#pragma unroll
-			for (int j = 0; j < N; j++) tau[j] += lt[j];
-		}
-
-		if constexpr (HAS_JT) {
+			// ---- joint task in the null space, s = n . M n, m = M^-1 n:
+			//   tau_jt = M n [ (n . qdd_d - m . tau_task) / (n . n) + (n . pid) / ((n . n) h) ]
+			// h = 1 under full decoupling; with one clamped entry e of M_b = M + delta e e^T, h = 1 - delta n_e^2 / (s (1 + delta mu)),
+			// mu = |L^-1 e|^2; impedance decoupling: (n . pid) / s
 			const DevJt& jt = P.jt[0];
 			const osc_joint_params& jp = jt.p;
-			constexpr int Mn = N - R;  // dimension of the remaining null space
-			if constexpr (Mn == 0) {
-				status |= OSC_STATUS_ZERO_RANGE;  // JointTask.cpp:234-239, 302-306
-			} else {
-				double pid[N], acc[N];
+			double m[N];
 #pragma unroll
-				for (int j = 0; j < N; j++) pid[j] = acc[j] = 0.0;
-				if constexpr (SPEC) {
-					if (alive) joint_control_law_staged<N, IDX, G>(jt, NR, i, smt + (size_t)kSmFactor<N> * sms, sms, pid, acc);
-				} else if (alive) {
-					double qj[N], dqj[N];  // re-read (L2 hot) rather than kept live across the task above
+			for (int j = 0; j < N; j++) m[j] = nv[j];
+			Ls.solve_lower(m);
+			Ls.solve_lower_t(m);
+			double pid[N], acc[N];
+#pragma unroll
+			for (int j = 0; j < N; j++) pid[j] = acc[j] = 0.0;
+			if (alive) joint_control_law_staged<N, IDX, G>(jt, NR, i, smt + (size_t)kSmFactor<N> * sms, sms, pid, acc);
+			double nn = 0.0, s = 0.0, mm = 0.0, na = 0.0, np = 0.0, mt = 0.0;
+#pragma unroll
+			for (int j = 0; j < N; j++) {
+				nn += nv[j] * nv[j];
+				s += nv[j] * Mn[j];
+				mm += Mn[j] * Mn[j];
+				na += nv[j] * acc[j];
+				np += nv[j] * pid[j];
+				mt += m[j] * tau[j];
+			}
+			// ||N_prec||_F^2 = (n . n)(M n . M n) / s^2 must stay < 1e6 for the reference's 1e-3 range tolerance
+			if (!(nn * mm < 1.0e6 * (s * s))) status |= OSC_STATUS_UNHANDLED;
+			const double inn = rcp_nz(nn);
+			double zp = inn;
+			const int jdec = jp.dynamic_decoupling_type;
+			if (jdec == OSC_IMPEDANCE)
+				zp = rcp_nz(s);
+			else if (jdec == OSC_BOUNDED_INERTIA_ESTIMATES) {
+				double hj[N], dj;
+				if (bie_shift<N>(Mdiag, jp.bie_threshold, hj, dj) == 1) {
+					double g[N], ne = 0.0, mu = 0.0;
 #pragma unroll
 					for (int j = 0; j < N; j++) {
-						qj[j] = P.q[(IDX)j * NR + i];
-						dqj[j] = P.dq[(IDX)j * NR + i];
+						g[j] = (hj[j] > 0.0) ? 1.0 : 0.0;
+						ne += (hj[j] > 0.0) ? nv[j] : 0.0;
 					}
-					joint_control_law<N, N, SPEC>(jt, NR, i, qj, dqj, pid, acc);
+					Ls.solve_lower(g);
+#pragma unroll
+					for (int j = 0; j < N; j++) mu += g[j] * g[j];
+					zp = div_nz(inn, 1.0 - dj * ne * ne * rcp_nz(s * (1.0 + dj * mu)));
 				}
-		OSC_LS_K();
-				// Q_perp = H_1..H_R [0; I],  W = L^-T Q_perp,  K = L Q_perp
-				double Qp[N][Mn], W[N][Mn], K[N][Mn];
+			}
+			const double zc = (na - (P.use_prev_torques ? mt : 0.0)) * inn + np * zp;
 #pragma unroll
-				for (int a = 0; a < Mn; a++) {
-					double e[N];
-#pragma unroll
-					for (int j = 0; j < N; j++) e[j] = (j == R + a) ? 1.0 : 0.0;
+			for (int j = 0; j < N; j++) tau[j] += Mn[j] * zc;
+		} else {
+			// ---- X = L^-1 J_t^T row by row (row r needs column r of J only), operands from shared memory
+			double X[N][R];
+	#pragma unroll
+			for (int r = 0; r < N; r++) {
+				double cr[R];
+	#pragma unroll
+				for (int a = 0; a < R; a++) cr[a] = Js[(r * R + a) * sms];
+	#pragma unroll
+				for (int k = 0; k < r; k++) {
+					const double l = Ls.L(r, k);
+	#pragma unroll
+					for (int a = 0; a < R; a++) cr[a] -= l * X[k][a];
+				}
+				const double inv = Ls.invd(r);
+	#pragma unroll
+				for (int a = 0; a < R; a++) X[r][a] = cr[a] * inv;
+			}
+			// the Jacobian columns are dead: their slots receive the joint task's goals, integrator and q, dq, requested now
+			// and read after the factorisation below
+			if constexpr (SPEC && HAS_JT) joint_stage_goals<N>(P.jt[0], P.q, P.dq, NR, i, smt + (size_t)kSmFactor<N> * sms, sms);
+			OSC_LS_K();
+			// bounded inertia estimates: M_BIE = M + diag(d); with one clamped entry: M + delta e e^T,
+			// g = L^-1 e, mu = g.g, z = J M^-1 e = X^T g
+			const int dec = p.dynamic_decoupling_type;
+			int kclamp = 0;
+			double z[R], mu = 0.0, delta = 0.0;
+			double h[N];
+			if (dec == OSC_BOUNDED_INERTIA_ESTIMATES) {
+				kclamp = bie_shift<N>(Mdiag, p.bie_threshold, h, delta);
+				if (kclamp == 1) {
+					double g[N];
+	#pragma unroll
+					for (int j = 0; j < N; j++) g[j] = (h[j] > 0.0) ? 1.0 : 0.0;
+					Ls.solve_lower(g);
+	#pragma unroll
+					for (int j = 0; j < N; j++) mu += g[j] * g[j];
+	#pragma unroll
+					for (int a = 0; a < R; a++) {
+						double s = 0.0;
+	#pragma unroll
+						for (int j = 0; j < N; j++) s += X[j][a] * g[j];
+						z[a] = s;
+					}
+				}
+			}
+			OSC_LS_K();
+			double vhead[R], beta[R], rinv[R];
+			householder_qr<N, R, 0>(X, vhead, beta, rinv);
+			OSC_LS_K();
+
+			if (dec == OSC_FULL_DYNAMIC_DECOUPLING || (dec == OSC_BOUNDED_INERTIA_ESTIMATES && kclamp == 0)) {
+				solve_rtr<N, R, 0>(X, rinv, yf);
+			} else if (dec == OSC_BOUNDED_INERTIA_ESTIMATES && kclamp == 1) {
+				// (A - delta z z^T / (1 + delta mu))^-1 y = A^-1 y + (A^-1 z) (z . A^-1 y) delta / ((1 + delta mu) - delta z . A^-1 z)
+				double sz[R];
+	#pragma unroll
+				for (int a = 0; a < R; a++) sz[a] = z[a];
+				solve_rtr<N, R, 0>(X, rinv, sz);
+				solve_rtr<N, R, 0>(X, rinv, yf);
+				double zs = 0.0, zt = 0.0;
+	#pragma unroll
+				for (int a = 0; a < R; a++) {
+					zs += z[a] * sz[a];
+					zt += z[a] * yf[a];
+				}
+				const double f = delta * zt / ((1.0 + delta * mu) - delta * zs);
+	#pragma unroll
+				for (int a = 0; a < R; a++) yf[a] += sz[a] * f;
+			}
+			else if (!SPEC && dec == OSC_BOUNDED_INERTIA_ESTIMATES) {
+				// general route (two or more clamped entries): A_b = W^T W, W = L_b^-1 J_t^T with J_t^T = L Q [R; 0]
+				double Lf[N][N], Lb[N][N], invdb[N];
+	#pragma unroll
+				for (int r = 0; r < N; r++)
+	#pragma unroll
+					for (int c = 0; c <= r; c++) Lf[r][c] = Ls.L(r, c);
+				bie_cholesky_from_factor<N>(Lf, h, Lb, invdb);
+				double Wb[N][R];
+	#pragma unroll
+				for (int a = 0; a < R; a++) {
+					double e[N], col[N];
+	#pragma unroll
+					for (int j = 0; j < N; j++) e[j] = (j <= a) ? X[j][a] : 0.0;  // column a of [R; 0]
 					apply_q<N, R, 0>(X, vhead, beta, e);
-					double k[N];
-					Ls.mul_lower(e, k);
-#pragma unroll
-					for (int j = 0; j < N; j++) Qp[j][a] = e[j];
-					Ls.solve_lower_t(e);
-#pragma unroll
-					for (int j = 0; j < N; j++) {
-						W[j][a] = e[j];
-						K[j][a] = k[j];
-					}
+					mul_lower<N>(Lf, e, col);
+					solve_lower<N>(Lb, invdb, col);
+	#pragma unroll
+					for (int j = 0; j < N; j++) Wb[j][a] = col[j];
 				}
-				double G[Mn][Mn], invg[Mn];
-				double nrm_chk = 0.0;
-#pragma unroll
-				for (int a = 0; a < Mn; a++)
-#pragma unroll
+				double Ab[R][R], invda[R];
+	#pragma unroll
+				for (int a = 0; a < R; a++)
+	#pragma unroll
 					for (int b = 0; b <= a; b++) {
-						double s = 0.0, kk = 0.0;
-#pragma unroll
-						for (int j = 0; j < N; j++) {
-							s += W[j][a] * W[j][b];
-							kk += K[j][a] * K[j][b];
-						}
-						G[a][b] = s;
-						nrm_chk += (a == b) ? s * kk : 2.0 * s * kk;
+						double s = 0.0;
+	#pragma unroll
+						for (int j = 0; j < N; j++) s += Wb[j][a] * Wb[j][b];
+						Ab[a][b] = s;
 					}
-				// ||N_prec||_F^2 = tr(G K^T K) must stay < 1e6 for the reference's 1e-3 range tolerance
-				if (!(nrm_chk < 1.0e6)) status |= OSC_STATUS_UNHANDLED;
-				cholesky_lower<Mn>(G, invg);
-		OSC_LS_K();
-				// u = W^T (qdd_d - M^-1 tau_prec)
-				double rhs[N];
-				if (P.use_prev_torques) {
-#pragma unroll
-					for (int j = 0; j < N; j++) rhs[j] = tau[j];
-					Ls.solve_lower(rhs);
-					Ls.solve_lower_t(rhs);
-#pragma unroll
-					for (int j = 0; j < N; j++) rhs[j] = acc[j] - rhs[j];
-				} else {
-#pragma unroll
-					for (int j = 0; j < N; j++) rhs[j] = acc[j];
+				cholesky_lower<R>(Ab, invda);
+				solve_spd<R>(Ab, invda, yf);
+			}  // IMPEDANCE: Lambda_modified = I
+			OSC_LS_K();
+			// tau_task = J_t^T y = L Q [R y; 0]
+			{
+				if (has_F) {
+	#pragma unroll
+					for (int a = 0; a < R; a++) yf[a] += yF[a];
 				}
-				double z1[Mn], z2[Mn];
-#pragma unroll
-				for (int a = 0; a < Mn; a++) {
-					double s1 = 0.0, s2 = 0.0;
-#pragma unroll
-					for (int j = 0; j < N; j++) {
-						s1 += W[j][a] * rhs[j];
-						s2 += W[j][a] * pid[j];
-					}
-					z1[a] = s1;
-					z2[a] = s2;
-				}
-				solve_spd<Mn>(G, invg, z1);
-				const int jdec = jp.dynamic_decoupling_type;
-				if (jdec == OSC_FULL_DYNAMIC_DECOUPLING) {
-					solve_spd<Mn>(G, invg, z2);
-				} else if (jdec == OSC_BOUNDED_INERTIA_ESTIMATES) {
-					solve_spd<Mn>(G, invg, z2);
-					double hj[N], dj = 0.0;
-					const int kj = bie_shift<N>(Mdiag, jp.bie_threshold, hj, dj);
-					if (kj == 1) {
-						// H = K^T M_b^-1 K = I - delta c c^T / (1 + delta mu),  c = Q_perp^T L^-1 e;
-						// H^-1 z = z + c (c . z) delta / ((1 + delta mu) - delta c . c)
-						double g[N];
-#pragma unroll
-						for (int j = 0; j < N; j++) g[j] = (hj[j] > 0.0) ? 1.0 : 0.0;
-						Ls.solve_lower(g);
-						double muj = 0.0;
-#pragma unroll
-						for (int j = 0; j < N; j++) muj += g[j] * g[j];
-						double c[Mn], cc = 0.0, cz = 0.0;
-#pragma unroll
-						for (int a = 0; a < Mn; a++) {
-							double s = 0.0;
-#pragma unroll
-							for (int j = 0; j < N; j++) s += Qp[j][a] * g[j];
-							c[a] = s;
-							cc += s * s;
-							cz += s * z2[a];
-						}
-						const double f = dj * cz / ((1.0 + dj * muj) - dj * cc);
-#pragma unroll
-						for (int a = 0; a < Mn; a++) z2[a] += c[a] * f;
-					}
-					else if (!SPEC && kj >= 2) {
-						double Lf[N][N], Lb[N][N], invdb[N];
-#pragma unroll
-						for (int r = 0; r < N; r++)
-#pragma unroll
-							for (int c = 0; c <= r; c++) Lf[r][c] = Ls.L(r, c);
-						bie_cholesky_from_factor<N>(Lf, hj, Lb, invdb);
-						double Z[N][Mn];
-#pragma unroll
-						for (int a = 0; a < Mn; a++) {
-							double col[N];
-#pragma unroll
-							for (int j = 0; j < N; j++) col[j] = K[j][a];
-							solve_lower<N>(Lb, invdb, col);
-#pragma unroll
-							for (int j = 0; j < N; j++) Z[j][a] = col[j];
-						}
-						double H[Mn][Mn], invh[Mn];
-#pragma unroll
-						for (int a = 0; a < Mn; a++)
-#pragma unroll
-							for (int b = 0; b <= a; b++) {
-								double s = 0.0;
-#pragma unroll
-								for (int j = 0; j < N; j++) s += Z[j][a] * Z[j][b];
-								H[a][b] = s;
-							}
-						cholesky_lower<Mn>(H, invh);
-						solve_spd<Mn>(H, invh, z2);
-					}
-				}  // IMPEDANCE: z2 = W^T t
-#pragma unroll
-				for (int j = 0; j < N; j++) {
+				double e[N], lt[N];
+	#pragma unroll
+				for (int r = 0; r < N; r++) {
 					double s = 0.0;
-#pragma unroll
-					for (int a = 0; a < Mn; a++) s += K[j][a] * (z1[a] + z2[a]);
-					tau[j] += s;
+					if (r < R) {
+	#pragma unroll
+						for (int a = r; a < R; a++) s += X[r][a] * yf[a];
+					}
+					e[r] = s;
+				}
+				apply_q<N, R, 0>(X, vhead, beta, e);
+				Ls.mul_lower(e, lt);
+	#pragma unroll
+				for (int j = 0; j < N; j++) tau[j] += lt[j];
+			}
+
+			if constexpr (HAS_JT) {
+				const DevJt& jt = P.jt[0];
+				const osc_joint_params& jp = jt.p;
+				constexpr int Mn = N - R;  // dimension of the remaining null space
+				if constexpr (Mn == 0) {
+					status |= OSC_STATUS_ZERO_RANGE;  // JointTask.cpp:234-239, 302-306
+				} else {
+					double pid[N], acc[N];
+	#pragma unroll
+					for (int j = 0; j < N; j++) pid[j] = acc[j] = 0.0;
+					if constexpr (SPEC) {
+						if (alive) joint_control_law_staged<N, IDX, G>(jt, NR, i, smt + (size_t)kSmFactor<N> * sms, sms, pid, acc);
+					} else if (alive) {
+						double qj[N], dqj[N];  // re-read (L2 hot) rather than kept live across the task above
+	#pragma unroll
+						for (int j = 0; j < N; j++) {
+							qj[j] = P.q[(IDX)j * NR + i];
+							dqj[j] = P.dq[(IDX)j * NR + i];
+						}
+						joint_control_law<N, N, SPEC>(jt, NR, i, qj, dqj, pid, acc);
+					}
+			OSC_LS_K();
+					// Q_perp = H_1..H_R [0; I],  W = L^-T Q_perp,  K = L Q_perp
+					double Qp[N][Mn], W[N][Mn], K[N][Mn];
+	#pragma unroll
+					for (int a = 0; a < Mn; a++) {
+						double e[N];
+	#pragma unroll
+						for (int j = 0; j < N; j++) e[j] = (j == R + a) ? 1.0 : 0.0;
+						apply_q<N, R, 0>(X, vhead, beta, e);
+						double k[N];
+						Ls.mul_lower(e, k);
+	#pragma unroll
+						for (int j = 0; j < N; j++) Qp[j][a] = e[j];
+						Ls.solve_lower_t(e);
+	#pragma unroll
+						for (int j = 0; j < N; j++) {
+							W[j][a] = e[j];
+							K[j][a] = k[j];
+						}
+					}
+					double G[Mn][Mn], invg[Mn];
+					double nrm_chk = 0.0;
+	#pragma unroll
+					for (int a = 0; a < Mn; a++)
+	#pragma unroll
+						for (int b = 0; b <= a; b++) {
+							double s = 0.0, kk = 0.0;
+	#pragma unroll
+							for (int j = 0; j < N; j++) {
+								s += W[j][a] * W[j][b];
+								kk += K[j][a] * K[j][b];
+							}
+							G[a][b] = s;
+							nrm_chk += (a == b) ? s * kk : 2.0 * s * kk;
+						}
+					// ||N_prec||_F^2 = tr(G K^T K) must stay < 1e6 for the reference's 1e-3 range tolerance
+					if (!(nrm_chk < 1.0e6)) status |= OSC_STATUS_UNHANDLED;
+					cholesky_lower<Mn>(G, invg);
+			OSC_LS_K();
+					// u = W^T (qdd_d - M^-1 tau_prec)
+					double rhs[N];
+					if (P.use_prev_torques) {
+	#pragma unroll
+						for (int j = 0; j < N; j++) rhs[j] = tau[j];
+						Ls.solve_lower(rhs);
+						Ls.solve_lower_t(rhs);
+	#pragma unroll
+						for (int j = 0; j < N; j++) rhs[j] = acc[j] - rhs[j];
+					} else {
+	#pragma unroll
+						for (int j = 0; j < N; j++) rhs[j] = acc[j];
+					}
+					double z1[Mn], z2[Mn];
+	#pragma unroll
+					for (int a = 0; a < Mn; a++) {
+						double s1 = 0.0, s2 = 0.0;
+	#pragma unroll
+						for (int j = 0; j < N; j++) {
+							s1 += W[j][a] * rhs[j];
+							s2 += W[j][a] * pid[j];
+						}
+						z1[a] = s1;
+						z2[a] = s2;
+					}
+					solve_spd<Mn>(G, invg, z1);
+					const int jdec = jp.dynamic_decoupling_type;
+					if (jdec == OSC_FULL_DYNAMIC_DECOUPLING) {
+						solve_spd<Mn>(G, invg, z2);
+					} else if (jdec == OSC_BOUNDED_INERTIA_ESTIMATES) {
+						solve_spd<Mn>(G, invg, z2);
+						double hj[N], dj = 0.0;
+						const int kj = bie_shift<N>(Mdiag, jp.bie_threshold, hj, dj);
+						if (kj == 1) {
+							// H = K^T M_b^-1 K = I - delta c c^T / (1 + delta mu),  c = Q_perp^T L^-1 e;
+							// H^-1 z = z + c (c . z) delta / ((1 + delta mu) - delta c . c)
+							double g[N];
+	#pragma unroll
+							for (int j = 0; j < N; j++) g[j] = (hj[j] > 0.0) ? 1.0 : 0.0;
+							Ls.solve_lower(g);
+							double muj = 0.0;
+	#pragma unroll
+							for (int j = 0; j < N; j++) muj += g[j] * g[j];
+							double c[Mn], cc = 0.0, cz = 0.0;
+	#pragma unroll
+							for (int a = 0; a < Mn; a++) {
+								double s = 0.0;
+	#pragma unroll
+								for (int j = 0; j < N; j++) s += Qp[j][a] * g[j];
+								c[a] = s;
+								cc += s * s;
+								cz += s * z2[a];
+							}
+							const double f = dj * cz / ((1.0 + dj * muj) - dj * cc);
+	#pragma unroll
+							for (int a = 0; a < Mn; a++) z2[a] += c[a] * f;
+						}
+						else if (!SPEC && kj >= 2) {
+							double Lf[N][N], Lb[N][N], invdb[N];
+	#pragma unroll
+							for (int r = 0; r < N; r++)
+	#pragma unroll
+								for (int c = 0; c <= r; c++) Lf[r][c] = Ls.L(r, c);
+							bie_cholesky_from_factor<N>(Lf, hj, Lb, invdb);
+							double Z[N][Mn];
+	#pragma unroll
+							for (int a = 0; a < Mn; a++) {
+								double col[N];
+	#pragma unroll
+								for (int j = 0; j < N; j++) col[j] = K[j][a];
+								solve_lower<N>(Lb, invdb, col);
+	#pragma unroll
+								for (int j = 0; j < N; j++) Z[j][a] = col[j];
+							}
+							double H[Mn][Mn], invh[Mn];
+	#pragma unroll
+							for (int a = 0; a < Mn; a++)
+	#pragma unroll
+								for (int b = 0; b <= a; b++) {
+									double s = 0.0;
+	#pragma unroll
+									for (int j = 0; j < N; j++) s += Z[j][a] * Z[j][b];
+									H[a][b] = s;
+								}
+							cholesky_lower<Mn>(H, invh);
+							solve_spd<Mn>(H, invh, z2);
+						}
+					}  // IMPEDANCE: z2 = W^T t
+	#pragma unroll
+					for (int j = 0; j < N; j++) {
+						double s = 0.0;
+	#pragma unroll
+						for (int a = 0; a < Mn; a++) s += K[j][a] * (z1[a] + z2[a]);
+						tau[j] += s;
+					}
 				}
 			}
 		}
