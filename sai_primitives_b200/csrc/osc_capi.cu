@@ -1470,7 +1470,7 @@ int osc_enable_joint_limit_avoidance(osc_handle* h, int enabled) {
 int osc_set_precision(osc_handle* h, int precision) {
 	ENTER(h);
 	if (precision != OSC_PRECISION_FP64 && precision != OSC_PRECISION_FP32) return fail(h, OSC_ERR_INVALID_ARGUMENT, "precision must be OSC_PRECISION_FP64 or OSC_PRECISION_FP32");
-	if (precision == OSC_PRECISION_FP32 && !osc::fused_f32_available(h->model.n))
+	if (precision == OSC_PRECISION_FP32 && !osc::cycle_f32_dof(h->model.n))
 		return fail(h, OSC_ERR_UNSUPPORTED, "FP32 mode: no single-precision kernel compiled for this robot dof");
 	h->prog.precision_fp32 = (precision == OSC_PRECISION_FP32) ? 1 : 0;
 	return OSC_OK;
@@ -1536,19 +1536,6 @@ static int run_cycle(osc_handle* h, double* tau_out, int mem_kind, bool sync_hos
 	if (!h->finalized) return fail(h, OSC_ERR_STATE, "controller not finalized");
 	if (!tau_out) return fail(h, OSC_ERR_INVALID_ARGUMENT, "null torque output");
 	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
-	if (h->prog.precision_fp32) {  // decided before anything is launched or counted: a refused cycle leaves the handle as it was
-		bool motion = false;
-		if (!(h->sig_R == 6 && h->prog.mft[0].full && osc::cycle_spec_eligible(h->prog, h->sig_jt, &motion) && motion && osc::fused_f32_available(h->model.n)))
-			return fail(h, OSC_ERR_UNSUPPORTED,
-						"FP32 mode covers a full six-dof MotionForceTask under pure motion control (alone or with a full JointTask) on an all-revolute-z chain only");
-		for (int k = 0; k < 2; k++)
-			if (h->prog.mft[k].gains || h->prog.jt[k].gains)
-				return fail(h, OSC_ERR_UNSUPPORTED, "FP32 mode: the kernels have no single-precision form with per-robot gains (osc_set_gains)");
-	}
-	h->prog.tau = (mem_kind == OSC_MEM_DEVICE) ? tau_out : h->d_tau;
-	h->prog.update_models = h->models_armed ? 1 : 0;
-	h->models_armed = false;
-	h->prog.epoch += 1;
 	// scheduling hint only (any grid size is correct): after a few cycles without hand-overs a handful of general-path blocks
 	// is launched instead of a grid that covers the machine
 	if (h->h_seen) {
@@ -1588,26 +1575,30 @@ static int run_cycle(osc_handle* h, double* tau_out, int mem_kind, bool sync_hos
 		}
 		h->prog.blend_split_on = (many && h->blend_split == 2) ? 1 : 0;
 	}
+	// The program the cycle kernels run.  RobotController.cpp:96-116: the avoidance blend comes after the task torques (and their
+	// saturation) and before gravity compensation, so with joint-limit avoidance the cycle kernels leave gravity to its kernel.
+	OscProgram prog = h->prog;
+	if (h->jla_enabled) prog.gravity_comp = 0;
+	// decided before anything is launched or counted: a refused cycle leaves the models armed and the epoch as they were
+	const osc::CyclePlan plan = osc::plan_cycle(prog, h->model.n, h->sig_R, h->sig_jt);
+	if (plan.error != OSC_OK) return fail(h, plan.error, plan.message);
+	h->prog.tau = prog.tau = (mem_kind == OSC_MEM_DEVICE) ? tau_out : h->d_tau;
+	h->prog.update_models = prog.update_models = h->models_armed ? 1 : 0;
+	h->models_armed = false;
+	prog.epoch = ++h->prog.epoch;
 	cudaError_t e;
 	if (h->otg_tasks > 0) {	 // the tasks' internal OTG produces this cycle's desired state first (JointTask.cpp:313-319, MotionForceTask.cpp:394-407)
 		CUDA_TRY(h, osc::launch_otg_update(h->prog, h->stream));
 		h->launches += 1;
 	}
-	if (h->jla_enabled) {
-		// RobotController.cpp:96-116: the avoidance blend comes after the task torques (and their saturation) and before
-		// gravity compensation, so the cycle kernels leave gravity to the avoidance kernel
-		OscProgram prog = h->prog;
-		prog.gravity_comp = 0;
-		e = osc::launch_cycle(h->model.n, h->sig_R, h->sig_jt, prog, h->stream);
-		if (e == cudaSuccess) e = osc::launch_jla(h->prog, h->stream);
+	e = osc::launch_cycle(h->model.n, h->sig_R, h->sig_jt, plan, prog, h->stream);
+	if (e == cudaSuccess && h->jla_enabled) {
+		e = osc::launch_jla(h->prog, h->stream);
 		if (e == cudaSuccess) h->launches += 1;
-	} else {
-		e = osc::launch_cycle(h->model.n, h->sig_R, h->sig_jt, h->prog, h->stream);
 	}
 	if (e == cudaErrorNotSupported) return fail(h, OSC_ERR_UNSUPPORTED, "no kernel compiled for this hierarchy signature");
 	CUDA_TRY(h, e);
-	// fused cycle kernel (+ the general-path kernel when a motion-force task leads, or the three of the split blending path)
-	h->launches += (h->sig_R > 0) ? (osc::blend_split_selected(h->prog) ? 4 : 2) : 1;
+	h->launches += plan.launches;
 	h->prog.sing_parity ^= 1;
 	if (mem_kind == OSC_MEM_HOST) {
 		CUDA_TRY(h, cudaMemcpyAsync(tau_out, h->d_tau, (size_t)h->model.n * h->NR * sizeof(double), cudaMemcpyDeviceToHost, h->stream));

@@ -78,8 +78,9 @@ DEVI void bie_cholesky_from_factor(const double (&L)[N][N], const double (&d)[N]
 // reduced Jacobian columns and the gravity vector.
 template <int N>
 constexpr int kSmFactor = N * (N + 1) / 2 + N;
-template <int N, int R, bool SPEC = false, bool MOTION = SPEC>
+template <int N, int R, unsigned V>
 constexpr int cycle_smem_doubles() {
+	constexpr bool SPEC = V & CV_SPEC, MOTION = V & CV_MOTION;
 	// rolled kinematics layout (osc_kindyn.cuh); factor and Jacobian columns fit underneath, the staged goals of the
 	// motion-force task (30) go behind the Jacobian columns, those of the joint task (6 N) later take their place
 	if (SPEC) {
@@ -228,19 +229,20 @@ DEVI void park_for_blend(const OscProgram& P, int slot, int64_t i, const double 
 	for (int k = 0; k < 9; k++) S[(int64_t)(BL::RC + k) * cap] = Rc[k];
 }
 
-// Signature <N, R, HAS_JT, FULL>:  R = rank of a leading MotionForceTask (0: none), FULL = that task controls all six
-// directions (B = I), HAS_JT = a full JointTask closes the hierarchy.
-// Dynamic shared memory: cycle_smem_doubles<N, R>() doubles per thread,
+// Signature <N, R, HAS_JT>:  R = rank of a leading MotionForceTask (0: none), HAS_JT = a full JointTask closes the hierarchy.
+// V: the flag word (CV_* bits, osc_launch.h, which also lists the instantiated words and their legal combinations).
+// Dynamic shared memory: cycle_smem_doubles<N, R, V>() doubles per thread,
 // element e of thread t at  sm[e * blockDim.x + t]  (conflict-free, 8-byte interleave).
 //
-// SPEC = true is the specialisation for the default configuration of the flagship hierarchy (cycle_spec_eligible()
-// in osc_cycle_kernels.cu states the conditions: every joint revolute about its local z axis, pure motion control, no
+// FULL: the motion-force task controls all six directions (B = I).
+// SPEC is the specialisation for the default configuration of the flagship hierarchy (cycle_spec_eligible()
+// in osc_launch.h states the conditions: every joint revolute about its local z axis, pure motion control, no
 // velocity saturation, FULL or BOUNDED_INERTIA decoupling).  Everything those conditions rule out is
 // compiled out, which brings the kernel from 223 KB to under 128 KB of code: beyond that size the instruction stream
 // no longer stays in the SM's instruction cache between blocks and every 256-byte line costs a round trip to L2
 // (profiles/r01_ifetch.md).  Robots whose bounded-inertia update has rank two or more leave through the general path.
 // GRAV (with SPEC only): gravity compensation compiled in; the non-specialised instantiations test the run-time flag.
-// MOTION (with SPEC only; default): the motion-force task is a full task under pure motion control, so only the two PID
+// MOTION (with SPEC only): the motion-force task is a full task under pure motion control, so only the two PID
 // laws are compiled in and its goals are staged through shared memory.  SPEC without MOTION keeps the general control
 // law (partial tasks, force / moment spaces, closed loops, POPC) on top of the same rolled kinematics.
 // PARK (full six-dof task only): hand-overs also leave kinematics and dynamics in the scratch block of the split blending path
@@ -248,8 +250,9 @@ DEVI void park_for_blend(const OscProgram& P, int slot, int64_t i, const double 
 // PRG (with SPEC, or for a JointTask alone): a task of the launch carries per-robot PID gains (osc_set_gains), read from its gain block in global
 // memory (a task without a block: its parameters); the instantiations without it read the broadcast parameters (SPEC) or test
 // the block pointer at run time (the others).
-template <int N, int R, bool HAS_JT, bool FULL, bool SPEC = false, bool GRAV = false, bool MOTION = SPEC, bool PARK = false, bool PRG = false>
+template <int N, int R, bool HAS_JT, unsigned V>
 __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(const __grid_constant__ OscProgram P) {
+	constexpr bool FULL = V & CV_FULL, SPEC = V & CV_SPEC, GRAV = V & CV_GRAV, MOTION = V & CV_MOTION, PARK = V & CV_PARK, PRG = V & CV_PRG;
 	extern __shared__ double sm[];
 	// Programmatic dependent launch on both sides: the general-path kernel of this cycle may be scheduled into whatever
 	// the last wave leaves free (it waits for this grid to complete before it reads the hand-over list), and this kernel
@@ -277,7 +280,6 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 	// in the middle of the control law cannot be hidden with two warps per scheduler, and a block that was scheduled
 	// while the previous kernel of the stream is still running (programmatic dependent launch) uses the wait for it.
 	// Prefetches are safe ahead of griddepcontrol.wait: they only move lines into L2, which stays coherent.
-	static_assert(!PRG || SPEC || R == 0, "per-robot gain instantiations: the specialised ones and the joint task alone");
 	// where the control laws read the gains: a JointTask alone (R = 0) has a per-robot instantiation like the specialised kernels,
 	// the other non-specialised instantiations test the block pointer at run time
 	constexpr int G = PRG ? GAINS_ROBOT : (SPEC || R == 0) ? GAINS_BCAST : GAINS_ANY;
@@ -506,7 +508,6 @@ __global__ void __launch_bounds__(kCycleBlock, OSC_MIN_BLOCKS) osc_cycle_kernel(
 				P.sing_list[slot] = (int32_t)i;
 				if constexpr (PARK) {
 					// split blending path (osc_blend.cuh): leave what is already known about this robot in its scratch block
-					static_assert(!PARK || (R == 6 && FULL), "the split blending path is for the full six-dof task");
 					if (P.blend_split_on) {
 						double gv[N];
 #pragma unroll

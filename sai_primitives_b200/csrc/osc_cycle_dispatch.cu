@@ -1,7 +1,7 @@
 #include "osc_launch.h"
 
 namespace osc {
-#define DECL(n) cudaError_t launch_cycle_n##n(int R, bool has_jt, const OscProgram& P, cudaStream_t stream);
+#define DECL(n) cudaError_t launch_cycle_n##n(int R, bool has_jt, const CyclePlan& plan, const OscProgram& P, cudaStream_t stream);
 OSC_CYCLE_DOFS(DECL)
 #undef DECL
 
@@ -16,11 +16,10 @@ bool cycle_signature_available(int n, int R, bool has_jt) {
 	return false;
 }
 
-cudaError_t launch_cycle(int n, int R, bool has_jt, const OscProgram& P, cudaStream_t stream) {
-	if (!cycle_signature_available(n, R, has_jt)) return cudaErrorNotSupported;
-	if (P.precision_fp32 && R != 6) return cudaErrorNotSupported;  // the single-precision mode covers the full six-dof task only (osc_cycle_f32.cu)
+cudaError_t launch_cycle(int n, int R, bool has_jt, const CyclePlan& plan, const OscProgram& P, cudaStream_t stream) {
+	if (!cycle_signature_available(n, R, has_jt) || plan.error != OSC_OK) return cudaErrorNotSupported;
 #define CALL(m) \
-	if (n == m) return launch_cycle_n##m(R, has_jt, P, stream);
+	if (n == m) return launch_cycle_n##m(R, has_jt, plan, P, stream);
 	OSC_CYCLE_DOFS(CALL)
 #undef CALL
 	return cudaErrorNotSupported;

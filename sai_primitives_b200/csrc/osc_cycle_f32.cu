@@ -3,7 +3,7 @@
 // in global memory (inputs, task state, torques) stay FP64, so robots the kernel hands over continue on the FP64 general path.
 #include "osc_dev_types.h"
 #include "osc_launch.h"
-#include <atomic>
+#include <utility>
 #define OSC_FP32_BUILD 1
 #define OSC_MIN_BLOCKS 3  // 168 registers, 54 KB of shared memory per block: three blocks (12 warps) per SM; four (128 registers) measured 4-8 % slower
 #include "fp32/osc_types32.h"
@@ -11,49 +11,27 @@
 
 namespace osc {
 
-template <int N, bool JT, bool GRAV>
-static cudaError_t launch_f32(const OscProgram& P, cudaStream_t stream) {
-	constexpr int R = 6;
-	const unsigned grid = (unsigned)((P.n_robots + kCycleBlock - 1) / kCycleBlock);
-	constexpr int smem = osc32::cycle_smem_doubles<N, R, true, true>() * kCycleBlock * (int)sizeof(float);
-	static std::atomic<bool> configured[64];
-	int dev = 0;
-	cudaGetDevice(&dev);
-	if (dev < 0 || dev >= 64 || !configured[dev].load(std::memory_order_acquire)) {
-		cudaError_t e = cudaFuncSetAttribute(osc32::osc_cycle_kernel<N, R, JT, true, true, GRAV, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-		if (e != cudaSuccess) return e;
-		if (dev >= 0 && dev < 64) configured[dev].store(true, std::memory_order_release);
-	}
-	cudaLaunchConfig_t cfg{};
-	cfg.gridDim = dim3(grid);
-	cfg.blockDim = dim3(kCycleBlock);
-	cfg.dynamicSmemBytes = smem;
-	cfg.stream = stream;
-	cudaLaunchAttribute attr[1];
-	attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-	attr[0].val.programmaticStreamSerializationAllowed = 1;
-	cfg.attrs = attr;
-	cfg.numAttrs = 1;
+// the single-precision kernel of word v: one instantiation per word of its list (cycle_words, osc_launch.h)
+template <int N, bool JT, size_t... I>
+static cudaError_t launch_f32(unsigned v, const osc32::OscProgram& P32, cudaStream_t stream, std::index_sequence<I...>) {
+	constexpr CycleWordList L = cycle_words(6, true);
+	cudaError_t e = cudaErrorNotSupported;
+	(void)((v == L.word[I] && ((e = launch_fused_kernel<osc32::osc_cycle_kernel<N, 6, JT, L.word[I]>>(
+										P32, osc32::cycle_smem_doubles<N, 6, L.word[I]>() * kCycleBlock * (int)sizeof(float), stream)),
+								true)) ||
+		   ...);
+	return e;
+}
+
+cudaError_t launch_cycle_fused_f32(int n, bool has_jt, unsigned word, const OscProgram& P, cudaStream_t stream) {
 	osc32::OscProgram P32;
 	osc32::to_f32(P, P32);
-	return cudaLaunchKernelEx(&cfg, osc32::osc_cycle_kernel<N, R, JT, true, true, GRAV, true>, P32);
-}
-
-// the fused kernel of [full six-dof MotionForceTask under pure motion control (+ full JointTask)] in single precision;
-// cudaErrorNotSupported for a dof that is not compiled in
-cudaError_t launch_cycle_fused_f32(int n, bool has_jt, const OscProgram& P, cudaStream_t stream) {
-	switch (n) {
+	constexpr auto seq = std::make_index_sequence<cycle_words(6, true).count>{};
 #define OSC_F32_CASE(NN) \
-	case NN: \
-		if (has_jt) return P.gravity_comp ? launch_f32<NN, true, true>(P, stream) : launch_f32<NN, true, false>(P, stream); \
-		return P.gravity_comp ? launch_f32<NN, false, true>(P, stream) : launch_f32<NN, false, false>(P, stream);
-		OSC_F32_CASE(7)
+	if (n == NN) return has_jt ? launch_f32<NN, true>(word & ~CV_F32, P32, stream, seq) : launch_f32<NN, false>(word & ~CV_F32, P32, stream, seq);
+	OSC_F32_DOFS(OSC_F32_CASE)
 #undef OSC_F32_CASE
-	default:
-		return cudaErrorNotSupported;
-	}
+	return cudaErrorNotSupported;
 }
-
-bool fused_f32_available(int n) { return n == 7; }
 
 }  // namespace osc

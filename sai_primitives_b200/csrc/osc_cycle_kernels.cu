@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
+#include <utility>
 #if defined(OSC_TRACE)
 #include <cstdio>
 #include <cstdlib>
@@ -39,21 +40,11 @@ static int sm_count() {
 	return v;
 }
 
-template <int N, int R, bool JT, bool FULL, bool SPEC = false, bool GRAV = false, bool MOTION = SPEC, bool PARK = false, bool PRG = false>
-static cudaError_t launch_variant(const OscProgram& P, cudaStream_t stream) {
-	const unsigned grid = (unsigned)((P.n_robots + kCycleBlock - 1) / kCycleBlock);
-	constexpr int smem = cycle_smem_doubles<N, R, SPEC, MOTION>() * kCycleBlock * (int)sizeof(double);
-	// per device: function attributes belong to the device's context.  Atomic flags: host threads driving different handles
-	// may get here at the same time (setting the attribute twice is harmless, a torn read of a plain bool is not defined).
-	static std::atomic<bool> configured[64];
-	int dev = 0;
-	cudaGetDevice(&dev);
-	if (dev < 0 || dev >= 64 || !configured[dev].load(std::memory_order_acquire)) {
-		cudaError_t e = cudaFuncSetAttribute(osc_cycle_kernel<N, R, JT, FULL, SPEC, GRAV, MOTION, PARK, PRG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-		if (e != cudaSuccess) return e;
-		if (dev >= 0 && dev < 64) configured[dev].store(true, std::memory_order_release);
-	}
+template <int N, int R, bool JT, unsigned V>
+static cudaError_t launch_fused(const OscProgram& P, cudaStream_t stream) {
+	constexpr int smem = cycle_smem_doubles<N, R, V>() * kCycleBlock * (int)sizeof(double);
 #if defined(OSC_TRACE)
+	const unsigned grid = (unsigned)((P.n_robots + kCycleBlock - 1) / kCycleBlock);
 	static unsigned long long* d_trace = nullptr;
 	const size_t tbytes = (size_t)grid * 32 * 2 * sizeof(unsigned long long);
 	if (!d_trace) {
@@ -62,20 +53,8 @@ static cudaError_t launch_variant(const OscProgram& P, cudaStream_t stream) {
 	}
 	cudaMemsetAsync(d_trace, 0, tbytes, stream);
 #endif
-	{
-		cudaLaunchConfig_t cfg{};
-		cfg.gridDim = dim3(grid);
-		cfg.blockDim = dim3(kCycleBlock);
-		cfg.dynamicSmemBytes = smem;
-		cfg.stream = stream;
-		cudaLaunchAttribute attr[1];
-		attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-		attr[0].val.programmaticStreamSerializationAllowed = 1;
-		cfg.attrs = attr;
-		cfg.numAttrs = 1;
-		cudaError_t e = cudaLaunchKernelEx(&cfg, osc_cycle_kernel<N, R, JT, FULL, SPEC, GRAV, MOTION, PARK, PRG>, P);
-		if (e != cudaSuccess) return e;
-	}
+	cudaError_t e = launch_fused_kernel<osc_cycle_kernel<N, R, JT, V>>(P, smem, stream);
+	if (e != cudaSuccess) return e;
 #if defined(OSC_TRACE)
 	if (const char* path = getenv("OSC_TRACE_FILE")) {
 		cudaStreamSynchronize(stream);
@@ -92,64 +71,21 @@ static cudaError_t launch_variant(const OscProgram& P, cudaStream_t stream) {
 	return cudaGetLastError();
 }
 
+// the fused kernel of the planned word: one instantiation per word of the signature's list (cycle_words, osc_launch.h)
+template <int N, int R, bool JT, size_t... I>
+static cudaError_t launch_listed(unsigned v, const OscProgram& P, cudaStream_t stream, std::index_sequence<I...>) {
+	constexpr CycleWordList L = cycle_words(R);
+	cudaError_t e = cudaErrorNotSupported;
+	(void)((v == L.word[I] && ((e = launch_fused<N, R, JT, L.word[I]>(P, stream)), true)) || ...);
+	return e;
+}
+
 template <int N, int R, bool JT>
-static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
-	cudaError_t e0;
-	if constexpr (R == 6) {
-		bool motion = false;
-		const bool spec = cycle_spec_eligible(P, JT, &motion);
-		// with many robots on the general path the hand-overs also park their kinematics and dynamics for the split blending path
-		const bool park = P.mft[0].full && blend_split_selected(P);
-		const bool prg = cycle_per_robot_gains(P, JT);
-		if (P.precision_fp32) {
-			// optional single-precision mode: only the specialised pure-motion kernel has an FP32 instantiation (osc_cycle_f32.cu)
-			if (!(P.mft[0].full && spec && motion)) return cudaErrorNotSupported;
-			e0 = launch_cycle_fused_f32(N, JT, P, stream);
-		} else if (!P.mft[0].full)
-			e0 = launch_variant<N, R, JT, false>(P, stream);
-		else if (prg && cycle_prg_specialised(R, spec, motion)) {
-			// per-robot gains: the pure-motion specialisation has its own instantiations (the others test the pointer at run time)
-			if (!park)
-				e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, true, false, true>(P, stream)
-									: launch_variant<N, R, JT, true, true, false, true, false, true>(P, stream);
-			else
-				e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, true, true, true>(P, stream)
-									: launch_variant<N, R, JT, true, true, false, true, true, true>(P, stream);
-		} else if (prg && !park)
-			e0 = launch_variant<N, R, JT, true>(P, stream);
-		else if (prg)
-			e0 = launch_variant<N, R, JT, true, false, false, false, true>(P, stream);
-		else if (spec && motion && !park)
-			e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true>(P, stream) : launch_variant<N, R, JT, true, true, false>(P, stream);
-		else if (spec && motion)
-			e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, true, true>(P, stream) : launch_variant<N, R, JT, true, true, false, true, true>(P, stream);
-		else if (spec && !park)	// full task with force / moment control or velocity saturation
-			e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, false>(P, stream) : launch_variant<N, R, JT, true, true, false, false>(P, stream);
-		else if (spec)
-			e0 = P.gravity_comp ? launch_variant<N, R, JT, true, true, true, false, true>(P, stream) : launch_variant<N, R, JT, true, true, false, false, true>(P, stream);
-		else if (!park)
-			e0 = launch_variant<N, R, JT, true>(P, stream);
-		else
-			e0 = launch_variant<N, R, JT, true, false, false, false, true>(P, stream);
-	} else if constexpr (R == 3) {
-		// the other common shape: three controlled directions (position only, or a planar task), any control law
-		bool motion = false;
-		const bool spec = cycle_spec_eligible(P, JT, &motion);
-		if (spec && cycle_per_robot_gains(P, JT) && cycle_prg_specialised(R, spec, motion))
-			e0 = P.gravity_comp ? launch_variant<N, R, JT, false, true, true, false, false, true>(P, stream)
-								: launch_variant<N, R, JT, false, true, false, false, false, true>(P, stream);
-		else if (spec)
-			e0 = P.gravity_comp ? launch_variant<N, R, JT, false, true, true, false>(P, stream) : launch_variant<N, R, JT, false, true, false, false>(P, stream);
-		else
-			e0 = launch_variant<N, R, JT, false>(P, stream);
-	} else if constexpr (R == 0) {
-		// a JointTask alone: per-robot gains have their own instantiation, the broadcast one reads the parameters
-		e0 = cycle_per_robot_gains(P, JT) ? launch_variant<N, R, JT, false, false, false, false, false, true>(P, stream) : launch_variant<N, R, JT, false>(P, stream);
-	} else {
-		e0 = launch_variant<N, R, JT, false>(P, stream);
-	}
+static cudaError_t launch_one(const CyclePlan& plan, const OscProgram& P, cudaStream_t stream) {
+	const cudaError_t e0 = (plan.fused & CV_F32) ? launch_cycle_fused_f32(N, JT, plan.fused, P, stream)
+												: launch_listed<N, R, JT>(plan.fused, P, stream, std::make_index_sequence<cycle_words(R).count>{});
 	if (e0 != cudaSuccess) return e0;
-	if constexpr (R > 0) {
+	if (plan.general != GeneralPath::None) {
 #ifdef OSC_TUNE_SKIP_GENERAL
 		return e0;	// tuning builds only: measure what the second launch costs when the hand-over list is empty
 #endif
@@ -170,7 +106,7 @@ static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
 		cfg.numAttrs = 1;
 		if constexpr (R == 6) {
 			// flagship hierarchy: unrolled blending path (osc_blend.cuh), general path only as its fallback
-			if (P.mft[0].full && blend_split_selected(P)) {
+			if (plan.general == GeneralPath::BlendSplit) {
 				// hand-overs are expected (host hint): prefix / variants / fallback as three kernels, each grid-stride over
 				// its list with as many blocks as the device holds at once
 				const bool motion = mft_pure_motion(P.mft[0]);
@@ -205,7 +141,7 @@ static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
 				cfg.dynamicSmemBytes = 0;
 				return cudaLaunchKernelEx(&cfg, osc_blend_fallback_kernel<N>, P);
 			}
-			if (P.mft[0].full) return cudaLaunchKernelEx(&cfg, osc_blend_kernel<N, JT>, P);
+			if (plan.general == GeneralPath::Blend) return cudaLaunchKernelEx(&cfg, osc_blend_kernel<N, JT>, P);
 		}
 		return cudaLaunchKernelEx(&cfg, osc_singular_kernel<N>, P);
 	}
@@ -214,12 +150,12 @@ static cudaError_t launch_one(const OscProgram& P, cudaStream_t stream) {
 
 // motion-force task of rank R (1..min(6,N)), with or without a closing full joint task
 template <int N, int R>
-static cudaError_t launch_rank(bool has_jt, const OscProgram& P, cudaStream_t stream) {
+static cudaError_t launch_rank(bool has_jt, const CyclePlan& plan, const OscProgram& P, cudaStream_t stream) {
 	if constexpr (R >= 1 && R <= N && R <= 6 && OSC_ONLY_R != 0) {
-		if constexpr (R == OSC_ONLY_R) return has_jt ? launch_one<N, R, true>(P, stream) : cudaErrorNotSupported;
+		if constexpr (R == OSC_ONLY_R) return has_jt ? launch_one<N, R, true>(plan, P, stream) : cudaErrorNotSupported;
 		return cudaErrorNotSupported;
 	} else if constexpr (R >= 1 && R <= N && R <= 6) {
-		return has_jt ? launch_one<N, R, true>(P, stream) : launch_one<N, R, false>(P, stream);
+		return has_jt ? launch_one<N, R, true>(plan, P, stream) : launch_one<N, R, false>(plan, P, stream);
 	} else {
 		return cudaErrorNotSupported;
 	}
@@ -235,19 +171,19 @@ static cudaError_t launch_generic(const OscProgram& P, cudaStream_t stream) {
 #define CONCAT_(a, b) a##b
 #define CONCAT(a, b) CONCAT_(a, b)
 
-cudaError_t CONCAT(launch_cycle_n, OSC_INST_N)(int R, bool has_jt, const OscProgram& P, cudaStream_t stream) {
+cudaError_t CONCAT(launch_cycle_n, OSC_INST_N)(int R, bool has_jt, const CyclePlan& plan, const OscProgram& P, cudaStream_t stream) {
 	constexpr int N = OSC_INST_N;
 	if (R < 0) return launch_generic<N>(P, stream);	 // general hierarchy: every robot on the general path
 	switch (R) {
 		case 0:
 			if constexpr (OSC_ONLY_R != 0) return cudaErrorNotSupported;
-			else return has_jt ? launch_one<N, 0, true>(P, stream) : cudaErrorNotSupported;
-		case 1: return launch_rank<N, 1>(has_jt, P, stream);
-		case 2: return launch_rank<N, 2>(has_jt, P, stream);
-		case 3: return launch_rank<N, 3>(has_jt, P, stream);
-		case 4: return launch_rank<N, 4>(has_jt, P, stream);
-		case 5: return launch_rank<N, 5>(has_jt, P, stream);
-		case 6: return launch_rank<N, 6>(has_jt, P, stream);
+			else return has_jt ? launch_one<N, 0, true>(plan, P, stream) : cudaErrorNotSupported;
+		case 1: return launch_rank<N, 1>(has_jt, plan, P, stream);
+		case 2: return launch_rank<N, 2>(has_jt, plan, P, stream);
+		case 3: return launch_rank<N, 3>(has_jt, plan, P, stream);
+		case 4: return launch_rank<N, 4>(has_jt, plan, P, stream);
+		case 5: return launch_rank<N, 5>(has_jt, plan, P, stream);
+		case 6: return launch_rank<N, 6>(has_jt, plan, P, stream);
 	}
 	return cudaErrorNotSupported;
 }
