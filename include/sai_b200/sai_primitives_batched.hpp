@@ -107,6 +107,8 @@ public:
 		: _robot(robot), _task_name(task_name), _task_type(type), _loop_timestep(loop_timestep) {}
 	virtual ~TemplateTask() = default;
 	virtual void reInitializeTask() { check(h(), osc_reinitialize_task(h(), _id)); }
+	// the robots a non-zero entry of mask (int32 x n_robots in `where` memory) selects (osc_reset_robots, OSC_RESET_REINITIALIZE)
+	void reInitializeTask(const int32_t* mask, osc_mem_kind where) { check(h(), osc_reset_robots(h(), _id, mask, where, OSC_RESET_REINITIALIZE)); }
 	const std::shared_ptr<BatchedRobot>& getConstRobotModel() const { return _robot; }
 	const double& getLoopTimestep() const { return _loop_timestep; }
 	const TaskType& getTaskType() const { return _task_type; }
@@ -472,6 +474,14 @@ public:
 	void enableJointLimitAvoidance(bool on) { check(_robot->handle(), osc_enable_joint_limit_avoidance(_robot->handle(), on)); }
 	void enableTorqueSaturation(bool on) { check(_robot->handle(), osc_enable_torque_saturation(_robot->handle(), on)); }
 	void reinitializeTasks() { check(_robot->handle(), osc_reinitialize_task(_robot->handle(), -1)); }
+	void reinitializeTasks(const int32_t* mask, osc_mem_kind where) {
+		check(_robot->handle(), osc_reset_robots(_robot->handle(), -1, mask, where, OSC_RESET_REINITIALIZE));
+	}
+	// episode reset (no reference counterpart): every task of the selected robots as right after construction at the current state
+	// (osc_reset_robots, OSC_RESET_CONSTRUCT); mask == nullptr: every robot
+	void resetRobots(const int32_t* mask = nullptr, osc_mem_kind where = OSC_MEM_HOST) {
+		check(_robot->handle(), osc_reset_robots(_robot->handle(), -1, mask, where, OSC_RESET_CONSTRUCT));
+	}
 	std::shared_ptr<JointTask> getJointTaskByName(const std::string& task_name) {
 		for (auto& t : _tasks)
 			if (t->getTaskName() == task_name) {

@@ -378,8 +378,33 @@ int osc_set_field(osc_handle* h, int task_id, int field, const double* data, int
 int osc_get_field(osc_handle* h, int task_id, int field, double* out, int mem_kind);
 
 /* ---- re-initialisation.  TemplateTask::reInitializeTask (JointTask.cpp:91-107, MotionForceTask.cpp:204-245);
- *      task_id < 0: RobotController::reinitializeTasks (RobotController.cpp:120-125) ---- */
+ *      task_id < 0: RobotController::reinitializeTasks (RobotController.cpp:120-125).  Every robot; the same as
+ *      osc_reset_robots(h, task_id, NULL, OSC_MEM_DEVICE, OSC_RESET_REINITIALIZE) ---- */
 int osc_reinitialize_task(osc_handle* h, int task_id);
+
+/* ---- per-robot resets (episode ends of batched rollouts: a robot moved to a new state starts its controller over there).
+ *   robot_mask: int32 x n_robots in mem_kind memory, a non-zero entry selects the robot; NULL selects every robot.  Any int32 is
+ *     a valid entry, so a device mask is never read by the host: the call is asynchronous and ordered with the control cycles
+ *     in the handle's stream like a goal write.  A host mask is copied into a handle-owned device buffer with cudaMemcpyAsync;
+ *     a pageable one may be reused when the call returns, a page-locked one must stay unchanged until the stream has reached
+ *     the call.
+ *   task_id < 0: every task of the handle, in hierarchy order (RobotController::reinitializeTasks); otherwise that task.
+ *   The reset is evaluated at the state of the latest osc_set_state / osc_step (device state buffers are borrowed, so values
+ *   written into them earlier in the handle's stream are the ones seen).
+ *   OSC_RESET_REINITIALIZE: TemplateTask::reInitializeTask for each selected robot, i.e. what osc_reinitialize_task does,
+ *     restricted to those robots: goals := current pose / position with zero velocity, acceleration, force and moment goals,
+ *     integrators and sensed wrench zeroed; a task with the internal OTG on has its generator re-initialised at the current
+ *     pose.  The singularity handler's memory and the POPC state stay, as in the reference.
+ *   OSC_RESET_CONSTRUCT: the state the tasks had right after construction at the current state (what osc_add_*_task leaves),
+ *     with the generator of a task that has the internal OTG on constructed anew as enabling it does.  On top of the above,
+ *     the singularity handler's memory is reset (type-1 posture _q_prior to mid-range -- so a posture set with
+ *     OSC_MFT_TYPE1_POSTURE is reset too --, type-2 directions, counters and history) and so are the POPC observer and window.
+ *   Configuration is never touched by either mode: broadcast parameters, per-robot gains, per-robot spaces and closed-loop
+ *   flags, passivity on/off and ring capacity, the force sensor frame, the OTG's enabled flag and limits.  Robots that are not
+ *   selected are not written.  A bad task_id, mode or mem_kind returns OSC_ERR_INVALID_ARGUMENT and changes nothing.  One
+ *   kernel launch per call, whatever the number of tasks. ---- */
+typedef enum { OSC_RESET_REINITIALIZE = 0, OSC_RESET_CONSTRUCT = 1 } osc_reset_mode;
+int osc_reset_robots(osc_handle* h, int task_id, const int32_t* robot_mask, int mem_kind, int mode);
 
 /* ---- controller options (RobotController.h:66-76) ---- */
 int osc_enable_gravity_compensation(osc_handle* h, int enabled);

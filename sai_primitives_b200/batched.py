@@ -51,6 +51,41 @@ def _soa(a, n_robots, ncomp):
     raise ValueError("expected an array of shape (%d, %d), got %s" % (n_robots, ncomp, a.shape))
 
 
+def robot_mask(robots, n_robots):
+    """The int32 [N] mask of osc_reset_robots for `robots`: None (every robot: no mask), a bool [N] array, or an array of robot
+    indices in 0..N-1.  Raises ValueError for anything else, an index out of range included."""
+    if robots is None:
+        return None
+    a = np.asarray(robots)
+    if a.dtype == np.bool_:
+        if a.shape != (n_robots,):
+            raise ValueError("a boolean robot selection must have shape (%d,), got %s" % (n_robots, a.shape))
+        return np.ascontiguousarray(a, dtype=np.int32)
+    if a.ndim != 1:
+        raise ValueError("robots must be a boolean array of shape (%d,) or a 1-D array of robot indices" % n_robots)
+    if a.size == 0:
+        return np.zeros(n_robots, dtype=np.int32)
+    # a list mixing booleans and integers is neither form (numpy would read [True, 2] as the indices [1, 2])
+    mixed = not isinstance(robots, np.ndarray) and any(isinstance(x, (bool, np.bool_)) for x in robots)
+    if mixed or not np.issubdtype(a.dtype, np.integer):
+        raise ValueError("robots must be a boolean array of shape (%d,) or a 1-D array of robot indices" % n_robots)
+    if a.min() < 0 or a.max() >= n_robots:
+        raise ValueError("robot index out of range [0, %d)" % n_robots)
+    mask = np.zeros(n_robots, dtype=np.int32)
+    mask[a] = 1
+    return mask
+
+
+def _reset(robot, task_id, robots, mode):
+    mask = robot_mask(robots, robot.n_robots)
+    ptr = None if mask is None else _int_ptr(mask)
+    _check(robot.handle, robot._lib.osc_reset_robots(robot.handle, task_id, ptr, capi.OSC_MEM_HOST, mode))
+
+
+def _reset_device(robot, task_id, mask_ptr, mode):
+    _check(robot.handle, robot._lib.osc_reset_robots(robot.handle, task_id, C.c_void_p(mask_ptr), capi.OSC_MEM_DEVICE, mode))
+
+
 def registerUrdf(model_name, urdf_file_or_text):
     """SURVEY.md row f-3: make a URDF robot (a serial chain) available under `model_name`, the counterpart of
     `SaiModel(robot_file)` (examples/05-using_robot_controller/05-using_robot_controller.cpp:64).  Accepts a file name
@@ -195,6 +230,25 @@ class BatchedSimulation:
         _check(self._robot.handle, self._lib.osc_sim_integrate(self._robot.handle, self._q.ctypes.data_as(P), self._dq.ctypes.data_as(P),
                                                                self._tau.ctypes.data_as(P), self._dt, int(substeps), capi.OSC_MEM_HOST))
 
+    def setJointPositions(self, q, robots=None):
+        """sai-simulation's setJointPositions, for every robot ([N, n]) or for the robots selected by `robots` (as in
+        RobotController.resetRobots; q is then [N, n] or [len(selected), n])"""
+        self._set_rows(self._q, q, robots)
+
+    def setJointVelocities(self, dq, robots=None):
+        self._set_rows(self._dq, dq, robots)
+
+    def _set_rows(self, dst, v, robots):
+        n, N = self._robot.dof(), self._robot.n_robots
+        v = np.asarray(v, dtype=np.float64)
+        mask = robot_mask(robots, N)
+        sel = np.ones(N, dtype=bool) if mask is None else mask != 0
+        if v.shape == (N, n):
+            v = v[sel]
+        if v.shape != (int(sel.sum()), n):
+            raise ValueError("expected an array of shape (%d, %d) or (%d, %d), got %s" % (N, n, int(sel.sum()), n, v.shape))
+        dst[:, sel] = v.T
+
     def getJointPositions(self):
         return self._q.T.copy()
 
@@ -283,8 +337,13 @@ class _Task:
                                                           capi.host_ptr(out[1]), capi.host_ptr(out[2]), capi.OSC_MEM_HOST))
         return tuple(o.T.copy() for o in out)
 
-    def reInitializeTask(self):
-        _check(self._robot.handle, self._lib.osc_reinitialize_task(self._robot.handle, self.task_id))
+    def reInitializeTask(self, robots=None):
+        """TemplateTask::reInitializeTask for every robot or for those `robots` selects (a bool [N] array or robot indices)"""
+        _reset(self._robot, self.task_id, robots, capi.OSC_RESET_REINITIALIZE)
+
+    def reInitializeTaskDevice(self, mask_ptr):
+        """the same with an int32 [N] device mask (non-zero selects), ordered with the cycles in the robot's stream"""
+        _reset_device(self._robot, self.task_id, mask_ptr, capi.OSC_RESET_REINITIALIZE)
 
     # TemplateTask.h:74,82,89 -- [N, n, n], evaluated from the robot's current state
     def _nullspace(self, field):
@@ -792,8 +851,21 @@ class RobotController:
     def enableJointLimitAvoidance(self, flag):
         _check(self._robot.handle, self._lib.osc_enable_joint_limit_avoidance(self._robot.handle, 1 if flag else 0))
 
-    def reinitializeTasks(self):
-        _check(self._robot.handle, self._lib.osc_reinitialize_task(self._robot.handle, -1))
+    def reinitializeTasks(self, robots=None):
+        """RobotController::reinitializeTasks for every robot or for those `robots` selects (a bool [N] array or robot indices)"""
+        _reset(self._robot, -1, robots, capi.OSC_RESET_REINITIALIZE)
+
+    def reinitializeTasksDevice(self, mask_ptr):
+        _reset_device(self._robot, -1, mask_ptr, capi.OSC_RESET_REINITIALIZE)
+
+    def resetRobots(self, robots=None):
+        """Episode reset (no reference counterpart): every task of the selected robots goes back to the state it had right after
+        construction at the robot's current state -- goals at the current pose, integrators, singularity-handler memory and
+        POPC state reset, the internal OTG constructed anew.  Gains, spaces and every other setting stay."""
+        _reset(self._robot, -1, robots, capi.OSC_RESET_CONSTRUCT)
+
+    def resetRobotsDevice(self, mask_ptr):
+        _reset_device(self._robot, -1, mask_ptr, capi.OSC_RESET_CONSTRUCT)
 
     def getJointTaskByName(self, name):
         for t in self._tasks:

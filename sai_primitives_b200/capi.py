@@ -29,6 +29,7 @@ OSC_ERR_STATE = -5
 OSC_MEM_HOST = 0
 OSC_MEM_DEVICE = 1
 OSC_PRECISION_FP64, OSC_PRECISION_FP32 = 0, 1
+OSC_RESET_REINITIALIZE, OSC_RESET_CONSTRUCT = 0, 1
 
 FULL_DYNAMIC_DECOUPLING = 0
 BOUNDED_INERTIA_ESTIMATES = 1
@@ -195,6 +196,7 @@ SYMBOLS = {
     "osc_set_field": (C.c_int, [_H, C.c_int, C.c_int, _PD, C.c_int, C.c_int]),
     "osc_get_field": (C.c_int, [_H, C.c_int, C.c_int, _PD, C.c_int]),
     "osc_reinitialize_task": (C.c_int, [_H, C.c_int]),
+    "osc_reset_robots": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_int]),
     "osc_enable_gravity_compensation": (C.c_int, [_H, C.c_int]),
     "osc_enable_torque_saturation": (C.c_int, [_H, C.c_int]),
     "osc_enable_joint_limit_avoidance": (C.c_int, [_H, C.c_int]),

@@ -21,8 +21,8 @@ static inline dim3 grid_for(int64_t n, int block) { return dim3((unsigned)((n + 
 		default: return cudaErrorInvalidValue;         \
 	}
 
-cudaError_t launch_reinit_mft(const OscProgram& P, int mft_index, int full_init, cudaStream_t stream) {
-	DISPATCH_N(P.model.n, (reinit_mft_kernel<N_><<<grid_for(P.n_robots, 128), 128, 0, stream>>>(P, mft_index, full_init)));
+cudaError_t launch_reset_robots(const OscProgram& P, const int32_t* mask, int task, int construct, cudaStream_t stream) {
+	DISPATCH_N(P.model.n, (reset_robots_kernel<N_><<<grid_for(P.n_robots, 128), 128, 0, stream>>>(P, mask, task, construct)));
 	return cudaGetLastError();
 }
 cudaError_t launch_popc_probe(const OscProgram& P, int mft_index, int K, const double* fd, const double* fs, const double* vcl, const double* vr,
@@ -81,8 +81,8 @@ cudaError_t launch_otg_update(const OscProgram& P, cudaStream_t stream) {
 	otg_update_kernel<<<grid_for(P.n_robots, 64), 64, 0, stream>>>(P);
 	return cudaGetLastError();
 }
-cudaError_t launch_otg_init(const OscProgram& P, int task, int mode, int fresh, cudaStream_t stream) {
-	DISPATCH_N(P.model.n, (otg_init_kernel<N_><<<grid_for(P.n_robots, 64), 64, 0, stream>>>(P, task, mode, fresh)));
+cudaError_t launch_otg_init(const OscProgram& P, int task, int mode, cudaStream_t stream) {
+	DISPATCH_N(P.model.n, (otg_init_kernel<N_><<<grid_for(P.n_robots, 64), 64, 0, stream>>>(P, task, mode)));
 	return cudaGetLastError();
 }
 cudaError_t launch_otg_disable(const OscProgram& P, int task, cudaStream_t stream) {
@@ -91,10 +91,6 @@ cudaError_t launch_otg_disable(const OscProgram& P, int task, cudaStream_t strea
 }
 cudaError_t launch_observer(const OscProgram& P, int task, int kind, double* out, cudaStream_t stream) {
 	DISPATCH_N(P.model.n, (osc_observer_kernel<N_><<<grid_for(P.n_robots, 64), 64, 0, stream>>>(P, task, kind, out)));
-	return cudaGetLastError();
-}
-cudaError_t launch_reinit_jt(const OscProgram& P, int jt_index, cudaStream_t stream) {
-	DISPATCH_N(P.model.n, (reinit_jt_kernel<N_><<<grid_for(P.n_robots, 128), 128, 0, stream>>>(P, jt_index)));
 	return cudaGetLastError();
 }
 cudaError_t launch_sensed_wrench(const OscProgram& P, int mft_index, const double* f, const double* m, cudaStream_t stream) {

@@ -1,8 +1,9 @@
-// Small per-robot service kernels around the fused cycle: task (re)initialisation from the
-// current state, sensed-wrench frame change, the stand-alone kinematics/dynamics export
+// Small per-robot service kernels around the fused cycle: task resets of selected robots from
+// their current state, sensed-wrench frame change, the stand-alone kinematics/dynamics export
 // used by the parity tests, and SoA component fills/copies.
 #pragma once
 #include "osc_kindyn.cuh"
+#include "osc_otg_kernels.cuh"
 #include "osc_tasks.cuh"
 
 namespace osc {
@@ -42,23 +43,12 @@ __global__ void fill_int_components_kernel(int32_t* ist, int64_t NR, int comp, i
 	for (int c = 0; c < ncomp; c++) ist[(int64_t)(comp + c) * NR + i] = value;
 }
 
-// MotionForceTask::reInitializeTask (MotionForceTask.cpp:204-245) + the singularity handler /
-// POPC initial state (SingularityHandler.cpp:53-63, POPCExplicitForceControl.cpp:10-21).
-// full_init = 1 also resets what only the constructor resets (handler + POPC state).
+// MotionForceTask::reInitializeTask (MotionForceTask.cpp:204-245) of robot i at its current pose (x, R).  construct also resets
+// what only the constructor resets: the singularity handler / POPC initial state (SingularityHandler.cpp:53-63,
+// POPCExplicitForceControl.cpp:10-21).
 template <int N>
-__global__ void reinit_mft_kernel(const __grid_constant__ OscProgram P, int mft_index, int full_init) {
-	const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	const int64_t NR = P.n_robots;
-	if (i >= NR) return;
-	const DevMft& t = P.mft[mft_index];
+DEVI void mft_reset_robot(const DevMft& t, const DevModel& model, int64_t NR, int64_t i, const double x[3], const double R[9], bool construct) {
 	double* st = t.st;
-	double q[N];
-#pragma unroll
-	for (int j = 0; j < N; j++) q[j] = P.q[(int64_t)j * NR + i];
-	KinDyn<N> kd;
-	forward_kinematics<N>(P.model, q, kd);
-	double x[3], R[9];
-	frame_pose<N>(kd, t.body, t.ctrl_R, t.ctrl_t, x, R);
 	for (int c = 0; c < MC_POPC; c++) ST(0, c) = 0.0;  // goals, sensed values, integrators, observers
 	store3(st, NR, i, MC_GOAL_POS, x);
 	store3(st, NR, i, MC_CUR_POS, x);
@@ -67,13 +57,13 @@ __global__ void reinit_mft_kernel(const __grid_constant__ OscProgram P, int mft_
 		ST(MC_GOAL_ORI, k) = R[k];
 		ST(MC_CUR_ORI, k) = R[k];
 	}
-	if (full_init) {
+	if (construct) {
 		ST(MC_POPC, 0) = 0.0;
 		ST(MC_POPC, 1) = 0.0;
 		ST(MC_POPC, 2) = 1.0;  // Rc
 		ST(MC_POPC, 3) = 0.0;
 		for (int j = 0; j < OSC_MAX_DOF; j++) {
-			const double mid = (j < N) ? 0.5 * (P.model.q_lower[j] + P.model.q_upper[j]) : 0.0;
+			const double mid = (j < N) ? 0.5 * (model.q_lower[j] + model.q_upper[j]) : 0.0;
 			ST(MC_Q_PRIOR, j) = mid;
 			ST(MC_DQ_PRIOR, j) = 0.0;
 			ST(MC_TYPE2_DIR, j) = 1.0;
@@ -83,20 +73,58 @@ __global__ void reinit_mft_kernel(const __grid_constant__ OscProgram P, int mft_
 	}
 }
 
-// JointTask::reInitializeTask (JointTask.cpp:91-107)
+// JointTask::reInitializeTask (JointTask.cpp:91-107) of robot i; pos receives the task-space position (jt_task_position).  The
+// constructor does nothing more (JointTask.cpp:45-89).
 template <int N>
-__global__ void reinit_jt_kernel(const __grid_constant__ OscProgram P, int jt_index) {
+DEVI void jt_reset_robot(const DevJt& t, int64_t NR, int64_t i, const double (&q)[N], double pos[OSC_MAX_DOF]) {
+	double* st = t.st;
+	for (int c = 0; c < JC_COUNT; c++) ST(0, c) = 0.0;
+	jt_task_position<N>(t, q, pos);
+	for (int a = 0; a < t.k; a++) ST(JC_GOAL_POS, a) = pos[a];
+}
+
+// osc_reset_robots: the selected robots (mask == null: all; otherwise mask[i] != 0) get the tasks `task` (< 0: every task) reset
+// at their current state, in hierarchy order, with the internal generator of a task that has it on (osc_otg_kernels.cuh).
+// construct = 0: TemplateTask::reInitializeTask, generator re-initialised; construct = 1: the state right after the task's
+// constructor, generator constructed as enabling it does.  Robots that are not selected are not written.
+template <int N>
+__global__ void reset_robots_kernel(const __grid_constant__ OscProgram P, const int32_t* mask, int task, int construct) {
 	const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	const int64_t NR = P.n_robots;
 	if (i >= NR) return;
-	const DevJt& t = P.jt[jt_index];
-	double* st = t.st;
-	for (int c = 0; c < JC_COUNT; c++) ST(0, c) = 0.0;
-	for (int a = 0; a < t.k; a++) {
-		double pos = 0.0;
+	if (mask && mask[i] == 0) return;
+	double q[N];
 #pragma unroll
-		for (int j = 0; j < N; j++) pos += t.S[a][j] * P.q[(int64_t)j * NR + i];
-		ST(JC_GOAL_POS, a) = pos;
+	for (int j = 0; j < N; j++) q[j] = P.q[(int64_t)j * NR + i];
+	// poses of the (at most two) motion-force tasks first, so that the kinematics are not live across the resets
+	double x[2][3], R[2][9];
+	{
+		KinDyn<N> kd;
+		forward_kinematics<N>(P.model, q, kd);
+#pragma unroll
+		for (int m = 0; m < 2; m++) {
+			const DevMft& t = P.mft[m];
+			if (t.st) frame_pose<N>(kd, t.body, t.ctrl_R, t.ctrl_t, x[m], R[m]);
+		}
+	}
+	for (int k = 0; k < P.n_tasks; k++) {
+		if (task >= 0 && k != task) continue;
+		if (P.tasks[k].type == OSC_TASK_MOTION_FORCE) {
+			const int m = P.tasks[k].index;
+			const DevMft& t = P.mft[m];
+			double xm[3], Rm[9];
+#pragma unroll
+			for (int c = 0; c < 3; c++) xm[c] = m ? x[1][c] : x[0][c];
+#pragma unroll
+			for (int c = 0; c < 9; c++) Rm[c] = m ? R[1][c] : R[0][c];
+			mft_reset_robot<N>(t, P.model, NR, i, xm, Rm, construct != 0);
+			if (t.otg.enabled) otg_cart_init(t, NR, i, xm, Rm, construct != 0);  // MotionForceTask.cpp:244
+		} else {
+			const DevJt& t = P.jt[P.tasks[k].index];
+			double pos[OSC_MAX_DOF];
+			jt_reset_robot<N>(t, NR, i, q, pos);
+			if (t.otg.enabled) otg_joint_init(t, NR, i, pos, construct != 0);  // JointTask.cpp:106
+		}
 	}
 }
 

@@ -59,6 +59,7 @@ struct osc_handle {
 	// staging of the per-robot space calls with host buffers: axes (3 x N), dims or flags (N) and was_reset / closed_loop (N)
 	double* d_space_axes = nullptr;
 	int32_t* d_space_ints = nullptr;
+	int32_t* d_reset_mask = nullptr;  // staging of osc_reset_robots with a host mask (N)
 	int clean_cycles = 0;
 	int blend_split = -1;  // split blending path: -1 not decided, 0 off (SAI_B200_BLEND_SPLIT=0 or no memory), 1 allocate when needed, 2 allocated
 	int64_t blend_split_min = 0;  // hand-over count (host hint) from which the split path is used
@@ -537,7 +538,7 @@ int osc_add_joint_task(osc_handle* h, const double* selection, int k, double loo
 	}
 	h->prog.tasks[h->tasks.size() - 1] = DevTask{OSC_TASK_JOINT, h->n_jt};
 	h->prog.n_tasks = (int)h->tasks.size();
-	CUDA_TRY(h, osc::launch_reinit_jt(h->prog, h->n_jt, h->stream));
+	CUDA_TRY(h, osc::launch_reset_robots(h->prog, nullptr, (int)h->tasks.size() - 1, 1, h->stream));
 	h->launches++;
 	h->n_jt++;
 	if (task_id) *task_id = (int)h->tasks.size() - 1;
@@ -615,7 +616,7 @@ int osc_add_motion_force_task(osc_handle* h, const osc_mft_desc* desc, int* task
 	}
 	h->prog.tasks[h->tasks.size() - 1] = DevTask{OSC_TASK_MOTION_FORCE, h->n_mft};
 	h->prog.n_tasks = (int)h->tasks.size();
-	CUDA_TRY(h, osc::launch_reinit_mft(h->prog, h->n_mft, 1, h->stream));
+	CUDA_TRY(h, osc::launch_reset_robots(h->prog, nullptr, (int)h->tasks.size() - 1, 1, h->stream));
 	h->launches++;
 	h->n_mft++;
 	if (task_id) *task_id = (int)h->tasks.size() - 1;
@@ -856,7 +857,7 @@ static int parametrize_common(osc_handle* h, int task_id, int dim, const double 
 	}
 	if (reset && t.otg.enabled) {
 		// the same resets with the internal OTG on: goals and generator together (_otg->reInitializeLinear / Angular, :854, :886)
-		CUDA_TRY(h, osc::launch_otg_init(h->prog, task_id, moment ? 2 : 1, 0, h->stream));
+		CUDA_TRY(h, osc::launch_otg_init(h->prog, task_id, moment ? 2 : 1, h->stream));
 		h->launches++;
 		if ((rc = zero_comps(h, t.st, moment ? MC_INT_ORI : MC_INT_POS, 3)) != OSC_OK) return rc;
 		if ((rc = zero_comps(h, t.st, moment ? MC_INT_MOMENT : MC_INT_FORCE, 3)) != OSC_OK) return rc;
@@ -1362,22 +1363,24 @@ int osc_get_field(osc_handle* h, int task_id, int field, double* out, int mem_ki
 	return OSC_OK;
 }
 
-int osc_reinitialize_task(osc_handle* h, int task_id) {
+int osc_reinitialize_task(osc_handle* h, int task_id) { return osc_reset_robots(h, task_id, nullptr, OSC_MEM_DEVICE, OSC_RESET_REINITIALIZE); }
+
+int osc_reset_robots(osc_handle* h, int task_id, const int32_t* robot_mask, int mem_kind, int mode) {
 	ENTER(h);
 	if (task_id >= (int)h->tasks.size()) return fail(h, OSC_ERR_INVALID_ARGUMENT, "task id out of range");
-	for (int id = 0; id < (int)h->tasks.size(); id++) {
-		if (task_id >= 0 && id != task_id) continue;
-		const TaskInfo& t = h->tasks[id];
-		if (t.type == OSC_TASK_MOTION_FORCE)
-			CUDA_TRY(h, osc::launch_reinit_mft(h->prog, t.index, 0, h->stream));
-		else
-			CUDA_TRY(h, osc::launch_reinit_jt(h->prog, t.index, h->stream));
-		h->launches++;
-		if (task_otg(h, id).enabled) {	// _otg->reInitialize(current) (JointTask.cpp:106, MotionForceTask.cpp:244)
-			CUDA_TRY(h, osc::launch_otg_init(h->prog, id, 0, 0, h->stream));
-			h->launches++;
+	if (mode != OSC_RESET_REINITIALIZE && mode != OSC_RESET_CONSTRUCT) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad reset mode");
+	if (mem_kind != OSC_MEM_HOST && mem_kind != OSC_MEM_DEVICE) return fail(h, OSC_ERR_INVALID_ARGUMENT, "bad mem_kind");
+	const int32_t* mask = robot_mask;
+	if (robot_mask && mem_kind == OSC_MEM_HOST) {
+		if (!h->d_reset_mask) {
+			int rc = dev_alloc(h, &h->d_reset_mask, (size_t)h->NR, false);
+			if (rc != OSC_OK) return rc;
 		}
+		CUDA_TRY(h, cudaMemcpyAsync(h->d_reset_mask, robot_mask, (size_t)h->NR * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+		mask = h->d_reset_mask;
 	}
+	CUDA_TRY(h, osc::launch_reset_robots(h->prog, mask, task_id, mode == OSC_RESET_CONSTRUCT ? 1 : 0, h->stream));
+	h->launches++;
 	return OSC_OK;
 }
 
@@ -1402,7 +1405,7 @@ static int otg_enable_common(osc_handle* h, int task_id, int dim, const double* 
 	g.enabled = 1;
 	// off -> on: the generator restarts at the current position (JointTask.cpp:372-374, MotionForceTask.cpp:514-516) and the
 	// user's goals stay; already on: new limits only (OTG_joints.cpp:44-92)
-	CUDA_TRY(h, osc::launch_otg_init(h->prog, task_id, was_on ? 3 : 0, was_on ? 0 : 1, h->stream));
+	CUDA_TRY(h, osc::launch_otg_init(h->prog, task_id, was_on ? 3 : 0, h->stream));
 	h->launches++;
 	if (!was_on) h->otg_tasks++;
 	return OSC_OK;

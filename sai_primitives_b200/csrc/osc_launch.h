@@ -246,15 +246,16 @@ cudaError_t launch_popc_probe(const OscProgram& P, int mft_index, int K, const d
 cudaError_t measure_fp64_peak(double seconds, double* tflops, cudaStream_t stream);
 cudaError_t launch_sim_integrate(const OscProgram& P, double* q, double* dq, const double* tau, double dt, int substeps, cudaStream_t stream);
 cudaError_t launch_jla(const OscProgram& P, cudaStream_t stream);
-// internal OTG of the tasks (osc_otg_kernels.cuh): per-cycle update, (re)initialisation (mode 0 whole task, 1 linear part,
-// 2 angular part, 3 limits changed; fresh = generator constructed), switch-off
+// internal OTG of the tasks (osc_otg_kernels.cuh): per-cycle update, (re)initialisation (mode 0 enabled: generator constructed,
+// 1 linear part, 2 angular part, 3 limits changed), switch-off
 cudaError_t launch_otg_update(const OscProgram& P, cudaStream_t stream);
-cudaError_t launch_otg_init(const OscProgram& P, int task, int mode, int fresh, cudaStream_t stream);
+cudaError_t launch_otg_init(const OscProgram& P, int task, int mode, cudaStream_t stream);
 cudaError_t launch_otg_disable(const OscProgram& P, int task, cudaStream_t stream);
 // read-only observers (osc_observers.cuh): kind = ObserverKind, task = position in the hierarchy, out = ncomp x N (SoA)
 cudaError_t launch_observer(const OscProgram& P, int task, int kind, double* out, cudaStream_t stream);
-cudaError_t launch_reinit_mft(const OscProgram& P, int mft_index, int full_init, cudaStream_t stream);
-cudaError_t launch_reinit_jt(const OscProgram& P, int jt_index, cudaStream_t stream);
+// task resets of the robots selected by mask (device int32 x N, != 0 selects; null: every robot), task < 0: every task, in one
+// launch (reset_robots_kernel, osc_aux_kernels.cuh).  construct = 0: reInitializeTask; 1: the state the constructor leaves
+cudaError_t launch_reset_robots(const OscProgram& P, const int32_t* mask, int task, int construct, cudaStream_t stream);
 cudaError_t launch_sensed_wrench(const OscProgram& P, int mft_index, const double* f, const double* m, cudaStream_t stream);
 cudaError_t launch_eval_model(const OscProgram& P, const osc_link_frame& frame, double* M, double* J, double* x, double* R,
 							  double* g, cudaStream_t stream);

@@ -143,55 +143,93 @@ __global__ void __launch_bounds__(64) otg_update_kernel(const __grid_constant__ 
 	}
 }
 
-// (re)initialisation of a generator from the task's current state.
-// mode 0: enable / reInitializeTask -- user goals := the task's goal slots (enable) or the current state (reinit), generator
-//         constructed / re-initialised at the current position (and orientation);
-// mode 1: parametrizeForceMotionSpaces reset -> reInitializeLinear; mode 2: parametrizeMomentRotMotionSpaces reset -> reInitializeAngular
+// Task-space position S q of a JointTask (k entries): the goal its reset sets and the position its generator starts from.
 template <int N>
-__global__ void otg_init_kernel(const __grid_constant__ OscProgram P, int task, int mode, int fresh) {
+DEVI void jt_task_position(const DevJt& t, const double (&q)[N], double pos[OSC_MAX_DOF]) {
+	for (int a = 0; a < t.k; a++) {
+		double s = 0.0;
+#pragma unroll
+		for (int j = 0; j < N; j++) s += t.S[a][j] * q[j];
+		pos[a] = s;
+	}
+}
+
+// (Re)initialisation of robot i's joint generator at the task-space position pos (k entries), then the desired state into the
+// task's goal slots.  fresh: constructed as enabling it does (JointTask.cpp:372-374), the user's goals become what the task's
+// goal slots hold; otherwise _otg->reInitialize of JointTask::reInitializeTask (JointTask.cpp:106): goal := current position,
+// zero velocity and acceleration goals.
+static __device__ __noinline__ void otg_joint_init(const DevJt& t, int64_t NR, int64_t i, const double* pos, bool fresh) {
+	const DevOtg& g = t.otg;
+	otg::JointsOtg<8> o;
+	if (fresh) {
+		for (int c = 0; c < OJ_CORE_DOUBLES; c++) reinterpret_cast<double*>(&o)[c] = 0.0;
+		o.flags = 0;
+		for (int a = 0; a < OSC_MAX_DOF; a++) {
+			g.st[(int64_t)(OJ_USER_POS + a) * NR + i] = t.st[(int64_t)(JC_GOAL_POS + a) * NR + i];
+			g.st[(int64_t)(OJ_USER_VEL + a) * NR + i] = t.st[(int64_t)(JC_GOAL_VEL + a) * NR + i];
+			g.st[(int64_t)(OJ_USER_ACC + a) * NR + i] = t.st[(int64_t)(JC_GOAL_ACC + a) * NR + i];
+		}
+	} else {
+		otg_load(o, g.st, NR, i, OJ_CORE, OJ_CORE_DOUBLES);
+		o.flags = g.flags[i];
+		for (int a = 0; a < OSC_MAX_DOF; a++) {
+			g.st[(int64_t)(OJ_USER_POS + a) * NR + i] = a < t.k ? pos[a] : 0.0;
+			g.st[(int64_t)(OJ_USER_VEL + a) * NR + i] = 0.0;
+			g.st[(int64_t)(OJ_USER_ACC + a) * NR + i] = 0.0;
+		}
+	}
+	o.reinitialize(t.k, pos);
+	otg_store(o, g.st, NR, i, OJ_CORE, OJ_CORE_DOUBLES);
+	g.flags[i] = o.flags;
+	for (int a = 0; a < t.k; a++) {
+		t.st[(int64_t)(JC_GOAL_POS + a) * NR + i] = o.out_pos[a];
+		t.st[(int64_t)(JC_GOAL_VEL + a) * NR + i] = 0.0;
+		t.st[(int64_t)(JC_GOAL_ACC + a) * NR + i] = 0.0;
+	}
+}
+
+// The same for the Cartesian generator at the current pose (x, R): fresh = constructed (MotionForceTask.cpp:514-516) with the
+// user's goals := the task's goal slots; otherwise _otg->reInitialize of MotionForceTask::reInitializeTask (:244).
+static __device__ __noinline__ void otg_cart_init(const DevMft& t, int64_t NR, int64_t i, const double x[3], const double R[9], bool fresh) {
+	const DevOtg& g = t.otg;
+	otg::CartesianOtg o;
+	if (fresh) {
+		for (int c = 0; c < 24; c++) g.st[(int64_t)(OC_USER + c) * NR + i] = t.st[(int64_t)(MC_GOAL_POS + c) * NR + i];
+		o.construct(x, R);
+	} else {
+		otg_load(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
+		o.g.flags = g.flags[i];
+		for (int c = 0; c < 24; c++) g.st[(int64_t)(OC_USER + c) * NR + i] = 0.0;
+		for (int c = 0; c < 3; c++) g.st[(int64_t)(OC_USER + MC_GOAL_POS + c) * NR + i] = x[c];
+		for (int c = 0; c < 9; c++) g.st[(int64_t)(OC_USER + MC_GOAL_ORI + c) * NR + i] = R[c];
+		o.reinitialize(x, R);
+	}
+	otg_store(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
+	g.flags[i] = o.g.flags;
+	otg_cart_write_desired(t, o, NR, i);
+}
+
+// Generator calls of the host layer other than resets (those are reset_robots_kernel, osc_aux_kernels.cuh):
+// mode 0: enabled -- constructed at the current position (and orientation), the user's goals are the task's goal slots;
+// mode 1: parametrizeForceMotionSpaces reset -> reInitializeLinear; mode 2: parametrizeMomentRotMotionSpaces reset -> reInitializeAngular;
+// mode 3: new limits.
+template <int N>
+__global__ void otg_init_kernel(const __grid_constant__ OscProgram P, int task, int mode) {
 	const int64_t NR = P.n_robots;
 	const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= NR) return;
 	if (P.tasks[task].type == OSC_TASK_JOINT) {
 		const DevJt& t = P.jt[P.tasks[task].index];
 		const DevOtg& g = t.otg;
-		double pos[OSC_MAX_DOF];
-		for (int a = 0; a < t.k; a++) {
-			double s = 0.0;
-			for (int j = 0; j < N; j++) s += t.S[a][j] * P.q[(int64_t)j * NR + i];
-			pos[a] = s;
-		}
 		if (mode == 3) {  // OTG_joints::setMaxVelocity / setMaxAcceleration / disableJerkLimits (:89-92): the acceleration state is dropped
 			for (int a = 0; a < OSC_MAX_DOF; a++) g.st[(int64_t)(OJ_CORE + 32 + a) * NR + i] = 0.0;  // JointsOtg::in_acc
 			g.flags[i] |= otg::OTG_DIRTY;
 			return;
 		}
-		otg::JointsOtg<8> o;
-		if (fresh) {
-			for (int c = 0; c < OJ_CORE_DOUBLES; c++) reinterpret_cast<double*>(&o)[c] = 0.0;
-			o.flags = 0;
-			for (int a = 0; a < OSC_MAX_DOF; a++) {	 // the user's goals stay what they were (the task's goal slots)
-				g.st[(int64_t)(OJ_USER_POS + a) * NR + i] = t.st[(int64_t)(JC_GOAL_POS + a) * NR + i];
-				g.st[(int64_t)(OJ_USER_VEL + a) * NR + i] = t.st[(int64_t)(JC_GOAL_VEL + a) * NR + i];
-				g.st[(int64_t)(OJ_USER_ACC + a) * NR + i] = t.st[(int64_t)(JC_GOAL_ACC + a) * NR + i];
-			}
-		} else {
-			otg_load(o, g.st, NR, i, OJ_CORE, OJ_CORE_DOUBLES);
-			o.flags = g.flags[i];
-			for (int a = 0; a < OSC_MAX_DOF; a++) {	 // JointTask::reInitializeTask: goal = current, zero velocity / acceleration goals
-				g.st[(int64_t)(OJ_USER_POS + a) * NR + i] = a < t.k ? pos[a] : 0.0;
-				g.st[(int64_t)(OJ_USER_VEL + a) * NR + i] = 0.0;
-				g.st[(int64_t)(OJ_USER_ACC + a) * NR + i] = 0.0;
-			}
-		}
-		o.reinitialize(t.k, pos);
-		otg_store(o, g.st, NR, i, OJ_CORE, OJ_CORE_DOUBLES);
-		g.flags[i] = o.flags;
-		for (int a = 0; a < t.k; a++) {
-			t.st[(int64_t)(JC_GOAL_POS + a) * NR + i] = o.out_pos[a];
-			t.st[(int64_t)(JC_GOAL_VEL + a) * NR + i] = 0.0;
-			t.st[(int64_t)(JC_GOAL_ACC + a) * NR + i] = 0.0;
-		}
+		double q[N], pos[OSC_MAX_DOF];
+		for (int j = 0; j < N; j++) q[j] = P.q[(int64_t)j * NR + i];
+		jt_task_position<N>(t, q, pos);
+		otg_joint_init(t, NR, i, pos, true);
 		return;
 	}
 	const DevMft& t = P.mft[P.tasks[task].index];
@@ -200,28 +238,14 @@ __global__ void otg_init_kernel(const __grid_constant__ OscProgram P, int task, 
 		g.flags[i] |= otg::OTG_DIRTY;
 		return;
 	}
-	if (!fresh && (mode == 1 || mode == 2)) {
+	if (mode == 1 || mode == 2) {
 		otg_cart_reinit_part(t, NR, i, mode == 2);
 		return;
 	}
 	double x[3], R[9];
 	for (int c = 0; c < 3; c++) x[c] = t.st[(int64_t)(MC_CUR_POS + c) * NR + i];
 	for (int c = 0; c < 9; c++) R[c] = t.st[(int64_t)(MC_CUR_ORI + c) * NR + i];
-	otg::CartesianOtg o;
-	if (fresh) {
-		for (int c = 0; c < 24; c++) g.st[(int64_t)(OC_USER + c) * NR + i] = t.st[(int64_t)(MC_GOAL_POS + c) * NR + i];
-		o.construct(x, R);
-	} else {
-		otg_load(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
-		o.g.flags = g.flags[i];
-		for (int c = 0; c < 24; c++) g.st[(int64_t)(OC_USER + c) * NR + i] = 0.0;  // mode 0
-		for (int c = 0; c < 3; c++) g.st[(int64_t)(OC_USER + MC_GOAL_POS + c) * NR + i] = x[c];
-		for (int c = 0; c < 9; c++) g.st[(int64_t)(OC_USER + MC_GOAL_ORI + c) * NR + i] = R[c];
-		o.reinitialize(x, R);
-	}
-	otg_store(o, g.st, NR, i, OC_CORE, OC_CORE_DOUBLES);
-	g.flags[i] = o.g.flags;
-	otg_cart_write_desired(t, o, NR, i);
+	otg_cart_init(t, NR, i, x, R, true);
 }
 
 // generator switched off: the user's goals go back into the slots the control laws read
